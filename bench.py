@@ -2,6 +2,7 @@
 """Headline benchmark: ST-encoder fbank frames/s (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg1]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic batch: per-utterance fbank CMVN, then the
 encoder forward (conv subsampling -> 11 pre-LN layers with log-penalty attention -> CTC argmax
@@ -135,6 +136,33 @@ def randomise_norm_stats(enc, seed):
             bn.running_var.copy_(torch.rand(bn.running_var.shape, generator=g) + 0.5)
             bn.weight.copy_(1.0 + 0.1 * torch.randn(bn.weight.shape, generator=g))
             bn.bias.copy_(0.1 * torch.randn(bn.bias.shape, generator=g))
+
+
+DUMP_BUDGET = 64 * 2 ** 20  # bytes --dump-outputs writes in all
+DUMP_SAMPLE = 6 * 2 ** 20   # elements kept of a larger output (ctc_out: T x B x vocab logits)
+
+
+def dump_outputs(out, dirname):
+    """--dump-outputs: every tensor of ``out`` (the output mapping the timed path hands its caller), as
+    DIR/<field>.npy (float32; lengths float64).  An output of more than DUMP_SAMPLE elements is written as
+    DIR/<field>_sample.npy: its elements at DUMP_SAMPLE flat indices drawn with a fixed seed, in index order,
+    so two builds given the same arguments can be compared element for element."""
+    import numpy as np
+    arrays = {}
+    for name, t in out.items():
+        if not isinstance(t, torch.Tensor) or name == "src_tokens":  # src_tokens is the input batch
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        arrays[name] = t.to(torch.float64 if name == "src_lengths" else torch.float32).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_BUDGET))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------ clocks sampler
@@ -419,6 +447,8 @@ def run_ours(args, rank, world, local_rank):
     launches = (ops.LAUNCHES - launches0) // args.steps
     dev_ms = ev0.elapsed_time(ev1)
     new_frames = float(out.src_lengths.sum().item())
+    if args.dump_outputs and rank == 0:  # before any later launch reuses the graph buffers `out` aliases
+        dump_outputs(out._asdict(), args.dump_outputs)
 
     # ---- informative: ONE forward at a time, L2 flushed (256 MB write, untimed) before each and ~1 ms of
     # untimed GPU-side delay so that the host enqueues the step while the GPU is still busy (no launch
@@ -762,6 +792,8 @@ def run_train(args, rank, world, local_rank):
     ev1.record()
     barrier()
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(dict(loss=last.detach()), args.dump_outputs)
     launches = (ops.LAUNCHES - launches0) // args.steps
     # e2e: batches start in pinned HOST memory (H2D inside), the loss is read back on the host every step
     host = [utils.apply_to_sample(lambda t: t.cpu().pin_memory(), s) for s in samples]
@@ -922,6 +954,8 @@ def run_ragged(args, rank, world, local_rank):
     out = run(1)
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:  # before the next pass reuses the graph buffers `out` aliases
+        dump_outputs(out._asdict(), args.dump_outputs)
     gc.enable()
     my_ms = ev0.elapsed_time(ev1)
     # untimed: every output of one more pass over the rank's batches must be finite (a ragged stream in persistent
@@ -1118,13 +1152,14 @@ def reference_gpu_eager(args, enc_state, plan, steps=3):
 def run_reference(args, rank, world):
     """Reference arm: the reference's own CPU implementation of the path (see cpu_reference) on ALL the
     utterances of the step -- the same config / metric / unit as our arm; under torchrun rank 0 alone
-    runs it.  The number of timed steps follows --steps but is cut when the run would exceed
-    --reference-budget-s (default 240 s; said in `cpu_baseline.sample`)."""
+    runs it.  It times --steps steps; --reference-budget-s stops it earlier (said in `cpu_baseline.sample`)."""
     if rank != 0:
         return None
     cfg = CONFIGS[args.config]
-    cb, _ = cpu_reference(args, steps=max(1, args.steps), warmup=max(1, min(args.warmup, 2)),
-                          sample_utts=len(cfg["lengths"]), budget_s=args.reference_budget_s)
+    cb, ref = cpu_reference(args, steps=max(1, args.steps), warmup=max(1, min(args.warmup, 2)),
+                            sample_utts=len(cfg["lengths"]), budget_s=args.reference_budget_s)
+    if args.dump_outputs:
+        dump_outputs(ref, args.dump_outputs)
     return dict(metric="encoder fbank frames/sec", value=cb["value"], unit="frames/s", n_gpus=world,
                 steps=args.steps, warmup=args.warmup, ms_per_step=cb["ms_per_sample"],
                 higher_is_better=True, scaling="weak", vs_baseline=None, dtype="f32", data="synthetic",
@@ -1135,8 +1170,8 @@ def run_reference(args, rank, world):
 
 
 def main():
-    # A run that is still going after 25 minutes is stuck (the default line takes ~1 minute, the reference arm is
-    # budgeted at 4): dump every thread's Python stack and exit non-zero instead of hanging without a trace.
+    # A run that is still going after 25 minutes is stuck (the default line takes ~1 minute, the reference arm
+    # a few seconds per step): dump every thread's Python stack and exit non-zero instead of hanging without a trace.
     import faulthandler
     faulthandler.dump_traceback_later(int(os.environ.get("FBKST_BENCH_DEADLINE_S", "1500")), exit=True)
     ap = argparse.ArgumentParser()
@@ -1158,10 +1193,15 @@ def main():
                          "kernels) instead of the fused epilogue's built-in bump")
     ap.add_argument("--port-baseline", action="store_true",
                     help="time the CPU oracle port even when the reference tree (baseline/_ref) is present")
-    ap.add_argument("--reference-budget-s", type=float, default=240.0,
-                    help="--impl reference: stop timing after this many seconds (>= 1 timed step)")
+    ap.add_argument("--reference-budget-s", type=float, default=None,
+                    help="--impl reference: stop timing after this many seconds (>= 1 timed step; default: "
+                         "time all --steps steps)")
     ap.add_argument("--soak-seconds", type=float, default=2.0,
                     help="length of the sustained-throughput soak reported under roofline.sustained (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (the encoder output tuple with a seeded "
+                         "sample of ctc_out; cfg4: the loss) to DIR/<name>.npy, rank 0; inputs are seeded, so "
+                         "runs with the same arguments can be compared")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))

@@ -13,6 +13,7 @@ Contents
                     in-process shims of SURVEY.md F1/F2/F11 (only usable in the
                     build container; the GPU box has no ``/root/reference``).
 ``make_golden``     regenerates ``tests/golden/*.pt`` from the live reference.
+``golden``          saves / loads those fixtures (one of more than 1 MB as parts of at most 1 MB).
 
 Parity pinning: the reference's own test-suite holds NO golden vector for this
 path (SURVEY.md section 4 / 8c) -- "parity unpinned" by the reference's suite.  The

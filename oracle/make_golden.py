@@ -6,8 +6,8 @@ Run in the build container (needs ``/root/reference``):
 
 Each fixture stores inputs, the reference's own ``state_dict`` and the outputs
 of the reference's own ``ConvolutionalTransformerEncoder.forward`` (eval mode,
-CPU fp32, shims of ``oracle/ref_loader.py``).  Fixtures are small (< 2 MB) so
-they can be committed; they travel to the GPU box where the reference cannot.
+CPU fp32, shims of ``oracle/ref_loader.py``).  They are committed, so the tests
+need no reference; ``oracle/golden.py`` stores a fixture of more than 1 MB as parts.
 """
 import os
 import sys
@@ -17,6 +17,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from oracle import encoder_oracle as O  # noqa: E402
+from oracle import golden  # noqa: E402
 from oracle import ref_loader as R  # noqa: E402
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
@@ -122,10 +123,10 @@ def cmvn_fixture():
 
 def main():
     os.makedirs(GOLDEN_DIR, exist_ok=True)
-    torch.save(encoder_fixture(TINY, [61, 47, 30], 0, ["avg", "weighted", "softmax"]),
-               os.path.join(GOLDEN_DIR, "enc_tiny_log.pt"))
-    torch.save(encoder_fixture(TINY_NOPEN, [40, 40], 1, ["avg"]),
-               os.path.join(GOLDEN_DIR, "enc_tiny_nopen.pt"))
+    golden.save(encoder_fixture(TINY, [61, 47, 30], 0, ["avg", "weighted", "softmax"]),
+                os.path.join(GOLDEN_DIR, "enc_tiny_log.pt"))
+    golden.save(encoder_fixture(TINY_NOPEN, [40, 40], 1, ["avg"]),
+                os.path.join(GOLDEN_DIR, "enc_tiny_nopen.pt"))
     torch.save(ctc_fixture(), os.path.join(GOLDEN_DIR, "ctc_compress.pt"))
     torch.save(cmvn_fixture(), os.path.join(GOLDEN_DIR, "cmvn.pt"))
     for f in sorted(os.listdir(GOLDEN_DIR)):

@@ -15,7 +15,7 @@ import random
 import numpy as np
 import torch
 
-from . import ref_loader
+from . import golden, ref_loader
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden",
                       "augment.pt")
@@ -74,7 +74,7 @@ def main():
         out["stretch"][name] = {"seed": seed, "x": x, "lengths": lengths, "pars": pars, "ref": y.clone(),
                                 "ref_lengths": nl.tolist(), "ref_ids": ids}
         print("stretch", name, lengths, "->", nl.tolist())
-    torch.save(out, GOLDEN)
+    golden.save(out, GOLDEN)
 
 
 if __name__ == "__main__":

@@ -13,7 +13,7 @@ import os
 import torch
 
 from . import cross_attention_oracle as X
-from . import ref_loader
+from . import golden, ref_loader
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden",
                       "xattn.pt")
@@ -72,8 +72,8 @@ def main():
         "single_beam5": run_case(MultiheadAttention, 3, 128, 2, 128, 45, [45], 5,
                                  [None, [4, 3, 2, 1, 0], [0, 0, 0, 1, 1]], False),
     }
-    torch.save(cases, GOLDEN)
-    print("wrote", GOLDEN, os.path.getsize(GOLDEN), "bytes")
+    for p in golden.save(cases, GOLDEN):
+        print("wrote", p, os.path.getsize(p), "bytes")
 
 
 if __name__ == "__main__":

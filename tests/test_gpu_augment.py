@@ -13,6 +13,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 from oracle import augment_oracle as A  # noqa: E402  (checker only)
+from oracle.golden import load as load_golden  # noqa: E402
 
 
 def seed(s):
@@ -26,7 +27,7 @@ def dev():
 
 def test_specaugment_golden(golden_dir):
     from fbkst_b200.augment import SpecAugment
-    golden = torch.load(os.path.join(golden_dir, "augment.pt"), weights_only=False)["spec"]
+    golden = load_golden(os.path.join(golden_dir, "augment.pt"))["spec"]
     for name, c in golden.items():
         seed(c["seed"])
         x = c["x"].to(dev())
@@ -37,7 +38,7 @@ def test_specaugment_golden(golden_dir):
 
 def test_time_stretch_golden(golden_dir):
     from fbkst_b200.augment import TimeStretch
-    golden = torch.load(os.path.join(golden_dir, "augment.pt"), weights_only=False)["stretch"]
+    golden = load_golden(os.path.join(golden_dir, "augment.pt"))["stretch"]
     for name, c in golden.items():
         seed(c["seed"])
         m = TimeStretch(*c["pars"])

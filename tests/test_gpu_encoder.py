@@ -10,6 +10,7 @@ pytestmark = pytest.mark.gpu
 
 from helpers import build_encoder, parity_report, rel_err  # noqa: E402
 from oracle import encoder_oracle as O  # noqa: E402  (checker only)
+from oracle.golden import load as load_golden  # noqa: E402
 
 TOL = 2e-2
 
@@ -34,7 +35,7 @@ def check_against(out, ref, lens_in, tol=TOL):
 
 @pytest.mark.parametrize("name", ["enc_tiny_log.pt", "enc_tiny_nopen.pt"])
 def test_encoder_golden(golden_dir, name):
-    fx = torch.load(os.path.join(golden_dir, name), weights_only=False)
+    fx = load_golden(os.path.join(golden_dir, name))
     cfg = fx["cfg"]
     for strategy, ref in fx["outputs"].items():
         enc = build_encoder(dict(cfg, ctc_strategy=strategy), fx["state_dict"])
@@ -55,7 +56,7 @@ def test_encoder_golden(golden_dir, name):
 def test_state_dict_layout_matches_reference(golden_dir):
     """Reference checkpoints load strict=True and our keys/shapes equal the reference's."""
     for name in ["enc_tiny_log.pt", "enc_tiny_nopen.pt"]:
-        fx = torch.load(os.path.join(golden_dir, name), weights_only=False)
+        fx = load_golden(os.path.join(golden_dir, name))
         enc = build_encoder(fx["cfg"], fx["state_dict"])
         ours = enc.state_dict()
         assert set(ours.keys()) == set(fx["state_dict"].keys())
@@ -96,7 +97,7 @@ def test_encoder_big2_ragged_vs_oracle(strategy):
 
 
 def test_reorder_and_non_torchscript(golden_dir):
-    fx = torch.load(os.path.join(golden_dir, "enc_tiny_log.pt"), weights_only=False)
+    fx = load_golden(os.path.join(golden_dir, "enc_tiny_log.pt"))
     enc = build_encoder(fx["cfg"], fx["state_dict"])
     net_input = dict(src_tokens=fx["src_tokens"].cuda(), src_lengths=fx["src_lengths"].cuda(),
                      prev_output_tokens=torch.zeros(3, 5), transcript_prev_output_tokens=None)
@@ -114,7 +115,7 @@ def test_pipeline_matches_direct_calls(golden_dir, graph, lanes):
     launch + deferred finish) returns exactly what direct calls return."""
     from fbkst_b200 import ops
     from fbkst_b200.pipeline import EncoderPipeline
-    fx = torch.load(os.path.join(golden_dir, "enc_tiny_log.pt"), weights_only=False)
+    fx = load_golden(os.path.join(golden_dir, "enc_tiny_log.pt"))
     enc = build_encoder(fx["cfg"], fx["state_dict"])
     batches = []
     for i, lens in enumerate([[61, 47, 30], [90, 90], [33, 20, 20, 7], [61, 47, 30], [61, 40, 33],

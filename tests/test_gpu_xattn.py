@@ -10,6 +10,7 @@ import torch
 from fbkst_b200 import ops
 from fbkst_b200.cross_attention import CrossAttention, reorder_tagged
 from oracle import cross_attention_oracle as X  # checker only
+from oracle.golden import load as load_golden
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -80,7 +81,7 @@ def test_bad_arguments_raise():
 
 @pytest.fixture(scope="module")
 def golden(golden_dir):
-    return torch.load(os.path.join(golden_dir, "xattn.pt"), weights_only=False)
+    return load_golden(os.path.join(golden_dir, "xattn.pt"))
 
 
 def _module(c):

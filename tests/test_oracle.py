@@ -6,11 +6,12 @@ import pytest
 import torch
 
 from oracle import encoder_oracle as O
+from oracle.golden import load as load_golden
 from oracle import ref_loader as R
 
 
 def load(golden_dir, name):
-    return torch.load(os.path.join(golden_dir, name), weights_only=False)
+    return load_golden(os.path.join(golden_dir, name))
 
 
 def assert_close(a, b, tol=1e-5):
@@ -98,13 +99,14 @@ def test_oracle_vs_live_reference_cfg1_shape():
     assert torch.equal(out["encoder_padding_mask"], ref.encoder_padding_mask)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not R.available(), reason="live reference not mounted")
-def test_init_state_dict_matches_reference_keys():
+def test_init_state_dict_matches_reference_keys(golden_dir):
+    """Keys and shapes of the reference encoder's state_dict for this configuration, as stored by
+    oracle/make_golden.py in enc_tiny_log.pt."""
     cfg = dict(embed_dim=128, ffn_dim=128, heads=2, layers=2, conv_channels=64, feat_dim=40,
                vocab=48, distance_penalty="log", ctc_layer=1, ctc_strategy="avg")
-    enc = R.build_reference_encoder(cfg, seed=0)
-    ref = enc.state_dict()
+    fx = load(golden_dir, "enc_tiny_log.pt")
+    assert {k: v for k, v in fx["cfg"].items() if k != "dropout"} == cfg
+    ref = fx["state_dict"]
     sd = O.init_state_dict(cfg)
     assert set(sd.keys()) == set(ref.keys())
     for k in ref:

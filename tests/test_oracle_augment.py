@@ -11,12 +11,13 @@ import pytest
 import torch
 
 from oracle import augment_oracle as A
+from oracle.golden import load as load_golden
 from oracle import ref_loader
 
 
 @pytest.fixture(scope="module")
 def golden(golden_dir):
-    return torch.load(os.path.join(golden_dir, "augment.pt"), weights_only=False)
+    return load_golden(os.path.join(golden_dir, "augment.pt"))
 
 
 def seed(s):

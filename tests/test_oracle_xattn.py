@@ -6,11 +6,12 @@ import pytest
 import torch
 
 from oracle import cross_attention_oracle as X
+from oracle.golden import load as load_golden
 
 
 @pytest.fixture(scope="module")
 def golden(golden_dir):
-    return torch.load(os.path.join(golden_dir, "xattn.pt"), weights_only=False)
+    return load_golden(os.path.join(golden_dir, "xattn.pt"))
 
 
 def _close(a, b, tol=2e-5):

@@ -1,12 +1,14 @@
 """Host logic of the N4 row (no GPU): beam tags left by reorder_encoder_out, the row-map form of
 reorder_incremental_state, state_dict compatibility with the reference block, no CPU fallback."""
+import os
+
 import pytest
 import torch
 
 from fbkst_b200.cross_attention import CrossAttention, beam_source, reorder_tagged, swap_cross_attention
 from fbkst_b200.encoder import ConvolutionalTransformerEncoder, EncoderOut
 from oracle import cross_attention_oracle as X
-from oracle import ref_loader as R
+from oracle.golden import load as load_golden
 
 
 def _enc_out(S=7, U=3, D=8):
@@ -70,16 +72,24 @@ def test_no_cpu_fallback_and_no_backward():
         CrossAttention(96, 2)  # head_dim 48
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not R.available(), reason="live reference not mounted")
-def test_state_dict_is_the_reference_blocks():
-    R.load()
-    from fairseq.modules.multihead_attention import MultiheadAttention
-    ref = MultiheadAttention(128, 2, kdim=192, vdim=192, encoder_decoder_attention=True)
-    ours = CrossAttention(128, 2, kdim=192, vdim=192)
-    assert {k: tuple(v.shape) for k, v in ref.state_dict().items()} == \
+def test_state_dict_is_the_reference_blocks(golden_dir):
+    """Parameters of the reference's MultiheadAttention(256, 4, kdim=192, vdim=192,
+    encoder_decoder_attention=True), as oracle/make_golden_xattn.py loaded them into it with strict=True
+    (xattn.pt, case nomask_heads): same keys and shapes here, strict load, and swap_cross_attention
+    keeps a decoder's state_dict keys and parameter tensors."""
+    case = load_golden(os.path.join(golden_dir, "xattn.pt"))["nomask_heads"]
+    D, H, kdim, params = case["D"], case["H"], case["kdim"], case["params"]
+    ours = CrossAttention(D, H, kdim=kdim, vdim=kdim)
+    assert {k: tuple(v.shape) for k, v in params.items()} == \
            {k: tuple(v.shape) for k, v in ours.state_dict().items()}
-    ours.load_state_dict(ref.state_dict(), strict=True)
+    ours.load_state_dict(params, strict=True)
+
+    ref = torch.nn.Module()  # what swap_cross_attention reads of a MultiheadAttention, in its layout
+    ref.embed_dim, ref.num_heads, ref.kdim, ref.vdim, ref.dropout = D, H, kdim, kdim, 0.0
+    for nm in ("k_proj", "v_proj", "q_proj", "out_proj"):  # multihead_attention.py registration order
+        w = params[nm + ".weight"]
+        setattr(ref, nm, torch.nn.Linear(w.shape[1], w.shape[0]))
+    ref.load_state_dict(params, strict=True)
 
     class _Layer(torch.nn.Module):
         def __init__(self):
