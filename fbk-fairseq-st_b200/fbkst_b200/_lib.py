@@ -48,6 +48,11 @@ SIGNATURES = {
     "fbkst_prep_conv2_weight": [P, P, I, P],
     "fbkst_prep_fc3_weight": [P, P, I, I, I, P],
     "fbkst_prep_bn_affine": [P, P, P, P, F, P, P, I, P],
+    # fp32-accurate inference path (split TF32)
+    "fbkst_linear_tf32x3": [P, I64, P, I64, P, P, P, P, I64, P, I64, I, I, I, I, P, I, P],
+    "fbkst_attention_tf32x3": [P, P, P, I, I, I, I, P, P],
+    "fbkst_conv1_relu_bn_f32": [P, P, P, P, P, P, I, I, I, I, P],
+    "fbkst_conv2_im2col_f32": [P, P, I, I, I, I, P],
     # training side
     "fbkst_dropout_add_ln": [P, P, P, P, P, P, F, I, I, F, U64, I, P],
     "fbkst_ln_bwd_blocks": [I],

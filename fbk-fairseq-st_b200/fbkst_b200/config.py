@@ -53,4 +53,5 @@ def build_encoder(cfg, state_dict=None, device="cuda:0"):
     # callers that want gradients re-enable requires_grad; fairseq's generate / validate run under no_grad.)
     for p in enc.parameters():
         p.requires_grad_(False)
+    enc.precision = cfg.get("precision", "bf16")  # "fp32": split-TF32 inference path (encoder.precision)
     return enc.to(device).eval()

@@ -184,9 +184,14 @@ class CtcProjection(nn.Linear):
     exact ties by a bf16 store (ADVICE r01).  ``logits_dtype = torch.bfloat16`` is an opt-in that halves
     the 2 x L*B*V*4 bytes this costs, for callers that accept bf16-rounded logits."""
     logits_dtype = torch.float32
+    precision = "bf16"  # set by the encoder's ``precision``: "fp32" runs the split-TF32 GEMM on fp32 operands
 
     def forward(self, x):  # noqa: D401
         L, B, D = x.shape
+        if self.precision == "fp32":
+            self._bf16_operand = None
+            w, b = self._prepared_f32()
+            return ops.linear_f32(x.reshape(L * B, D).contiguous(), w, b).view(L, B, -1)
         w, b = self._prepared()
         pre = getattr(self, "_bf16_operand", None)  # (data_ptr of x, bf16(x)) left by the fc2 epilogue
         self._bf16_operand = None
@@ -208,6 +213,16 @@ class CtcProjection(nn.Linear):
             self._prep = (ops.cast_bf16(self.weight.detach()), self.bias.detach().float().contiguous())
             self._prep_key = key
         return self._prep
+
+    def _prepared_f32(self):
+        key = (self.weight._version, self.bias._version, self.weight.data_ptr())
+        if getattr(self, "_prep32_key", None) != key:
+            self._prep32 = (self.weight.detach().float().contiguous(), self.bias.detach().float().contiguous())
+            self._prep32_key = key
+        return self._prep32
+
+
+PRECISIONS = ("bf16", "fp32")
 
 
 def make_encoder_class(base):
@@ -288,6 +303,9 @@ def make_encoder_class(base):
                     raise ValueError("unknown --ctc-compress-strategy %r" % self.ctc_compress_strategy)
             self._prep = None
             self._prep_key = None
+            self._prep32 = None
+            self._prep32_key = None
+            self._precision = "bf16"
             self._pos_table = None
             self._ws = None
             self._ws_key = None
@@ -303,7 +321,68 @@ def make_encoder_class(base):
             self.ctc_logit_bump = None
             self._pins = _PinnedPool()  # pinned staging vectors for lengths (H2D sources, D2H results)
 
+        @property
+        def precision(self):
+            """Operand precision of the inference forward: ``"bf16"`` (default; bf16 / fp16 tensor-core operands,
+            fp32 accumulation) or ``"fp32"`` (split-TF32 tensor-core operands, about 21 significant bits, fp32
+            softmax and LayerNorm: within 1e-3 of an fp32 reference).  Training runs in bf16 only."""
+            return self._precision
+
+        @precision.setter
+        def precision(self, value):
+            if value not in PRECISIONS:
+                raise ValueError("fbkst_b200: precision must be one of %s, got %r" % (PRECISIONS, value))
+            self._precision = value
+            if self.ctc_compress_out:
+                self.ctc_fc.precision = value
+
         # ------------------------------------------------------------------ derived operand formats
+        def _params_key(self):
+            return tuple((p._version, p.data_ptr()) for p in list(self.parameters()) + list(self.buffers()))
+
+        def _prepared_active(self):
+            return self._prepared_f32() if self._precision == "fp32" else self._prepared()
+
+        def _prepared_f32(self):
+            """Operands of the fp32 path: plain fp32 (the kernels split them), no LayerNorm folding (the fold
+            feeds an uncentred operand); the conv and fc3 weights permuted to the channels-last patch order."""
+            key = self._params_key()
+            if self._prep32_key == key:
+                return self._prep32
+            f32 = lambda t: t.detach().float().contiguous()
+            with torch.no_grad():
+                P = {}
+                C = self.conv_channels
+                P["w1"] = f32(self.convolutions[0].weight.reshape(C, 9))
+                P["b1"] = f32(self.convolutions[0].bias)
+                P["w2"] = ops.prep_conv2_weight_f32(self.convolutions[1].weight)
+                P["b2"] = f32(self.convolutions[1].bias)
+                for i in range(2):
+                    bn = self.bn[i]
+                    P["bn%d" % i] = ops.prep_bn_affine(f32(bn.weight), f32(bn.bias), f32(bn.running_mean),
+                                                       f32(bn.running_var), bn.eps)
+                P["w3"] = ops.prep_fc3_weight_f32(self.fc3.weight, C, self.feat_out)
+                P["b3"] = f32(self.fc3.bias)
+                D = self.embed_dim
+                layers = []
+                for lyr in self.layers:
+                    w, b = lyr.self_attn.qkv()
+                    w, b = w.detach().float().clone(), b.detach().float().clone()
+                    w[:D] *= 64 ** -0.5  # head_dim ** -0.5 on the q rows (exact: 2^-3), local_attention.py:98
+                    b[:D] *= 64 ** -0.5
+                    ln1, ln2 = lyr.self_attn_layer_norm, lyr.final_layer_norm
+                    layers.append(dict(
+                        ln1=(f32(ln1.weight), f32(ln1.bias)), eps1=ln1.eps, wqkv=w.contiguous(), bqkv=b.contiguous(),
+                        wo=f32(lyr.self_attn.out_proj.weight), bo=f32(lyr.self_attn.out_proj.bias),
+                        ln2=(f32(ln2.weight), f32(ln2.bias)), eps2=ln2.eps,
+                        w1=f32(lyr.fc1.weight), b1=f32(lyr.fc1.bias), w2=f32(lyr.fc2.weight), b2=f32(lyr.fc2.bias)))
+                P["layers"] = layers
+                P["lnf"] = (f32(self.layer_norm.weight), f32(self.layer_norm.bias))
+                if self.layernorm_embedding is not None:
+                    P["lne"] = (f32(self.layernorm_embedding.weight), f32(self.layernorm_embedding.bias))
+            self._prep32, self._prep32_key = P, key
+            return P
+
         def _prepared(self):
             params = list(self.parameters()) + list(self.buffers())
             key = tuple((p._version, p.data_ptr()) for p in params)
@@ -375,6 +454,10 @@ def make_encoder_class(base):
             # dropout).  Both run fbkst_b200.train: hand-written forward + backward kernels, no PyTorch
             # arithmetic.  Everything else is the inference path.
             if self.training or (torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())):
+                if self._precision != "bf16":
+                    raise NotImplementedError(
+                        "fbkst_b200: precision=%r is inference only (eval() under torch.no_grad()); training and "
+                        "the backward run with precision='bf16'" % self._precision)
                 from .train import forward_train
                 return forward_train(self, src_tokens, src_lengths, return_all_hiddens)
             with torch.no_grad():
@@ -430,8 +513,8 @@ def make_encoder_class(base):
             else:
                 lengths = len_dev if len_dev is not None else \
                     torch.tensor(len_host, dtype=torch.int32).to(dev, non_blocking=True)
-                r = self._body(self._prepared(), x_in, lengths, len_host, L, B, return_all_hiddens,
-                               self._workspace(L * B, dev) if compress and not return_all_hiddens else None)
+                r = self._run_body(self._prepared_active(), x_in, lengths, len_host, L, B, return_all_hiddens,
+                                   self._workspace(L * B, dev) if compress and not return_all_hiddens else None)
             x, limit, new_len, states = r["x"], r["limit"], r["new_len"], r["states"]
             mask_in = r["mask"]
             if self.use_cuda_graph and not return_all_hiddens:
@@ -442,7 +525,7 @@ def make_encoder_class(base):
             if return_all_hiddens and compress:
                 len_host, L = r["len_host"], r["L"]
                 mask = r["mask2"] if min(len_host) < L else None
-            xf = ops.layernorm(x, *self._prepared()["lnf"], out_dtype=torch.float32, rows_limit=limit)
+            xf = ops.layernorm(x, *self._prepared_active()["lnf"], out_dtype=torch.float32, rows_limit=limit)
             deferred = limit is not None or len_host is None
             h = dict(xf=xf, mask=mask, ctc_mask=ctc_mask, mask_in=mask_in, states=states, len_host=len_host,
                      L=L, B=B, x_ctc=r["x_ctc"], src_tokens=src_tokens, len_dtype=src_lengths.dtype, dev=dev,
@@ -579,11 +662,67 @@ def make_encoder_class(base):
             r.update(x=x, limit=limit, new_len=new_len, states=states)
             return r
 
+        def _run_body(self, *args):
+            return (self._body_f32 if self._precision == "fp32" else self._body)(*args)
+
+        def _body_f32(self, P, x_in, lengths, len_host, L, B, want_states, ws):
+            """``_body`` with fp32 activations and split-TF32 operands (``precision = "fp32"``): the same
+            shapes, row limits and outputs, explicit LayerNorms in fp32, no bf16 copies."""
+            dev = x_in.device
+            D, H = self.embed_dim, self.heads
+            f32 = torch.float32
+            y = ops.conv1_relu_bn_f32(x_in, P["w1"], P["b1"], *P["bn0"])
+            y = ops.conv2_relu_bn_f32(y, P["w2"], P["b2"], *P["bn1"])  # [B, T2, F2, C]
+            assert y.shape[1] == L
+            h3 = ops.linear_f32(y.view(B * L, -1), P["w3"], P["b3"], relu=True)  # (b, t) rows, :227
+            table = self._positions(L + 1, dev) if self.embed_positions is not None else None
+            x = ops.embed_remap_stats(h3, L, B, table, lengths if table is not None else None)[0]
+            if self.layernorm_embedding is not None:
+                x = ops.layernorm(x, *P["lne"], out_dtype=f32)
+            mask = ops.lengths_to_mask(lengths, L)[0]
+            r = dict(mask=mask, mask2=None, x_ctc=None, len_host=len_host, L=L, lengths_in=lengths,
+                     tables=table)
+            states = [] if want_states else None
+            limit, new_len = None, None
+            for li, W in enumerate(P["layers"]):
+                ctc_here = self.ctc_compress_out and self.ctc_layer == li + 1
+                if limit is None:  # transformer_layer.py:105-135 (pre-LayerNorm)
+                    h = ops.layernorm(x, *W["ln1"], out_dtype=f32, eps=W["eps1"])
+                    qkv = ops.linear_f32(h, W["wqkv"], W["bqkv"])
+                    att = ops.attention_f32(qkv, lengths, L, B, H, self.log_penalty)
+                    x = ops.linear_f32(att, W["wo"], W["bo"], residual=x)
+                    h = ops.layernorm(x, *W["ln2"], out_dtype=f32, eps=W["eps2"])
+                    f = ops.linear_f32(h, W["w1"], W["b1"], relu=True)
+                    x = ops.linear_f32(f, W["w2"], W["b2"], residual=x)
+                else:
+                    h = ops.layernorm(x, *W["ln1"], out_dtype=f32, eps=W["eps1"], out=ws["h"], rows_limit=limit)
+                    qkv = ops.linear_f32(h, W["wqkv"], W["bqkv"], out=ws["qkv"], rows_limit=limit)
+                    att = ops.attention_f32(qkv, lengths, L, B, H, self.log_penalty, out=ws["att"],
+                                            q_limit=limit[0])
+                    x1 = ops.linear_f32(att, W["wo"], W["bo"], residual=x, out=ws["x1"], rows_limit=limit)
+                    h = ops.layernorm(x1, *W["ln2"], out_dtype=f32, eps=W["eps2"], out=ws["h"], rows_limit=limit)
+                    f = ops.linear_f32(h, W["w1"], W["b1"], relu=True, out=ws["f"], rows_limit=limit)
+                    x = ops.linear_f32(f, W["w2"], W["b2"], residual=x1, out=ws["x0"], rows_limit=limit)
+                if ctc_here:
+                    if want_states:
+                        r["x_ctc"], x, lengths, len_host, L = self._ctc_compress(x, lengths, L, B)
+                        r["mask2"] = ops.lengths_to_mask(lengths, L)[0]
+                        r["len_host"], r["L"] = len_host, L
+                    else:
+                        r["x_ctc"], x, lengths, max_new = self._ctc_compress(x, lengths, L, B, out=ws["x0"])
+                        new_len = lengths
+                        limit = (max_new, B)
+                if want_states:
+                    states.append(x.view(L, B, D))
+            r.update(x=x, limit=limit, new_len=new_len, states=states)
+            return r
+
         # ------------------------------------------------------------------------- CUDA graphs
         def _graph_key(self, B, T, Fd, dev):
             hooks = tuple(sorted(self.ctc_fc._forward_hooks)) if self.ctc_compress_out else ()
             bump = None if self.ctc_logit_bump is None else (id(self.ctc_logit_bump[0]), self.ctc_logit_bump[1])
-            return (B, T, Fd, str(dev), self._prep_key, hooks, bump, self.graph_lane)
+            prep_key = self._prep32_key if self._precision == "fp32" else self._prep_key
+            return (B, T, Fd, str(dev), self._precision, prep_key, hooks, bump, self.graph_lane)
 
         def _replay(self, x_in, len_host, len_dev, B, T, Fd, L):
             """Graph mode (``use_cuda_graph``): the ~90 launches of ``_body`` for one input shape are
@@ -592,7 +731,7 @@ def make_encoder_class(base):
             length vector.  ``ctc_out`` then aliases a buffer owned by the graph: it is valid until
             the next forward with the same input shape."""
             dev = x_in.device
-            P = self._prepared()
+            P = self._prepared_active()
             key = self._graph_key(B, T, Fd, dev)
             G = self._graphs.get(key)
             if G is None:
@@ -636,13 +775,13 @@ def make_encoder_class(base):
             side = torch.cuda.Stream(dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):  # warm-up outside capture: lazy one-time initialisation
-                self._body(P, G["x"], G["lengths"], None, L, B, False, G["ws"])
+                self._run_body(P, G["x"], G["lengths"], None, L, B, False, G["ws"])
             torch.cuda.current_stream(dev).wait_stream(side)
             torch.cuda.synchronize(dev)
             graph = torch.cuda.CUDAGraph()
             n0 = ops.LAUNCHES
             with torch.cuda.graph(graph):
-                G["out"] = self._body(P, G["x"], G["lengths"], None, L, B, False, G["ws"])
+                G["out"] = self._run_body(P, G["x"], G["lengths"], None, L, B, False, G["ws"])
             G["launches"] = ops.LAUNCHES - n0
             G["graph"] = graph
             return G
@@ -653,13 +792,16 @@ def make_encoder_class(base):
             product of a partially valid key tile)."""
             D, Dff = self.embed_dim, self.layers[0].fc1.out_features
             z = lambda n, dt: torch.zeros(M, n, dtype=dt, device=dev)
+            if self._precision == "fp32":
+                f32 = torch.float32
+                return dict(h=z(D, f32), qkv=z(3 * D, f32), att=z(D, f32), f=z(Dff, f32), x0=z(D, f32), x1=z(D, f32))
             return dict(h=z(D, torch.bfloat16), qkv=z(3 * D, torch.bfloat16), att=z(D, torch.bfloat16),
                         f=z(Dff, torch.bfloat16), x0=z(D, torch.float32), x1=z(D, torch.float32),
                         st=torch.zeros(M, (D + 127) // 128, 2, dtype=torch.float32, device=dev))
 
         def _workspace(self, M, dev):
             """The eager path keeps one workspace per lane (for the last shape seen on it)."""
-            key = (M, str(dev))
+            key = (M, str(dev), self._precision)
             if self._ws is None:
                 self._ws = {}
             got = self._ws.get(self.graph_lane)
@@ -685,7 +827,7 @@ def make_encoder_class(base):
             # sum of exponentials (weighted / softmax) the 8 epilogue warps become the bottleneck (342 us against
             # 217 + 127: a tie), so those strategies keep the separate pass (scripts/bench_ctc_fc.py)
             fused = (not self.ctc_fc._forward_hooks and not self.ctc_fc._forward_pre_hooks
-                     and self.ctc_fc.logits_dtype == torch.float32 and not want_prob
+                     and self.ctc_fc.logits_dtype == torch.float32 and not want_prob and self._precision == "bf16"
                      and os.environ.get("FBKST_CTC_FUSED", "1") != "0")
             if fused:
                 # ctc_fc on tcgen05 with the arg-max (+ sum exp) folded into its epilogue: the logits are written

@@ -575,6 +575,100 @@ def prep_bn_affine(gamma, beta, mean, var, eps=1e-5):
     return scale, shift
 
 
+# ----------------------------------------------------------------- fp32-accurate path (split TF32, DESIGN F)
+def linear_f32(a, w, bias=None, relu=False, residual=None, affine=None, out=None, rows_limit=None):
+    """out = epi(a @ w.T) on the split-TF32 tensor-core GEMM.  a [M,K] fp32 (unit column stride, pitch % 4 == 0),
+    w [N,K] fp32, bias [N] fp32, affine=(scale [N], shift [N]) applied after the ReLU, residual [M,N] fp32.
+    rows_limit=(count [1] int32 device tensor, mult): only rows < count*mult are computed."""
+    lib = _lib.require_device()
+    for t, name in ((a, "a"), (w, "w")):
+        if not (t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 and t.stride(1) == 1):
+            raise ValueError("fbkst_b200.linear_f32: %s must be a 2-D CUDA fp32 tensor with unit column stride" % name)
+    M, K = a.shape
+    N = w.shape[0]
+    if w.shape[1] != K:
+        raise ValueError("fbkst_b200.linear_f32: K mismatch %s vs %s" % (tuple(a.shape), tuple(w.shape)))
+    if bias is not None:
+        _req(bias, torch.float32, "linear_f32.bias")
+    sc, sh = (None, None) if affine is None else affine
+    ldr = 0
+    if residual is not None:
+        if residual.dtype != torch.float32 or residual.stride(1) != 1 or tuple(residual.shape) != (M, N):
+            raise ValueError("fbkst_b200.linear_f32: residual must be [M, N] fp32 with unit column stride")
+        ldr = residual.stride(0)
+    if out is None:
+        ldo = (N + 3) // 4 * 4
+        out = torch.empty(M, ldo, dtype=torch.float32, device=a.device)
+        if ldo != N:
+            out = out[:, :N]
+    if out.dtype != torch.float32 or out.stride(-1) != 1 or tuple(out.shape) != (M, N):
+        raise ValueError("fbkst_b200.linear_f32: bad out tensor")
+    check(lib.fbkst_linear_tf32x3(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(sc),
+                                  _ptr(sh), _ptr(residual), ldr, out.data_ptr(), out.stride(0), M, N, K,
+                                  1 if relu else 0, _ptr(rows_limit[0]) if rows_limit else 0,
+                                  rows_limit[1] if rows_limit else 0, _stream()))
+    _count()
+    return out
+
+
+def attention_f32(qkv, lengths, L, B, H, log_penalty=True, out=None, q_limit=None):
+    """qkv [L*B, 3*H*64] fp32 (row t*B+b, q pre-scaled) -> [L*B, H*64] fp32 on split-TF32 tensor cores.
+    ``q_limit`` as in ``attention``."""
+    lib = _lib.require_device()
+    _req(qkv, torch.float32, "attention_f32.qkv"); _req(lengths, torch.int32, "attention_f32.lengths")
+    if qkv.shape != (L * B, 3 * H * 64):
+        raise ValueError("fbkst_b200.attention_f32: qkv shape %s != (%d, %d)" %
+                         (tuple(qkv.shape), L * B, 3 * H * 64))
+    if out is None:
+        out = torch.empty(L * B, H * 64, dtype=torch.float32, device=qkv.device)
+    _req(out, torch.float32, "attention_f32.out")
+    if q_limit is not None:
+        _req(q_limit, torch.int32, "attention_f32.q_limit")
+    check(lib.fbkst_attention_tf32x3(qkv.data_ptr(), out.data_ptr(), lengths.data_ptr(), L, B, H,
+                                     1 if log_penalty else 0, _ptr(q_limit), _stream()))
+    _count()
+    return out
+
+
+def conv1_relu_bn_f32(x, w, bias, scale, shift):
+    """x [B,T,F] fp32, w [C,9] fp32 -> y [B,T1,F1,C] fp32 = BN(ReLU(conv1(x)))."""
+    lib = _lib.require_device()
+    _req(x, torch.float32, "conv1_f32.x"); _req(w, torch.float32, "conv1_f32.w")
+    B, T, Fd = x.shape
+    C = w.shape[0]
+    y = torch.empty(B, (T + 1) // 2, (Fd + 1) // 2, C, dtype=torch.float32, device=x.device)
+    check(lib.fbkst_conv1_relu_bn_f32(x.data_ptr(), w.data_ptr(), bias.data_ptr(), scale.data_ptr(),
+                                      shift.data_ptr(), y.data_ptr(), B, T, Fd, C, _stream()))
+    _count()
+    return y
+
+
+def conv2_relu_bn_f32(y1, w2, bias, scale, shift):
+    """y1 [B,T1,F1,C] fp32 -> [B,T2,F2,C] fp32 = BN(ReLU(conv2(y1))): fp32 patches (im2col), then the split-TF32
+    GEMM with ``w2`` [C, 9*C] from ``prep_conv2_weight_f32``."""
+    lib = _lib.require_device()
+    _req(y1, torch.float32, "conv2_f32.y1")
+    B, T1, F1, C = y1.shape
+    T2, F2 = (T1 + 1) // 2, (F1 + 1) // 2
+    col = torch.empty(B * T2 * F2, 9 * C, dtype=torch.float32, device=y1.device)
+    check(lib.fbkst_conv2_im2col_f32(y1.data_ptr(), col.data_ptr(), B, T1, F1, C, _stream()))
+    _count()
+    y = linear_f32(col, w2, bias, relu=True, affine=(scale, shift))
+    return y.view(B, T2, F2, C)
+
+
+def prep_conv2_weight_f32(w):
+    """conv2 weight [C,C,3,3] -> [C, 9*C] fp32, column (kt*3 + kf)*C + c (the patch order of conv2_relu_bn_f32)."""
+    C = w.shape[0]
+    return w.detach().float().permute(0, 2, 3, 1).reshape(C, 9 * C).contiguous()
+
+
+def prep_fc3_weight_f32(w, C, F2):
+    """fc3 weight [D, C*F2] (reference flatten c*F2+f) -> [D, F2*C] fp32 (channels-last flatten f*C+c)."""
+    D = w.shape[0]
+    return w.detach().float().view(D, C, F2).permute(0, 2, 1).reshape(D, F2 * C).contiguous()
+
+
 # ------------------------------------------------------------------------------------- training side
 # Batched launches: the job tables of fbkst_reduce_sum_batch / fbkst_prep_batch are packed HOST arrays of the
 # structs declared in include/fbkst_b200.h (fbkst_reduce_desc_t: 56 bytes, fbkst_prep_desc_t: 64 bytes).

@@ -42,7 +42,7 @@ class EncoderPipeline:
         self._n_in = self.lanes + 2
         self._consumed = [None] * self._n_in  # event: CMVN / encoder finished reading input slot
         with torch.cuda.device(self.device):
-            encoder._prepared()  # derive the operand formats once, before any lane uses them
+            encoder._prepared_active()  # derive the operand formats once, before any lane uses them
             torch.cuda.synchronize(self.device)
 
     def _in_buffer(self, slot, shape):

@@ -64,6 +64,7 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
         encoder = B200ConvolutionalTransformerEncoder(
             args, src_dict if src_dict is not None else tgt_dict,
             audio_features=args.input_feat_per_channel)
+        encoder.precision = getattr(args, "b200_precision", "bf16") or "bf16"
         decoder = TransformerDecoder(args, tgt_dict, emb)
         # SURVEY 8f N4: encoder-decoder attention on the device kernel (K/V once per utterance, beam
         # reorders move an index vector).  Same parameters / state_dict keys; inference only, so it
@@ -82,6 +83,10 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
         parser.add_argument("--b200-lazy-beam-reorder", action="store_true",
                             help="with --b200-cross-attention: never replicate the encoder output "
                                  "x beam (reorder_encoder_out returns tagged aliases)")
+        parser.add_argument("--b200-precision", choices=["bf16", "fp32"], default="bf16",
+                            help="encoder operand precision at inference: bf16 tensor-core operands (default) "
+                                 "or fp32 on split-TF32 tensor cores (within 1e-3 of an fp32 reference; "
+                                 "inference only)")
 
 
 # ---------------------------------------------------------------------------------------------------

@@ -55,6 +55,10 @@ _def("linear(Tensor a, Tensor w, Tensor? bias, bool relu, Tensor? residual, bool
 _def("layernorm(Tensor x, Tensor gamma, Tensor beta, bool out_f32, float eps) -> Tensor", _layernorm)
 _def("attention(Tensor qkv, Tensor lengths, int L, int B, int H, bool log_penalty) -> Tensor",
      lambda qkv, lengths, L, B, H, log_penalty: ops.attention(qkv, lengths, L, B, H, log_penalty))
+_def("linear_f32(Tensor a, Tensor w, Tensor? bias, bool relu, Tensor? residual) -> Tensor",
+     lambda a, w, bias, relu, residual: ops.linear_f32(a, w, bias, relu=relu, residual=residual))
+_def("attention_f32(Tensor qkv, Tensor lengths, int L, int B, int H, bool log_penalty) -> Tensor",
+     lambda qkv, lengths, L, B, H, log_penalty: ops.attention_f32(qkv, lengths, L, B, H, log_penalty))
 _def("ctc_argmax(Tensor logits, Tensor lengths, int L, int B, int V, bool want_prob) -> (Tensor, Tensor)",
      _ctc_argmax)
 _def("ctc_segment(Tensor labels, Tensor? top_prob, Tensor lengths, str strategy, int L, int B)"
@@ -77,5 +81,6 @@ def _xattn(q, kv, mask, row_map, tgt_len, H, weights):
 _def("xattn(Tensor q, Tensor kv, Tensor? mask, Tensor row_map, int tgt_len, int H, int weights)"
      " -> (Tensor, Tensor)", _xattn)
 
-OPS = ["cmvn", "conv1_relu_bn", "conv2_relu_bn", "linear", "layernorm", "attention", "ctc_argmax",
+OPS = ["cmvn", "conv1_relu_bn", "conv2_relu_bn", "linear", "layernorm", "attention", "linear_f32",
+       "attention_f32", "ctc_argmax",
        "ctc_segment", "ctc_compress", "lengths_to_mask", "xattn"]

@@ -178,6 +178,35 @@ int fbkst_attention_fwd(const void* qkv, void* out, const int32_t* lengths, int 
 int fbkst_attention_fwd_limited(const void* qkv, void* out, const int32_t* lengths, int L, int B, int H,
                                 int log_penalty, const int32_t* q_limit, fbkst_stream_t stream);
 
+/* ---- F: fp32-accurate inference path (encoder.precision = "fp32"), split-TF32 tensor-core kernels -------
+ * Every operand x is split in shared memory into hi = tf32(x) (rounded) and lo = tf32(x - hi); products are
+ * hi.hi + hi.lo + lo.hi in one fp32 accumulator (about 21 significant bits per operand; fp32 in HBM).
+ *
+ * Linear: replaces every F.linear / nn.Linear on the fp32 path (conv_transformer.py:227,279;
+ * local_attention.py:178,141; transformer_layer.py:131-133) and conv2 over fbkst_conv2_im2col_f32
+ * (conv_transformer.py:205-212).  A [M,K] fp32 (pitch lda), W [N,K] fp32 (pitch ldw), K, lda, ldw % 4 == 0.
+ * y = A W^T + bias; ReLU if relu; y = y * col_scale[n] + col_shift[n] if col_scale (eval BatchNorm after the
+ * ReLU); y += residual[m, n] (pitch ldr) if residual.  out [M, N] fp32 (pitch ldo).  m_limit (device int32 [1]
+ * or NULL): only rows m < *m_limit * m_limit_mult are computed (the layers after CTC compression). */
+int fbkst_linear_tf32x3(const float* A, int64_t lda, const float* W, int64_t ldw, const float* bias,
+                        const float* col_scale, const float* col_shift, const float* residual, int64_t ldr,
+                        float* out, int64_t ldo, int M, int N, int K, int relu, const int32_t* m_limit,
+                        int m_limit_mult, fbkst_stream_t stream);
+/* Attention: replaces local_attention.py:115-139 (log_penalty = 1) and the math of
+ * F.multi_head_attention_forward (log_penalty = 0) as fbkst_attention_fwd does, in fp32: qkv [L*B, 3D] fp32
+ * (q pre-scaled by head_dim^-0.5), out [L*B, D] fp32, H <= 16, fp32 softmax.  Query rows of 128-row tiles
+ * entirely beyond lengths[b] are zero; with q_limit (device int32 [1] or NULL) tiles starting at or beyond
+ * *q_limit are left untouched. */
+int fbkst_attention_tf32x3(const float* qkv, float* out, const int32_t* lengths, int L, int B, int H,
+                           int log_penalty, const int32_t* q_limit, fbkst_stream_t stream);
+/* conv1 + ReLU + eval BatchNorm in fp32 (conv_transformer.py:205-212, first convolution): x [B,T,F] fp32,
+ * w [C,9] fp32 -> y [B,T1,F1,C] fp32 channels-last. */
+int fbkst_conv1_relu_bn_f32(const float* x, const float* w, const float* bias, const float* bn_scale,
+                            const float* bn_shift, float* y, int B, int T, int F, int C, fbkst_stream_t stream);
+/* conv2's patches: y1 [B,T1,F1,C] fp32 -> col [B*T2*F2, 9*C] fp32, column (kt*3 + kf)*C + c, zero padding 1,
+ * stride 2.  C % 4 == 0. */
+int fbkst_conv2_im2col_f32(const float* y1, float* col, int B, int T1, int F1, int C, fbkst_stream_t stream);
+
 /* ---- a4: sinusoidal position table (row 0 = zeros) ---------------------------------------
  * replaces fairseq/modules/sinusoidal_positional_embedding.py:36-58.  table [rows, D] fp32. */
 int fbkst_sinusoidal_table(float* table, int rows, int D, fbkst_stream_t stream);
