@@ -5,7 +5,7 @@
 // sequence_generator.py:193-198) and re-gathered by reorder_incremental_state (:407-420).
 //
 // Here K and V are projected ONCE per utterance (not per beam hypothesis) into one time-major
-// bf16 buffer kv [S, U, 2D]; every hypothesis row carries an index into it (row_map), so beam
+// buffer kv [S, U, 2D]; every hypothesis row carries an index into it (row_map), so beam
 // replication and beam reordering are a gather of B*beam int32 values instead of copies of
 // B*beam*H*S*64 elements per layer.  The kernel is HBM/L2-bound byte work (q.K^T and p.V for ONE
 // query per row: 4 flop per K/V byte): no tensor cores, 16-byte loads, fp32 softmax.
@@ -14,14 +14,19 @@
 //          ALL of them (x tgt_len queries each) from one pass over K_h and V_h of the utterance, in
 //          chunks of 8 query rows: the K/V bytes are read once per chunk instead of once per row
 //          (beam 5 -> 5x less L2 traffic than a CTA per row, and U*H CTAs fill the 148 SMs).
-//   scores  lane <-> key: a lane pulls whole 128-byte K rows (8 x LDG.128) into registers and dots
-//           them with the (up to) 8 queries of the chunk, broadcast from shared memory
+//   scores  lane <-> key: a lane pulls a whole K row (bf16: 128 bytes, 8 x LDG.128; fp32: 256 bytes,
+//           16 x LDG.128) into registers as 64 floats and dots it with the (up to) 8 queries of the
+//           chunk, broadcast from shared memory
 //   softmax fp32, warp <-> query row, probabilities stay in shared memory ([S][8] floats)
-//   p.V     lane <-> two output dims, the 8 warps split the keys (a warp reads one coalesced 128-byte
-//           V row per key), partial sums reduced through shared memory in a fixed order
+//   p.V     lane <-> two output dims, the 8 warps split the keys (a warp reads one coalesced V row
+//           per key), partial sums reduced through shared memory in a fixed order
 //   weights per head straight from shared memory; the head average the reference returns
 //           (multihead_attention.py:355-362) is a second tiny kernel over the per-head buffer, so the
 //           summation order over heads is fixed (no atomics).
+//
+// One kernel body serves both operand types (template on the element type T): bf16 q / kv / out
+// (fbkst_xattn_fwd) and fp32 (fbkst_xattn_fwd_f32, the fp32-accurate decode path).  Only the loads
+// and stores differ; arithmetic and summation order are the same fp32 FMAs for both.
 #include <math.h>
 
 #include <cuda_bf16.h>
@@ -42,6 +47,41 @@ constexpr int XA_SCAN = 1024;  // hypothesis rows scanned per list refill
 __device__ __forceinline__ float bf16_lo(uint32_t v) { return __uint_as_float(v << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t v) { return __uint_as_float(v & 0xffff0000u); }
 
+// two consecutive elements (8-byte aligned for fp32, 4-byte for bf16) as floats
+__device__ __forceinline__ float2 xa_ld2(const __nv_bfloat16* p) {
+  const uint32_t w = __ldg(reinterpret_cast<const uint32_t*>(p));
+  return make_float2(bf16_lo(w), bf16_hi(w));
+}
+__device__ __forceinline__ float2 xa_ld2(const float* p) { return __ldg(reinterpret_cast<const float2*>(p)); }
+
+__device__ __forceinline__ void xa_st2(__nv_bfloat16* p, float2 v) {
+  *reinterpret_cast<__nv_bfloat162*>(p) = __floats2bfloat162_rn(v.x, v.y);
+}
+__device__ __forceinline__ void xa_st2(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+
+// one 64-element head row (16-byte aligned) -> kf[64]
+__device__ __forceinline__ void xa_ld_row(const __nv_bfloat16* p, float (&kf)[XA_HD]) {
+  const uint4* kp = reinterpret_cast<const uint4*>(p);
+  uint4 kr[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) kr[i] = __ldg(kp + i);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    kf[8 * i + 0] = bf16_lo(kr[i].x); kf[8 * i + 1] = bf16_hi(kr[i].x);
+    kf[8 * i + 2] = bf16_lo(kr[i].y); kf[8 * i + 3] = bf16_hi(kr[i].y);
+    kf[8 * i + 4] = bf16_lo(kr[i].z); kf[8 * i + 5] = bf16_hi(kr[i].z);
+    kf[8 * i + 6] = bf16_lo(kr[i].w); kf[8 * i + 7] = bf16_hi(kr[i].w);
+  }
+}
+__device__ __forceinline__ void xa_ld_row(const float* p, float (&kf)[XA_HD]) {
+  const float4* kp = reinterpret_cast<const float4*>(p);
+#pragma unroll
+  for (int i = 0; i < XA_HD / 4; ++i) {
+    const float4 v = __ldg(kp + i);
+    kf[4 * i + 0] = v.x; kf[4 * i + 1] = v.y; kf[4 * i + 2] = v.z; kf[4 * i + 3] = v.w;
+  }
+}
+
 static inline size_t xattn_smem_bytes(int S) {
   return sizeof(int) * (XA_SCAN + 4) + sizeof(float) * (XA_RC * XA_HD + XA_WARPS * XA_RC * XA_HD + XA_RC) +
          sizeof(float) * (size_t)S * XA_RC;
@@ -49,11 +89,12 @@ static inline size_t xattn_smem_bytes(int S) {
 
 // A hypothesis row whose map entry is outside [0, U) belongs to no CTA: the CTAs of utterance 0 give
 // it defined zeros (rare path, kept out of line).
-__device__ __noinline__ void xattn_zero_row(__nv_bfloat16* out, float* attn_w, int b, int h, int S, int bsz,
-                                            int tgt_len, int D) {
+template <typename T>
+__device__ __noinline__ void xattn_zero_row(T* out, float* attn_w, int b, int h, int S, int bsz, int tgt_len,
+                                            int D) {
   for (int t = 0; t < tgt_len; ++t) {
     uint4* o = reinterpret_cast<uint4*>(out + ((size_t)t * bsz + b) * D + h * XA_HD);
-    for (int c = 0; c < 8; ++c) o[c] = make_uint4(0u, 0u, 0u, 0u);
+    for (int c = 0; c < XA_HD * (int)sizeof(T) / 16; ++c) o[c] = make_uint4(0u, 0u, 0u, 0u);
     if (attn_w != nullptr) {
       float* w = attn_w + (((size_t)h * bsz + b) * tgt_len + t) * S;
       for (int k = 0; k < S; ++k) w[k] = 0.0f;
@@ -61,11 +102,11 @@ __device__ __noinline__ void xattn_zero_row(__nv_bfloat16* out, float* attn_w, i
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(XA_THREADS)
-    xattn_fwd_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ kv,
-                     const uint8_t* __restrict__ mask, const int* __restrict__ row_map,
-                     __nv_bfloat16* __restrict__ out, float* __restrict__ attn_w, int S, int U, int bsz,
-                     int tgt_len, int H) {
+    xattn_fwd_kernel(const T* __restrict__ q, const T* __restrict__ kv, const uint8_t* __restrict__ mask,
+                     const int* __restrict__ row_map, T* __restrict__ out, float* __restrict__ attn_w, int S,
+                     int U, int bsz, int tgt_len, int H) {
   extern __shared__ __align__(16) uint8_t xa_raw[];
   int* s_list = reinterpret_cast<int*>(xa_raw);                 // [XA_SCAN] hypothesis rows of this utterance
   int* s_n = s_list + XA_SCAN;                                  // [4]
@@ -77,16 +118,19 @@ __global__ void __launch_bounds__(XA_THREADS)
   const int u = blockIdx.x / H, h = blockIdx.x - u * H;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const size_t row_stride = (size_t)U * 2 * D;  // elements between consecutive keys
-  const __nv_bfloat16* kbase = kv + (size_t)u * 2 * D + h * XA_HD;
+  const T* kbase = kv + (size_t)u * 2 * D + h * XA_HD;
   const uint8_t* mrow = mask ? mask + (size_t)u * S : nullptr;
 
-  // Pull this CTA's K_h and V_h rows (128 bytes per key each) towards L2 now: they do not depend on
-  // the row list, and every later phase is a chain of dependent round trips (scan -> queries ->
-  // K -> softmax -> V) that would otherwise each pay HBM latency.
+  // Pull this CTA's K_h and V_h rows (128 or 256 bytes per key each) towards L2 now: they do not
+  // depend on the row list, and every later phase is a chain of dependent round trips (scan ->
+  // queries -> K -> softmax -> V) that would otherwise each pay HBM latency.
   for (int s = tid; s < S; s += XA_THREADS) {
-    const __nv_bfloat16* kp = kbase + (size_t)s * row_stride;
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(kp));
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(kp + D));
+    const T* kp = kbase + (size_t)s * row_stride;
+#pragma unroll
+    for (int c = 0; c < XA_HD * (int)sizeof(T); c += 128) {  // one prefetch per 128-byte line
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(kp) + c));
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(kp + D) + c));
+    }
   }
   for (int b0 = 0; b0 < bsz; b0 += XA_SCAN) {
     // ---- hypothesis rows of this utterance in [b0, b0 + XA_SCAN)
@@ -104,7 +148,7 @@ __global__ void __launch_bounds__(XA_THREADS)
       const int b = b0 + i + tid;
       const int rm = rms[k];
       const bool hit = rm == u;
-      if (u == 0 && b < bsz && (rm < 0 || rm >= U)) xattn_zero_row(out, attn_w, b, h, S, bsz, tgt_len, D);
+      if (u == 0 && b < bsz && (rm < 0 || rm >= U)) xattn_zero_row<T>(out, attn_w, b, h, S, bsz, tgt_len, D);
       const unsigned bal = __ballot_sync(0xffffffffu, hit);
       // the order of the list is irrelevant: every row is computed independently of its chunk mates
       int base = 0;
@@ -124,26 +168,15 @@ __global__ void __launch_bounds__(XA_THREADS)
         if (j < nr) {
           const int idx = r0 + j;
           const int b = s_list[idx / tgt_len], t = idx % tgt_len;
-          const uint32_t w = __ldg(reinterpret_cast<const uint32_t*>(q + ((size_t)t * bsz + b) * D + h * XA_HD) + c);
-          v = make_float2(bf16_lo(w), bf16_hi(w));
+          v = xa_ld2(q + ((size_t)t * bsz + b) * D + h * XA_HD + 2 * c);
         }
         reinterpret_cast<float2*>(s_q)[i] = v;
       }
       __syncthreads();
       // ---- scores: lane <-> key
       for (int s = warp * 32 + lane; s < S; s += XA_THREADS) {
-        const uint4* kp = reinterpret_cast<const uint4*>(kbase + (size_t)s * row_stride);
-        uint4 kr[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) kr[i] = __ldg(kp + i);
         float kf[XA_HD];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          kf[8 * i + 0] = bf16_lo(kr[i].x); kf[8 * i + 1] = bf16_hi(kr[i].x);
-          kf[8 * i + 2] = bf16_lo(kr[i].y); kf[8 * i + 3] = bf16_hi(kr[i].y);
-          kf[8 * i + 4] = bf16_lo(kr[i].z); kf[8 * i + 5] = bf16_hi(kr[i].z);
-          kf[8 * i + 6] = bf16_lo(kr[i].w); kf[8 * i + 7] = bf16_hi(kr[i].w);
-        }
+        xa_ld_row(kbase + (size_t)s * row_stride, kf);
         const bool masked = mrow && mrow[s];  // multihead_attention.py:330-335
         // rolled over the rows on purpose: every CTA runs this code once, cold -- the fully unrolled
         // version (6k instructions) spent its time in instruction fetch (profiles/r01f_ncu_xattn_v2_unrolled.txt)
@@ -188,21 +221,20 @@ __global__ void __launch_bounds__(XA_THREADS)
       __syncthreads();
       // ---- p.V: lane <-> output dims (2 * lane, 2 * lane + 1); warp w takes keys w, w + 4, ...
       {
-        const uint32_t* vbase = reinterpret_cast<const uint32_t*>(kbase + D) + lane;
-        const size_t vstride = row_stride / 2;  // in 32-bit words
+        const T* vbase = kbase + D + 2 * lane;
         float acc[XA_RC][2];
 #pragma unroll
         for (int j = 0; j < XA_RC; ++j) acc[j][0] = acc[j][1] = 0.0f;
         int s = warp;
         for (; s + 7 * XA_WARPS < S; s += 8 * XA_WARPS) {
-          uint32_t vv[8];
+          float2 vv[8];
 #pragma unroll
-          for (int i = 0; i < 8; ++i) vv[i] = __ldg(vbase + (size_t)(s + i * XA_WARPS) * vstride);
+          for (int i = 0; i < 8; ++i) vv[i] = xa_ld2(vbase + (size_t)(s + i * XA_WARPS) * row_stride);
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
             const float4* pp = reinterpret_cast<const float4*>(s_p + (size_t)(s + i * XA_WARPS) * XA_RC);
             const float4 p0 = pp[0], p1 = pp[1];  // broadcast
-            const float v0 = bf16_lo(vv[i]), v1 = bf16_hi(vv[i]);
+            const float v0 = vv[i].x, v1 = vv[i].y;
             acc[0][0] = fmaf(p0.x, v0, acc[0][0]); acc[0][1] = fmaf(p0.x, v1, acc[0][1]);
             acc[1][0] = fmaf(p0.y, v0, acc[1][0]); acc[1][1] = fmaf(p0.y, v1, acc[1][1]);
             acc[2][0] = fmaf(p0.z, v0, acc[2][0]); acc[2][1] = fmaf(p0.z, v1, acc[2][1]);
@@ -214,10 +246,10 @@ __global__ void __launch_bounds__(XA_THREADS)
           }
         }
         for (; s < S; s += XA_WARPS) {
-          const uint32_t v = __ldg(vbase + (size_t)s * vstride);
+          const float2 v = xa_ld2(vbase + (size_t)s * row_stride);
           const float4* pp = reinterpret_cast<const float4*>(s_p + (size_t)s * XA_RC);
           const float4 p0 = pp[0], p1 = pp[1];
-          const float v0 = bf16_lo(v), v1 = bf16_hi(v);
+          const float v0 = v.x, v1 = v.y;
           acc[0][0] = fmaf(p0.x, v0, acc[0][0]); acc[0][1] = fmaf(p0.x, v1, acc[0][1]);
           acc[1][0] = fmaf(p0.y, v0, acc[1][0]); acc[1][1] = fmaf(p0.y, v1, acc[1][1]);
           acc[2][0] = fmaf(p0.z, v0, acc[2][0]); acc[2][1] = fmaf(p0.z, v1, acc[2][1]);
@@ -232,7 +264,7 @@ __global__ void __launch_bounds__(XA_THREADS)
           reinterpret_cast<float2*>(s_red + (warp * XA_RC + j) * XA_HD)[lane] = make_float2(acc[j][0], acc[j][1]);
       }
       __syncthreads();
-      // ---- outputs: fixed-order sum over the 4 warps, 1 / row sum, bf16
+      // ---- outputs: fixed-order sum over the warps, 1 / row sum, stored as T
       for (int i = tid; i < nr * (XA_HD / 2); i += XA_THREADS) {
         const int j = i / (XA_HD / 2), c = i - j * (XA_HD / 2);
         float2 a = make_float2(0.f, 0.f);
@@ -245,8 +277,7 @@ __global__ void __launch_bounds__(XA_THREADS)
         const float inv = s_inv[j];
         const int idx = r0 + j;
         const int b = s_list[idx / tgt_len], t = idx % tgt_len;
-        reinterpret_cast<__nv_bfloat162*>(out + ((size_t)t * bsz + b) * D + h * XA_HD)[c] =
-            __floats2bfloat162_rn(a.x * inv, a.y * inv);
+        xa_st2(out + ((size_t)t * bsz + b) * D + h * XA_HD + 2 * c, make_float2(a.x * inv, a.y * inv));
       }
       if (attn_w != nullptr) {  // per-head weights [H, bsz, tgt_len, S]
         for (int j = 0; j < nr; ++j) {
@@ -273,35 +304,35 @@ __global__ void xattn_head_mean_kernel(const float* __restrict__ per_head, float
   }
 }
 
-}  // namespace fbkst
-
-extern "C" int fbkst_xattn_fwd(const void* q, const void* kv, const uint8_t* key_padding_mask,
-                               const int32_t* row_map, void* out, float* attn_w, float* head_ws, int w_mode,
-                               int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream) {
-  using namespace fbkst;
-  FBKST_REQUIRE(q && kv && row_map && out, "xattn_fwd: null pointer");
-  FBKST_REQUIRE(S >= 1 && U >= 1 && bsz >= 1 && tgt_len >= 1, "xattn_fwd: empty problem (S=%d U=%d bsz=%d tgt_len=%d)",
-                S, U, bsz, tgt_len);
-  FBKST_REQUIRE(H >= 1 && H <= 16, "xattn_fwd: heads must be in [1,16] (head_dim is 64), got %d", H);
-  FBKST_REQUIRE(w_mode >= 0 && w_mode <= 2 && (w_mode == 0 || attn_w), "xattn_fwd: bad attention-weight mode");
-  FBKST_REQUIRE(w_mode != 1 || head_ws, "xattn_fwd: head-averaged weights need the [H, bsz, tgt_len, S] workspace");
-  FBKST_REQUIRE((reinterpret_cast<uintptr_t>(q) & 3) == 0 && (reinterpret_cast<uintptr_t>(kv) & 15) == 0 &&
-                    (reinterpret_cast<uintptr_t>(out) & 15) == 0,
-                "xattn_fwd: kv and out must be 16-byte aligned");
+// The launch behind both entry points: T is the element type of q, kv and out.
+template <typename T>
+int xattn_launch(const char* name, const void* q, const void* kv, const uint8_t* key_padding_mask,
+                 const int32_t* row_map, void* out, float* attn_w, float* head_ws, int w_mode, int S, int U,
+                 int bsz, int tgt_len, int H, fbkst_stream_t stream) {
+  FBKST_REQUIRE(q && kv && row_map && out, "%s: null pointer", name);
+  FBKST_REQUIRE(S >= 1 && U >= 1 && bsz >= 1 && tgt_len >= 1, "%s: empty problem (S=%d U=%d bsz=%d tgt_len=%d)",
+                name, S, U, bsz, tgt_len);
+  FBKST_REQUIRE(H >= 1 && H <= 16, "%s: heads must be in [1,16] (head_dim is 64), got %d", name, H);
+  FBKST_REQUIRE(w_mode >= 0 && w_mode <= 2 && (w_mode == 0 || attn_w), "%s: bad attention-weight mode", name);
+  FBKST_REQUIRE(w_mode != 1 || head_ws, "%s: head-averaged weights need the [H, bsz, tgt_len, S] workspace", name);
+  FBKST_REQUIRE((reinterpret_cast<uintptr_t>(q) & (2 * sizeof(T) - 1)) == 0 &&
+                    (reinterpret_cast<uintptr_t>(kv) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
+                "%s: q must be aligned to two elements, kv and out to 16 bytes", name);
   const size_t smem = xattn_smem_bytes(S);
-  FBKST_REQUIRE(smem <= 200 * 1024, "xattn_fwd: src_len %d too long (scores of 8 rows must fit in shared memory)", S);
-  static PerDeviceFlag configured;
+  FBKST_REQUIRE(smem <= 200 * 1024, "%s: src_len %d too long (scores of 8 rows must fit in shared memory)", name, S);
+  static PerDeviceFlag configured;  // one per instantiation
   if (smem > 48 * 1024 && !configured) {
-    FBKST_CHECK_CUDA(cudaFuncSetAttribute(xattn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    FBKST_CHECK_CUDA(
+        cudaFuncSetAttribute(xattn_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     configured = true;
   }
   const long long rows = (long long)bsz * tgt_len, ctas = (long long)U * H;
-  FBKST_REQUIRE(rows <= 0x7fffffffLL && ctas <= 0x7fffffffLL, "xattn_fwd: problem too large");
+  FBKST_REQUIRE(rows <= 0x7fffffffLL && ctas <= 0x7fffffffLL, "%s: problem too large", name);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* per_head = w_mode == 2 ? attn_w : (w_mode == 1 ? head_ws : nullptr);
-  xattn_fwd_kernel<<<(unsigned)ctas, XA_THREADS, smem, st>>>(
-      static_cast<const __nv_bfloat16*>(q), static_cast<const __nv_bfloat16*>(kv), key_padding_mask, row_map,
-      static_cast<__nv_bfloat16*>(out), per_head, S, U, bsz, tgt_len, H);
+  xattn_fwd_kernel<T><<<(unsigned)ctas, XA_THREADS, smem, st>>>(static_cast<const T*>(q), static_cast<const T*>(kv),
+                                                                key_padding_mask, row_map, static_cast<T*>(out),
+                                                                per_head, S, U, bsz, tgt_len, H);
   if (w_mode == 1) {
     const size_t n = (size_t)rows * S;
     const unsigned grid = (unsigned)((n + 255) / 256 < 1184 ? (n + 255) / 256 : 1184);
@@ -309,4 +340,20 @@ extern "C" int fbkst_xattn_fwd(const void* q, const void* kv, const uint8_t* key
   }
   FBKST_CHECK_CUDA(cudaGetLastError());
   return 0;
+}
+
+}  // namespace fbkst
+
+extern "C" int fbkst_xattn_fwd(const void* q, const void* kv, const uint8_t* key_padding_mask,
+                               const int32_t* row_map, void* out, float* attn_w, float* head_ws, int w_mode,
+                               int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream) {
+  return fbkst::xattn_launch<__nv_bfloat16>("xattn_fwd", q, kv, key_padding_mask, row_map, out, attn_w, head_ws,
+                                            w_mode, S, U, bsz, tgt_len, H, stream);
+}
+
+extern "C" int fbkst_xattn_fwd_f32(const float* q, const float* kv, const uint8_t* key_padding_mask,
+                                   const int32_t* row_map, float* out, float* attn_w, float* head_ws, int w_mode,
+                                   int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream) {
+  return fbkst::xattn_launch<float>("xattn_fwd_f32", q, kv, key_padding_mask, row_map, out, attn_w, head_ws,
+                                    w_mode, S, U, bsz, tgt_len, H, stream);
 }

@@ -44,6 +44,7 @@ SIGNATURES = {
     "fbkst_specaugment_f32": [P, P, I, I, I, I, I, P],
     "fbkst_time_stretch_f32": [P, P, I, P, P, I, I, I, I, P],
     "fbkst_xattn_fwd": [P, P, P, P, P, P, P, I, I, I, I, I, I, P],
+    "fbkst_xattn_fwd_f32": [P, P, P, P, P, P, P, I, I, I, I, I, I, P],
     "fbkst_cast_bf16": [P, P, I64, F, P],
     "fbkst_prep_conv2_weight": [P, P, I, P],
     "fbkst_prep_fc3_weight": [P, P, I, I, I, P],

@@ -18,6 +18,10 @@ What changes is the data path:
   * scores, key-padding mask, fp32 softmax, P.V and the head-averaged weights are one kernel
     (``fbkst_xattn_fwd``); q/out projections are the tcgen05 linear kernel.
 
+``precision = "fp32"`` keeps every operand in fp32 instead: the K/V, q and out projections run on the
+split-TF32 GEMM (``ops.linear_f32``) and the core on ``fbkst_xattn_fwd_f32``, the same kernel on fp32
+operands; the cached K/V is then ``[S, U, 2D]`` fp32.
+
 The replication is recognised through tags the encoder's ``reorder_encoder_out`` leaves on the tensors
 it returns (``beam_source`` below); an untagged ``key`` is simply treated as U = bsz utterances.
 There is no CPU / PyTorch fallback, and no backward: training-mode calls with grad enabled raise.
@@ -31,6 +35,7 @@ import torch.nn as nn
 from torch import Tensor
 
 from . import ops
+from .encoder import PRECISIONS
 
 
 # ------------------------------------------------------------------ beam tags on encoder outputs
@@ -106,6 +111,22 @@ class CrossAttention(nn.Module):
         self._incremental_state_id = str(uuid.uuid4())  # incremental_decoding_utils.py:18-19
         self._prep = None
         self._prep_key = None
+        self._prep32 = None
+        self._prep32_key = None
+        self._precision = "bf16"
+
+    @property
+    def precision(self):
+        """Operand precision of the forward: ``"bf16"`` (default; bf16 tensor-core projections and bf16 K/V,
+        q and head outputs) or ``"fp32"`` (split-TF32 projections and an fp32 core: within 1e-3 of an fp32
+        reference).  An incremental cache is only valid under the precision it was built with."""
+        return self._precision
+
+    @precision.setter
+    def precision(self, value):
+        if value not in PRECISIONS:
+            raise ValueError("fbkst_b200: precision must be one of %s, got %r" % (PRECISIONS, value))
+        self._precision = value
 
     def reset_parameters(self):
         """multihead_attention.py:88-106"""
@@ -119,9 +140,11 @@ class CrossAttention(nn.Module):
         nn.init.constant_(self.out_proj.bias, 0.0)
 
     # -------------------------------------------------------------- derived operand formats
+    def _params_key(self):
+        return tuple((p._version, p.data_ptr()) for p in self.parameters())
+
     def _prepared(self):
-        params = list(self.parameters())
-        key = tuple((p._version, p.data_ptr()) for p in params)
+        key = self._params_key()
         if self._prep_key != key:
             with torch.no_grad():
                 f = lambda t: t.detach().float().contiguous()
@@ -134,6 +157,19 @@ class CrossAttention(nn.Module):
                     wo=ops.cast_bf16(f(self.out_proj.weight)), bo=f(self.out_proj.bias))
             self._prep_key = key
         return self._prep
+
+    def _prepared_f32(self):
+        key = self._params_key()
+        if self._prep32_key != key:
+            with torch.no_grad():
+                f = lambda t: t.detach().float().contiguous()
+                self._prep32 = dict(
+                    wkv=torch.cat([f(self.k_proj.weight), f(self.v_proj.weight)], 0),
+                    bkv=torch.cat([f(self.k_proj.bias), f(self.v_proj.bias)], 0),
+                    wq=f(self.q_proj.weight) * self.scaling, bq=f(self.q_proj.bias) * self.scaling,
+                    wo=f(self.out_proj.weight), bo=f(self.out_proj.bias))
+            self._prep32_key = key
+        return self._prep32
 
     # ------------------------------------------------------------------ incremental state
     def _full_key(self):
@@ -179,10 +215,15 @@ class CrossAttention(nn.Module):
         S, U, kd = base.shape
         if kd != self.kdim:
             raise ValueError("fbkst_b200.CrossAttention: key feature size %d != kdim %d" % (kd, self.kdim))
-        P = self._prepared()
         a = base.reshape(S * U, kd)
-        a = ops.cast_bf16(a.float().contiguous()) if a.dtype != torch.bfloat16 else a.contiguous()
-        kv = ops.linear(a, P["wkv"], P["bkv"]).view(S, U, 2 * self.embed_dim)
+        if self._precision == "fp32":
+            P = self._prepared_f32()
+            kv = ops.linear_f32(a.float().contiguous(), P["wkv"], P["bkv"])
+        else:
+            P = self._prepared()
+            a = ops.cast_bf16(a.float().contiguous()) if a.dtype != torch.bfloat16 else a.contiguous()
+            kv = ops.linear(a, P["wkv"], P["bkv"])
+        kv = kv.view(S, U, 2 * self.embed_dim)
         if rows is None:
             if U != bsz:
                 raise ValueError("fbkst_b200.CrossAttention: %d key columns for %d queries" % (U, bsz))
@@ -212,6 +253,7 @@ class CrossAttention(nn.Module):
             need_weights = True
         tgt_len, bsz, D = query.shape
         assert D == self.embed_dim
+        f32 = self._precision == "fp32"
         with torch.no_grad():
             buf = self._get_input_buffer(incremental_state) if incremental_state is not None else {}
             if "fbkst_kv" in buf and static_kv:  # :181-186: cached, key/value ignored
@@ -219,6 +261,12 @@ class CrossAttention(nn.Module):
                 if row_map.numel() != bsz:
                     raise RuntimeError("fbkst_b200.CrossAttention: cached state holds %d hypotheses, "
                                        "query has %d" % (row_map.numel(), bsz))
+                # the cached K/V's dtype records the precision it was projected in
+                if (kv.dtype == torch.float32) != f32:
+                    raise RuntimeError("fbkst_b200.CrossAttention: the incremental state was built with "
+                                       "precision=%r, the module now runs precision=%r; start a new "
+                                       "incremental state after switching precision" %
+                                       ("fp32" if kv.dtype == torch.float32 else "bf16", self._precision))
             else:
                 if key is None:
                     raise ValueError("fbkst_b200.CrossAttention: no key and no cached state")
@@ -227,15 +275,21 @@ class CrossAttention(nn.Module):
                     self._set_input_buffer(incremental_state, dict(fbkst_kv=kv, fbkst_mask=mask,
                                                                    fbkst_row_map=row_map))
             S, U = kv.shape[0], kv.shape[1]
-            P = self._prepared()
             qa = query.reshape(tgt_len * bsz, D)
-            qa = ops.cast_bf16(qa.float().contiguous()) if qa.dtype != torch.bfloat16 else qa.contiguous()
-            q = ops.linear(qa, P["wq"], P["bq"])
-            if not q.is_contiguous():
-                q = q.contiguous()
-            heads, w = ops.xattn(q, kv, mask, row_map, S, U, bsz, tgt_len, self.num_heads,
-                                 weights=2 if need_head_weights else (1 if need_weights else 0))
-            attn = ops.linear(heads, P["wo"], P["bo"], out_dtype=torch.float32).view(tgt_len, bsz, D)
+            weights = 2 if need_head_weights else (1 if need_weights else 0)
+            if f32:
+                P = self._prepared_f32()
+                q = ops.linear_f32(qa.float().contiguous(), P["wq"], P["bq"])
+                heads, w = ops.xattn_f32(q, kv, mask, row_map, S, U, bsz, tgt_len, self.num_heads, weights)
+                attn = ops.linear_f32(heads, P["wo"], P["bo"]).view(tgt_len, bsz, D)
+            else:
+                P = self._prepared()
+                qa = ops.cast_bf16(qa.float().contiguous()) if qa.dtype != torch.bfloat16 else qa.contiguous()
+                q = ops.linear(qa, P["wq"], P["bq"])
+                if not q.is_contiguous():
+                    q = q.contiguous()
+                heads, w = ops.xattn(q, kv, mask, row_map, S, U, bsz, tgt_len, self.num_heads, weights=weights)
+                attn = ops.linear(heads, P["wo"], P["bo"], out_dtype=torch.float32).view(tgt_len, bsz, D)
             if attn.dtype != query.dtype:
                 attn = attn.to(query.dtype)
         return attn, w
@@ -246,16 +300,24 @@ class CrossAttention(nn.Module):
         return state_dict
 
 
-def swap_cross_attention(decoder):
+def swap_cross_attention(decoder, precision="bf16"):
     """Replace every ``layer.encoder_attn`` of a fairseq ``TransformerDecoder`` with a
-    ``CrossAttention`` holding the SAME parameter tensors (state_dict keys and values unchanged)."""
+    ``CrossAttention`` holding the SAME parameter tensors (state_dict keys and values unchanged), and
+    set every layer's ``CrossAttention.precision`` (already swapped layers included) to ``precision``.
+    Returns the number of layers swapped."""
+    if precision not in PRECISIONS:
+        raise ValueError("fbkst_b200: precision must be one of %s, got %r" % (PRECISIONS, precision))
     n = 0
     for layer in getattr(decoder, "layers", []):
         old = getattr(layer, "encoder_attn", None)
-        if old is None or isinstance(old, CrossAttention):
+        if old is None:
+            continue
+        if isinstance(old, CrossAttention):
+            old.precision = precision
             continue
         new = CrossAttention(old.embed_dim, old.num_heads, kdim=old.kdim, vdim=old.vdim,
                              dropout=old.dropout, encoder_decoder_attention=True)
+        new.precision = precision
         for nm in ("k_proj", "v_proj", "q_proj", "out_proj"):
             getattr(new, nm).weight = getattr(old, nm).weight
             getattr(new, nm).bias = getattr(old, nm).bias

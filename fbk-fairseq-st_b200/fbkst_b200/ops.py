@@ -508,28 +508,38 @@ def xattn(q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights=0):
     q [tgt_len*bsz, D] bf16 (pre-scaled), kv [S, U, 2D] bf16, mask [U, S] bool/uint8 or None,
     row_map [bsz] int32.  weights: 0 none, 1 head-averaged [bsz, tgt_len, S], 2 per head
     [H, bsz, tgt_len, S].  Returns (out [tgt_len*bsz, D] bf16, weights or None)."""
+    return _xattn("xattn", torch.bfloat16, q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights)
+
+
+def xattn_f32(q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights=0):
+    """``xattn`` with fp32 q [tgt_len*bsz, D], kv [S, U, 2D] and out (fp32 FMA throughout)."""
+    return _xattn("xattn_f32", torch.float32, q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights)
+
+
+def _xattn(name, dtype, q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights):
     lib = _lib.require_device()
-    _req(q, torch.bfloat16, "xattn.q"); _req(kv, torch.bfloat16, "xattn.kv")
-    _req(row_map, torch.int32, "xattn.row_map")
+    _req(q, dtype, name + ".q"); _req(kv, dtype, name + ".kv")
+    _req(row_map, torch.int32, name + ".row_map")
     D = 64 * H
     if tuple(q.shape) != (tgt_len * bsz, D) or tuple(kv.shape) != (S, U, 2 * D) or row_map.numel() != bsz:
-        raise ValueError("fbkst_b200.xattn: shape mismatch q %s kv %s row_map %s" %
-                         (tuple(q.shape), tuple(kv.shape), tuple(row_map.shape)))
+        raise ValueError("fbkst_b200.%s: shape mismatch q %s kv %s row_map %s" %
+                         (name, tuple(q.shape), tuple(kv.shape), tuple(row_map.shape)))
     if mask is not None:
         if mask.dtype == torch.bool:
             mask = mask.view(torch.uint8)
-        _req(mask, torch.uint8, "xattn.mask")
+        _req(mask, torch.uint8, name + ".mask")
         if tuple(mask.shape) != (U, S):
-            raise ValueError("fbkst_b200.xattn: mask must be [U, S]")
-    out = torch.empty(tgt_len * bsz, D, dtype=torch.bfloat16, device=q.device)
+            raise ValueError("fbkst_b200.%s: mask must be [U, S]" % name)
+    out = torch.empty(tgt_len * bsz, D, dtype=dtype, device=q.device)
     w = ws = None
     if weights == 1:
         w = torch.empty(bsz, tgt_len, S, dtype=torch.float32, device=q.device)
         ws = torch.empty(H, bsz, tgt_len, S, dtype=torch.float32, device=q.device)
     elif weights == 2:
         w = torch.empty(H, bsz, tgt_len, S, dtype=torch.float32, device=q.device)
-    check(lib.fbkst_xattn_fwd(q.data_ptr(), kv.data_ptr(), _ptr(mask), row_map.data_ptr(), out.data_ptr(),
-                              _ptr(w), _ptr(ws), weights, S, U, bsz, tgt_len, H, _stream()))
+    fn = lib.fbkst_xattn_fwd_f32 if dtype == torch.float32 else lib.fbkst_xattn_fwd
+    check(fn(q.data_ptr(), kv.data_ptr(), _ptr(mask), row_map.data_ptr(), out.data_ptr(),
+             _ptr(w), _ptr(ws), weights, S, U, bsz, tgt_len, H, _stream()))
     _count(2 if weights == 1 else 1)
     return out, w
 

@@ -51,6 +51,10 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
 
     @classmethod
     def build_model(cls, args, task):
+        xattn_precision = getattr(args, "b200_cross_attention_precision", "bf16") or "bf16"
+        if xattn_precision != "bf16" and not getattr(args, "b200_cross_attention", False):
+            raise ValueError("--b200-cross-attention-precision %s selects the precision of the sm_100a "
+                             "cross-attention: it needs --b200-cross-attention" % xattn_precision)
         _ref.base_architecture(args)
         if not hasattr(args, "max_source_positions"):
             args.max_source_positions = 100000
@@ -70,7 +74,7 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
         # reorders move an index vector).  Same parameters / state_dict keys; inference only, so it
         # is opt-in: --b200-cross-attention (generate.py), never needed for train.py.
         if getattr(args, "b200_cross_attention", False):
-            swap_cross_attention(decoder)
+            swap_cross_attention(decoder, precision=xattn_precision)
             encoder.lazy_beam_reorder = getattr(args, "b200_lazy_beam_reorder", False)
         return cls(encoder, decoder)
 
@@ -87,6 +91,11 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
                             help="encoder operand precision at inference: bf16 tensor-core operands (default) "
                                  "or fp32 on split-TF32 tensor cores (within 1e-3 of an fp32 reference; "
                                  "inference only)")
+        parser.add_argument("--b200-cross-attention-precision", choices=["bf16", "fp32"], default="bf16",
+                            help="with --b200-cross-attention: operand precision of the decoder's "
+                                 "encoder-decoder attention, bf16 (default) or fp32 (split-TF32 projections, "
+                                 "fp32 core: within 1e-3 of an fp32 reference); --b200-precision sets the "
+                                 "encoder's only")
 
 
 # ---------------------------------------------------------------------------------------------------

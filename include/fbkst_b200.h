@@ -349,6 +349,12 @@ int fbkst_time_stretch_f32(const float* x, const int32_t* windows, int n_windows
 int fbkst_xattn_fwd(const void* q, const void* kv, const uint8_t* key_padding_mask,
                     const int32_t* row_map, void* out, float* attn_w, float* head_ws, int w_mode,
                     int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream);
+/* fbkst_xattn_fwd with fp32 q [tgt_len * bsz, D] (8-byte aligned), kv [S, U, 2D] and out [tgt_len * bsz, D]
+ * (16-byte aligned): the fp32-accurate decode path (CrossAttention.precision = "fp32").  Same kernel body,
+ * fp32 FMA and softmax; every other argument as above. */
+int fbkst_xattn_fwd_f32(const float* q, const float* kv, const uint8_t* key_padding_mask,
+                        const int32_t* row_map, float* out, float* attn_w, float* head_ws, int w_mode,
+                        int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream);
 
 /* ---- weight preparation (fp32 master parameters -> kernel operand formats) ----------------- */
 /* dst[i] = bf16(src[i] * scale) */

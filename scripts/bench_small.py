@@ -2,6 +2,7 @@
 stream; a 256 MB L2 flush is queued before every launch, which also keeps the GPU behind the CPU so
 that no launch gap leaks into the event interval).  usage: bench_small.py [reps] [name]"""
 import os
+import subprocess
 import sys
 
 import torch
@@ -17,6 +18,12 @@ flush = torch.empty(256 << 20, dtype=torch.uint8, device=d)
 reps = int(sys.argv[1]) if len(sys.argv) > 1 else 10
 only = sys.argv[2] if len(sys.argv) > 2 else None
 HBM = bench.peaks()["hbm"]
+try:  # a time is only worth something with the card and the power limit it was measured at
+    _smi = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                          capture_output=True, text=True, timeout=30).stdout.strip()
+except (OSError, subprocess.SubprocessError):
+    _smi = "nvidia-smi unavailable"
+print("device: %s | %s" % (torch.cuda.get_device_name(d), _smi), flush=True)
 
 
 def timeit(name, fn, nbytes):
@@ -36,6 +43,26 @@ def timeit(name, fn, nbytes):
     med = ts[len(ts) // 2]
     print("%-26s %8.1f us  %7.0f GB/s  %5.1f%% of %.0f  (min %.1f us)" %
           (name, med * 1e3, nbytes / med / 1e6, 100 * nbytes / med / 1e6 / HBM, HBM, ts[0] * 1e3), flush=True)
+
+
+def warm_us(fn, n=20, replays=5):
+    """Device time per call of ``fn`` with its operands L2-resident: n back-to-back calls captured in one CUDA
+    graph, so the host launch path is not what is timed."""
+    fn()
+    torch.cuda.synchronize()
+    gr = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(gr):
+        for _ in range(n):
+            fn()
+    gr.replay()
+    torch.cuda.synchronize()
+    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    s.record()
+    for _ in range(replays):
+        gr.replay()
+    e.record()
+    torch.cuda.synchronize()
+    return s.elapsed_time(e) / (n * replays) * 1e3
 
 
 B, T, F, L, D, V = 64, 1500, 40, 375, 512, 8005
@@ -106,23 +133,43 @@ if not only or "xattn" in only:
                nb + bsz_ * S_ * 4 * (2 * H_ + 1))
         if not only or "xattn" in only:
             # decode re-reads the same K/V every step: the steady state is L2-resident, not cold
-            # (20 calls captured in one CUDA graph, so the host launch path is not what is timed)
-            ops.xattn(q_, kv_, mk_, rm_, S_, U_, bsz_, 1, H_, weights=0)
-            torch.cuda.synchronize()
-            gr_ = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(gr_):
-                for _ in range(20):
-                    o_ = ops.xattn(q_, kv_, mk_, rm_, S_, U_, bsz_, 1, H_, weights=0)
-            gr_.replay()
-            torch.cuda.synchronize()
-            s_, e_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            s_.record()
-            for _ in range(5):
-                gr_.replay()
-            e_.record()
-            torch.cuda.synchronize()
-            w_us = s_.elapsed_time(e_) / 100 * 1e3
+            w_us = warm_us(lambda: ops.xattn(q_, kv_, mk_, rm_, S_, U_, bsz_, 1, H_, weights=0))
             print("    warm (graph of 20 back-to-back steps, K/V L2-resident): %.1f us/step, %.0f GB/s of K/V" %
                   (w_us, nb / w_us / 1e3))
         print("    (reference cache traffic for the step: %.1f MB fp32; unique K/V here: %.1f MB bf16)" %
               (bsz_ * 2 * S_ * D_ * 4 / 1e6, kv_.numel() * 2 / 1e6))
+
+    # the fp32 decode path (CrossAttention.precision = "fp32") against bf16 at the cfg2 generate shape: the core
+    # alone, one module call per layer-step (q projection + core + out_proj, no weights, K/V cached) and the
+    # once-per-utterance K/V projection.  Bytes: unique K/V + q + out, plus the weights each projection reads.
+    from fbkst_b200.cross_attention import CrossAttention
+    S_, U_, beam_, H_ = 95, 64, 5, 8
+    D_ = 64 * H_
+    bsz_ = U_ * beam_
+    rm_ = torch.arange(U_, device=d).repeat_interleave(beam_).int()
+    mk_ = (torch.arange(S_, device=d)[None, :] >= torch.randint(S_ // 2, S_ + 1, (U_, 1), device=d))
+    q32 = torch.randn(bsz_, D_, device=d) * 0.125
+    kv32 = torch.randn(S_, U_, 2 * D_, device=d)
+    nb32 = kv32.numel() * 4 + q32.numel() * 8
+    timeit("xattn f32 S=%d U=%d beam=%d H=%d" % (S_, U_, beam_, H_),
+           lambda: ops.xattn_f32(q32, kv32, mk_, rm_, S_, U_, bsz_, 1, H_, weights=0), nb32)
+    w_us = warm_us(lambda: ops.xattn_f32(q32, kv32, mk_, rm_, S_, U_, bsz_, 1, H_, weights=0))
+    print("    warm (graph of 20 back-to-back steps, K/V L2-resident): %.1f us/step, %.0f GB/s of K/V" %
+          (w_us, nb32 / w_us / 1e3))
+    enc_ = torch.randn(S_, U_, D_, device=d)
+    mpad_ = mk_.view(U_, S_)
+    xq_ = torch.randn(1, bsz_, D_, device=d)
+    for prec, esz in (("bf16", 2), ("fp32", 4)):
+        m_ = CrossAttention(D_, H_).eval().to(d)
+        m_.precision = prec
+        inc_ = {}
+        with torch.no_grad():
+            m_(xq_[:, :U_], enc_, enc_, key_padding_mask=mpad_, incremental_state=inc_, static_kv=True)
+        m_.reorder_incremental_state(inc_, rm_.long())  # x beam: the row map gathers, the K/V stays per utterance
+        step = lambda: m_(xq_, None, None, incremental_state=inc_, static_kv=True, need_weights=False)
+        nbm = S_ * U_ * 2 * D_ * esz + 2 * D_ * D_ * esz + bsz_ * D_ * 8
+        timeit("xattn module %s step" % prec, step, nbm)
+        w_us = warm_us(step)
+        print("    warm (graph of 20 back-to-back steps, K/V L2-resident): %.1f us/step" % w_us)
+        timeit("xattn module %s K/V proj" % prec, lambda: m_._project_kv(enc_, mpad_, U_),
+               enc_.numel() * 4 + 2 * D_ * D_ * esz + S_ * U_ * 2 * D_ * esz)
