@@ -169,8 +169,7 @@ __device__ __forceinline__ int4 attn_decode_raw(int w, const int* __restrict__ l
   const int b = bh / H, h = bh - b * H;
   const int q0 = qt * AT_BM;
   const int len = min(__ldg(lengths + b), L);
-  const int n_kv = (q0 < len) ? (len + AT_BN - 1) / AT_BN : 0;
-  return make_int4(q0, b, h, (len << 8) | n_kv);
+  return make_int4(q0, b, h, q0 < len ? len : 0);  // length 0: a tile of padded queries
 }
 struct AttnList {
   const int4* table;  // shared memory
@@ -183,8 +182,9 @@ struct AttnList {
     it.q0 = r.x;
     it.b = r.y;
     it.h = r.z;
-    it.len = r.w >> 8;
-    it.n_kv = r.w & 255;
+    it.len = r.w;
+    // derived here, not packed beside the length: an 8-bit count wraps at 256 key tiles (L > 16320)
+    it.n_kv = static_cast<unsigned>(it.len + AT_BN - 1) / AT_BN;
   }
   // next item at or after index k that has pipeline work (n_kv > 0); returns its index
   __device__ __forceinline__ int next_work(AttnItem& it, int k) const {

@@ -256,9 +256,11 @@ __device__ __forceinline__ int4 aw_decode(int w, const int* __restrict__ lengths
   const int b = bh / H, h = bh - b * H;
   const int q0 = qt * AW_BM;
   const int len = min(__ldg(lengths + b), L);
-  const int n_kv = (q0 < len) ? (len + AW_BN - 1) / AW_BN : 0;
-  return make_int4(q0, b, h, (len << 8) | n_kv);
+  return make_int4(q0, b, h, q0 < len ? len : 0);  // length 0: a tile of padded queries
 }
+// key tiles of an item, derived where the item is read (an 8-bit count packed beside the length wraps at 256
+// tiles, L > 32640)
+__device__ __forceinline__ int aw_n_kv(int len) { return static_cast<unsigned>(len + AW_BN - 1) / AW_BN; }
 struct WList {
   const int4* table;  // shared memory: the CTA's first AW_TABLE items, decoded once
   const int* lengths;
@@ -270,8 +272,8 @@ struct WList {
     it.q0 = r.x;
     it.b = r.y;
     it.h = r.z;
-    it.len = r.w >> 8;
-    it.n_kv = r.w & 255;
+    it.len = r.w;
+    it.n_kv = aw_n_kv(it.len);
   }
 };
 // Tile stream of one softmax group: items k = grp, grp + 2, ... of the CTA's list, key tiles in order.
@@ -560,8 +562,8 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
       it.q0 = r_cur.x;
       it.b = r_cur.y;
       it.h = r_cur.z;
-      it.len = r_cur.w >> 8;
-      it.n_kv = r_cur.w & 255;
+      it.len = r_cur.w;
+      it.n_kv = aw_n_kv(it.len);
       w_cur += 2 * gridDim.x;
       if (w_cur < n_items) r_cur = (k + 2 < AW_TABLE) ? sItems[k + 2] : aw_decode(w_cur, lengths, L, H, nq);
       const int i = it.q0 + q;

@@ -17,6 +17,7 @@ run small tests/test_gpu_ops.py -k "layernorm or cmvn or fc3_weight or row_stats
 run ctc tests/test_gpu_ops.py -k "ctc"
 run conv tests/test_gpu_ops.py -k "conv_stack"
 run attn tests/test_gpu_ops.py -k "attention"
+run attn_edges tests/test_attention_edges.py
 run encoder tests/test_gpu_encoder.py
 run misc tests/test_gpu_ops.py -k "custom_ops or collater"
 run criterion tests/test_gpu_criterion.py
