@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "fbkst_b200", "libfbkst_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["host_common.cu", "elementwise.cu", "ctc.cu", "ctc_criterion.cu", "augment.cu", "cross_attention.cu", "gemm_tcgen05.cu", "gemm2_tcgen05.cu", "conv2_tcgen05.cu", "conv1_tcgen05.cu",
+SOURCES = ["host_common.cu", "elementwise.cu", "ctc.cu", "ctc_criterion.cu", "augment.cu", "cross_attention.cu", "self_attention.cu", "gemm_tcgen05.cu", "gemm2_tcgen05.cu", "conv2_tcgen05.cu", "conv1_tcgen05.cu",
            "attention_tcgen05.cu", "attention_wide.cu", "attention_train.cu", "train_elementwise.cu", "conv_train.cu", "tf32x3.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -10,6 +10,7 @@ ERR_ARG, ERR_CUDA, ERR_OOM = -1, -2, -3
 BF16, F32 = 0, 1
 CTC_STRATEGY = {"avg": 0, "weighted": 1, "softmax": 2}
 EPI_RELU, EPI_OUT_F32, EPI_ROW_REMAP, EPI_POSEMB, EPI_AB_F16 = 1, 2, 4, 8, 16
+SA_INCREMENTAL, SA_FULL, SA_CAUSAL = 0, 1, 2
 
 P, I, I64, F, U64 = c_void_p, c_int, c_int64, c_float, c_uint64
 
@@ -45,6 +46,8 @@ SIGNATURES = {
     "fbkst_time_stretch_f32": [P, P, I, P, P, I, I, I, I, P],
     "fbkst_xattn_fwd": [P, P, P, P, P, P, P, I, I, I, I, I, I, P],
     "fbkst_xattn_fwd_f32": [P, P, P, P, P, P, P, I, I, I, I, I, I, P],
+    "fbkst_dec_self_attn_fwd": [P, I64, P, P, P, P, P, I, I, I, I, I, I, I, P],
+    "fbkst_dec_self_attn_fwd_f32": [P, I64, P, P, P, P, P, I, I, I, I, I, I, I, P],
     "fbkst_cast_bf16": [P, P, I64, F, P],
     "fbkst_prep_conv2_weight": [P, P, I, P],
     "fbkst_prep_fc3_weight": [P, P, I, I, I, P],

@@ -4,7 +4,8 @@ library or the GPU is missing (no fallback)."""
 import torch
 
 from . import _lib
-from ._lib import BF16, CTC_STRATEGY, EPI_AB_F16, EPI_OUT_F32, EPI_POSEMB, EPI_RELU, EPI_ROW_REMAP, F32, check
+from ._lib import (BF16, CTC_STRATEGY, EPI_AB_F16, EPI_OUT_F32, EPI_POSEMB, EPI_RELU, EPI_ROW_REMAP, F32, SA_CAUSAL,
+                   SA_FULL, SA_INCREMENTAL, check)
 
 LAUNCHES = 0  # kernels launched through this module (bench.py reports it as gpu_launches)
 
@@ -541,6 +542,62 @@ def _xattn(name, dtype, q, kv, mask, row_map, S, U, bsz, tgt_len, H, weights):
     check(fn(q.data_ptr(), kv.data_ptr(), _ptr(mask), row_map.data_ptr(), out.data_ptr(),
              _ptr(w), _ptr(ws), weights, S, U, bsz, tgt_len, H, _stream()))
     _count(2 if weights == 1 else 1)
+    return out, w
+
+
+def dec_self_attn(q, cache, anc, pad, n_keys, bsz, tgt_len, H, mode=SA_INCREMENTAL, weights=0):
+    """Decoder self-attention of ``tgt_len * bsz`` query rows over an append-only cache.
+    q [tgt_len*bsz, D] bf16 (pre-scaled; unit column stride, any even row pitch: usually a view of the cache's
+    q columns), cache [T_cap, R, 3D] bf16 (per step: q | k | v of R cache rows), anc [>= n_keys, bsz] int32 or
+    None (hypothesis b reads cache row anc[s, b] at step s), pad [T_cap, R] bool/uint8 or None (padding keys by
+    step and cache row).  mode: SA_INCREMENTAL (tgt_len 1, keys 0..n_keys-1), SA_FULL or SA_CAUSAL (n_keys ==
+    tgt_len).  weights: 0 none, 1 head-averaged [bsz, tgt_len, n_keys], 2 per head [H, bsz, tgt_len, n_keys].
+    Returns (out [tgt_len*bsz, D] bf16, weights or None)."""
+    return _dec_self_attn("dec_self_attn", torch.bfloat16, q, cache, anc, pad, n_keys, bsz, tgt_len, H, mode,
+                          weights)
+
+
+def dec_self_attn_f32(q, cache, anc, pad, n_keys, bsz, tgt_len, H, mode=SA_INCREMENTAL, weights=0):
+    """``dec_self_attn`` with fp32 q, cache and out (fp32 FMA throughout)."""
+    return _dec_self_attn("dec_self_attn_f32", torch.float32, q, cache, anc, pad, n_keys, bsz, tgt_len, H, mode,
+                          weights)
+
+
+def _dec_self_attn(name, dtype, q, cache, anc, pad, n_keys, bsz, tgt_len, H, mode, weights):
+    lib = _lib.require_device()
+    _req(cache, dtype, name + ".cache")
+    D = 64 * H
+    if not (isinstance(q, torch.Tensor) and q.is_cuda and q.dtype == dtype):
+        raise ValueError("fbkst_b200.%s.q: expected a CUDA %s tensor" % (name, dtype))
+    if q.dim() != 2 or tuple(q.shape) != (tgt_len * bsz, D) or q.stride(1) != 1:
+        raise ValueError("fbkst_b200.%s: q must be [tgt_len*bsz, D] = (%d, %d) with unit column stride, got %s" %
+                         (name, tgt_len * bsz, D, tuple(q.shape)))
+    if cache.dim() != 3 or cache.shape[2] != 3 * D or cache.shape[0] < n_keys:
+        raise ValueError("fbkst_b200.%s: cache %s must be [>= %d steps, R, 3D = %d]" %
+                         (name, tuple(cache.shape), n_keys, 3 * D))
+    R = cache.shape[1]
+    if anc is not None:
+        _req(anc, torch.int32, name + ".anc")
+        if anc.dim() != 2 or anc.shape[0] < n_keys or anc.shape[1] != bsz:
+            raise ValueError("fbkst_b200.%s: anc %s must be [>= %d, bsz = %d]" % (name, tuple(anc.shape), n_keys, bsz))
+    if pad is not None:
+        if pad.dtype == torch.bool:
+            pad = pad.view(torch.uint8)
+        _req(pad, torch.uint8, name + ".pad")
+        if tuple(pad.shape) != tuple(cache.shape[:2]):
+            raise ValueError("fbkst_b200.%s: pad must be [T_cap, R] = %s" % (name, tuple(cache.shape[:2])))
+    if mode not in (SA_INCREMENTAL, SA_FULL, SA_CAUSAL) or weights not in (0, 1, 2):
+        raise ValueError("fbkst_b200.%s: mode %r / weights %r out of range" % (name, mode, weights))
+    out = torch.empty(tgt_len * bsz, D, dtype=dtype, device=q.device)
+    w = None
+    if weights == 1:
+        w = torch.empty(bsz, tgt_len, n_keys, dtype=torch.float32, device=q.device)
+    elif weights == 2:
+        w = torch.empty(H, bsz, tgt_len, n_keys, dtype=torch.float32, device=q.device)
+    fn = lib.fbkst_dec_self_attn_fwd_f32 if dtype == torch.float32 else lib.fbkst_dec_self_attn_fwd
+    check(fn(q.data_ptr(), q.stride(0), cache.data_ptr(), _ptr(anc), _ptr(pad), out.data_ptr(), _ptr(w), weights,
+             mode, n_keys, R, bsz, tgt_len, H, _stream()))
+    _count()
     return out, w
 
 

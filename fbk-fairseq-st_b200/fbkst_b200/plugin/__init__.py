@@ -38,6 +38,7 @@ from examples.speech_recognition.models import conv_transformer as _ref  # noqa:
 
 from fbkst_b200 import encoder as _enc  # noqa: E402
 from fbkst_b200.cross_attention import swap_cross_attention  # noqa: E402
+from fbkst_b200.self_attention import swap_self_attention  # noqa: E402
 
 B200ConvolutionalTransformerEncoder = _enc.make_encoder_class(FairseqEncoder)
 # hand fairseq's own NamedTuple types to downstream isinstance checks
@@ -55,6 +56,10 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
         if xattn_precision != "bf16" and not getattr(args, "b200_cross_attention", False):
             raise ValueError("--b200-cross-attention-precision %s selects the precision of the sm_100a "
                              "cross-attention: it needs --b200-cross-attention" % xattn_precision)
+        sattn_precision = getattr(args, "b200_self_attention_precision", "bf16") or "bf16"
+        if sattn_precision != "bf16" and not getattr(args, "b200_self_attention", False):
+            raise ValueError("--b200-self-attention-precision %s selects the precision of the sm_100a decoder "
+                             "self-attention: it needs --b200-self-attention" % sattn_precision)
         _ref.base_architecture(args)
         if not hasattr(args, "max_source_positions"):
             args.max_source_positions = 100000
@@ -76,6 +81,10 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
         if getattr(args, "b200_cross_attention", False):
             swap_cross_attention(decoder, precision=xattn_precision)
             encoder.lazy_beam_reorder = getattr(args, "b200_lazy_beam_reorder", False)
+        # N5: decoder self-attention on the device kernel (append-only K/V cache, beam reorders move an
+        # ancestry table).  Same parameters / state_dict keys; inference only, opt-in like N4.
+        if getattr(args, "b200_self_attention", False):
+            swap_self_attention(decoder, precision=sattn_precision)
         return cls(encoder, decoder)
 
     @staticmethod
@@ -96,6 +105,12 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
                                  "encoder-decoder attention, bf16 (default) or fp32 (split-TF32 projections, "
                                  "fp32 core: within 1e-3 of an fp32 reference); --b200-precision sets the "
                                  "encoder's only")
+        parser.add_argument("--b200-self-attention", action="store_true",
+                            help="run the decoder's self-attention on the sm_100a kernel with an append-only K/V "
+                                 "cache that beam reorders never copy (inference: generate.py)")
+        parser.add_argument("--b200-self-attention-precision", choices=["bf16", "fp32"], default="bf16",
+                            help="with --b200-self-attention: operand precision of the decoder's self-attention, "
+                                 "bf16 (default) or fp32 (split-TF32 projections, fp32 core)")
 
 
 # ---------------------------------------------------------------------------------------------------

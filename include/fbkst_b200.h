@@ -39,6 +39,9 @@ enum { FBKST_BF16 = 0, FBKST_F32 = 1 };
 
 enum { FBKST_CTC_AVG = 0, FBKST_CTC_WEIGHTED = 1, FBKST_CTC_SOFTMAX = 2 };
 
+/* query modes of fbkst_dec_self_attn_fwd */
+enum { FBKST_SA_INCREMENTAL = 0, FBKST_SA_FULL = 1, FBKST_SA_CAUSAL = 2 };
+
 /* epilogue flags of fbkst_linear_bf16 */
 enum {
   FBKST_EPI_RELU = 1,      /* y = max(y, 0) after the bias                                  */
@@ -355,6 +358,37 @@ int fbkst_xattn_fwd(const void* q, const void* kv, const uint8_t* key_padding_ma
 int fbkst_xattn_fwd_f32(const float* q, const float* kv, const uint8_t* key_padding_mask,
                         const int32_t* row_map, float* out, float* attn_w, float* head_ws, int w_mode,
                         int S, int U, int bsz, int tgt_len, int H, fbkst_stream_t stream);
+
+/* ---- next row N5: decoder self-attention over an append-only K/V cache ---------------------------
+ * fbkst_dec_self_attn_fwd replaces fairseq/modules/multihead_attention.py:108-367 with
+ * self_attention=True as TransformerDecoderLayer.forward calls it (fairseq/modules/transformer_layer.py).  In
+ * generation the reference appends each step's key and value to per-hypothesis caches with torch.cat and
+ * gathers them in reorder_incremental_state (:407-420); here the cache is written once per step and a beam
+ * reorder moves only the ancestry table, through which the kernel gathers the keys.
+ *   q        [tgt_len * bsz, D] with row pitch ldq elements (even), row r = i * bsz + b, already scaled by
+ *            head_dim^-0.5 (:209); usually a view of the cache's q columns
+ *   cache    [>= n_keys, R, 3D] time-major, one [R, 3D] slab per step: columns [0, D) q, [D, 2D) k,
+ *            [2D, 3D) v; R = cache rows per step (the hypothesis count at step 0)
+ *   anc      [>= n_keys, bsz] int32 or NULL (identity): anc[s * bsz + b] is the cache row that holds, at step s,
+ *            the ancestor of hypothesis b.  An entry outside [0, R) is a masked key.
+ *   key_padding [>= n_keys, R] uint8 (1 = padding key, :330-335) indexed by (step, cache row), or NULL
+ *   mode     FBKST_SA_INCREMENTAL: tgt_len == 1, the query of row b sees keys 0 .. n_keys-1;
+ *            FBKST_SA_FULL: n_keys == tgt_len, every query sees every key;
+ *            FBKST_SA_CAUSAL: n_keys == tgt_len, query i sees keys 0 .. i (fairseq's future mask)
+ *   out      [tgt_len * bsz, D] (heads concatenated; input of out_proj, :353)
+ *   attn_w   w_mode 0: unused; 1: [bsz, tgt_len, n_keys] fp32 averaged over heads (:355-362);
+ *            2: [H, bsz, tgt_len, n_keys] fp32 per head.  Masked and future keys get exactly 0.
+ * A query whose visible keys are all masked gets a zero output row and zero weights (the reference would
+ * produce NaN), as in fbkst_xattn_fwd.  D = 64 * H, H <= 16; 4 * (n_keys * (H + 1) + 64 * H) bytes of shared
+ * memory must fit in 200 KB (n_keys <= 2948 at H = 16, <= 5632 at H = 8). */
+int fbkst_dec_self_attn_fwd(const void* q, int64_t ldq, const void* cache, const int32_t* anc,
+                            const uint8_t* key_padding, void* out, float* attn_w, int w_mode, int mode,
+                            int n_keys, int R, int bsz, int tgt_len, int H, fbkst_stream_t stream);
+/* fbkst_dec_self_attn_fwd with fp32 q, cache and out: the fp32-accurate decode path.  Same kernel body,
+ * fp32 FMA and softmax; every other argument as above. */
+int fbkst_dec_self_attn_fwd_f32(const float* q, int64_t ldq, const float* cache, const int32_t* anc,
+                                const uint8_t* key_padding, float* out, float* attn_w, int w_mode, int mode,
+                                int n_keys, int R, int bsz, int tgt_len, int H, fbkst_stream_t stream);
 
 /* ---- weight preparation (fp32 master parameters -> kernel operand formats) ----------------- */
 /* dst[i] = bf16(src[i] * scale) */
