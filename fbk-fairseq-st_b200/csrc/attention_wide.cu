@@ -1,10 +1,11 @@
-// Self-attention core, "wide" layout: the default kernel for L <~ 2500 (reference: local_attention.py:115-139
-// with LogPenalty conv_transformer_layer.py:22-27).  Same arithmetic and the same pipeline roles as
-// attention_fwd_dec_kernel (attention_tcgen05.cu, the round-1 kernel, still selected by FBKST_ATTN_WIDE=0 and
-// for longer inputs), re-cut for what that kernel's profile showed (profiles/r02y_ncu_attention.txt): softmax
-// warps at 7.3 issued instructions per score and ~0.1 IPC each (96 registers: one 8-score chunk in flight),
-// 64 KB of P written to and read back from shared memory per 128 x 128 scores next to 64 KB of penalty loads
-// on a 128 B/clk path, and 16 M128 x N64 tensor instructions per 128 x 128 scores at 133 cycles apiece.
+// Self-attention core, "wide" layout: the kernel for every L without the penalty and for L <= 2560 with it
+// (reference: local_attention.py:115-139 with LogPenalty conv_transformer_layer.py:22-27); longer inputs with the
+// penalty go to the split-KV kernel of attention_tcgen05.cu.  Same arithmetic and the same pipeline roles as the
+// round-1 decoupled kernel it replaced (since removed), re-cut for what that kernel's profile showed
+// (profiles/r02y_ncu_attention.txt): softmax warps at 7.3 issued instructions per score and ~0.1 IPC each
+// (96 registers: one 8-score chunk in flight), 64 KB of P written to and read back from shared memory per
+// 128 x 128 scores next to 64 KB of penalty loads on a 128 B/clk path, and 16 M128 x N64 tensor instructions
+// per 128 x 128 scores at 133 cycles apiece.
 //
 //   * ONE CTA per SM, 384 threads: a producer warpgroup that shrinks to 56 registers (warp 0 TMA loads,
 //     warp 1 QK issue, warps 2 / 3 PV issue of group 0 / 1) and two softmax warpgroups that grow to 224,
@@ -773,7 +774,7 @@ extern "C" int fbkst_debug_set_attention_wide_trace(long long* buf) {
 namespace fbkst {
 
 // Returns FBKST_OK after launching, or 1 when this shape is not served by the wide kernel (the caller
-// falls through to the decoupled / split-KV kernels).
+// falls through to the split-KV kernel of attention_tcgen05.cu).
 int attention_wide_launch(const void* qkv, void* out, const int32_t* lengths, int L, int B, int H, int log_penalty,
                           const int32_t* q_limit, cudaStream_t st) {
   const int smem = aw_smem_bytes(L, log_penalty);

@@ -2,10 +2,10 @@
 // padding 1) -> ReLU -> BatchNorm2d(eval)) on the tensor pipe.
 //
 // Cin = 1, so the implicit GEMM has K = 9: far too little work to be tensor-bound -- the kernel's job is
-// to WRITE 2*C bytes per output pixel (cfg2: 123 MB) at HBM speed, and the SIMT version (elementwise.cu:
-// 72 FMAs + epilogue per pixel and 8-channel group, 128 registers) spends 65 us issuing instructions for
-// a 19 us write.  Here one tile = 128 consecutive output pixels (the channels-last output is one
-// contiguous [pixels, C] matrix):
+// to WRITE 2*C bytes per output pixel (cfg2: 123 MB) at HBM speed, and the SIMT version this replaced
+// (since removed: 72 FMAs + epilogue per pixel and 8-channel group, 128 registers) spent 65 us issuing
+// instructions for a 19 us write.  Here one tile = 128 consecutive output pixels (the channels-last output
+// is one contiguous [pixels, C] matrix):
 //   build     thread <-> pixel: 9 predicated loads (zero outside the image = the conv padding), fp16,
 //             two 16-byte chunks into a K-major 128B-swizzled A tile (K padded 9 -> 16, ONE UMMA k-step)
 //   MMA       one tcgen05.mma M128 x N=C x K16 against the weight tile (built once per CTA), fp32 in TMEM

@@ -1,7 +1,6 @@
-// HBM-bound kernels of the path: fbank CMVN, conv1 (Cin=1, K=9: no tensor cores), LayerNorm,
-// sinusoidal table, padding mask, and the weight-format preparation kernels.
+// HBM-bound kernels of the path: fbank CMVN, LayerNorm, sinusoidal table, padding mask, and the
+// weight-format preparation kernels; also the conv1 entry points (the kernel is in conv1_tcgen05.cu).
 #include <math.h>
-#include <stdlib.h>
 
 #include <cuda_fp16.h>
 
@@ -181,75 +180,6 @@ __global__ void __launch_bounds__(256)
       o.w = (v.w - m4.w) * i4.w;
     }
     yp[(size_t)t * Q] = o;
-  }
-}
-
-// ----------------------------------------------------------------- conv1 (a2)
-// MEASURED ALTERNATIVE (r01g, not kept): a persistent version that stages the (2*R1+1) x (F+2) input patch
-// of 8 output rows in shared memory (double-buffered, next patch prefetched into registers), reads the 9
-// taps with broadcast LDS and accumulates channel pairs with packed fp32 FMAs was SLOWER (75.8 us vs 67.6
-// us here at cfg2) although it removes every global-load stall from the pixel loop: the kernel is not
-// bound by its input loads.  The next step for conv1 is the tensor pipe (im2col K=9->16 in smem, one UMMA
-// per 128 pixels, TMEM epilogue), which cuts the instruction count ~4x.
-// Thread = (output row (b,t1), 8-channel group g): the 72 weights + 24 epilogue constants of the
-// group live in registers; the thread slides along the F1 output columns of its row (stride-2
-// window: 6 new inputs per pixel, no index division in the loop).  The 8 threads of a pixel write
-// its 128 contiguous bytes of channels-last bf16 output.
-template <int C>
-__global__ void __launch_bounds__(256, 2)
-    conv1_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                 const float* __restrict__ bias, const float* __restrict__ scale,
-                 const float* __restrict__ shift, uint4* __restrict__ y, int B, int T, int F, int T1,
-                 int F1) {
-  constexpr int G = C / 8;
-  const int g = threadIdx.x % G;
-  float wr[8][9], br[8], sr[8], hr[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const int c = g * 8 + j;
-#pragma unroll
-    for (int k = 0; k < 9; ++k) wr[j][k] = __ldg(w + c * 9 + k);
-    br[j] = __ldg(bias + c);
-    sr[j] = __ldg(scale + c);
-    hr[j] = __ldg(shift + c);
-  }
-  const int rows_per_block = blockDim.x / G;
-  const int total_rows = B * T1;
-  for (int row = blockIdx.x * rows_per_block + threadIdx.x / G; row < total_rows;
-       row += gridDim.x * rows_per_block) {
-    const int t1 = row % T1, b = row / T1;
-    const float* xr[3];
-    bool ok[3];
-#pragma unroll
-    for (int kh = 0; kh < 3; ++kh) {
-      const int t = 2 * t1 - 1 + kh;
-      ok[kh] = (t >= 0 && t < T);
-      xr[kh] = x + ((size_t)b * T + (ok[kh] ? t : 0)) * F;
-    }
-    float in[9];
-#pragma unroll
-    for (int kh = 0; kh < 3; ++kh) in[kh * 3 + 2] = 0.0f;  // column -1 (left zero padding)
-    uint4* yp = y + (size_t)row * F1 * G + g;
-    for (int f1 = 0; f1 < F1; ++f1) {
-      const int f = 2 * f1;
-#pragma unroll
-      for (int kh = 0; kh < 3; ++kh) {
-        in[kh * 3 + 0] = in[kh * 3 + 2];
-        in[kh * 3 + 1] = (ok[kh] && f < F) ? __ldg(xr[kh] + f) : 0.0f;
-        in[kh * 3 + 2] = (ok[kh] && f + 1 < F) ? __ldg(xr[kh] + f + 1) : 0.0f;
-      }
-      float o[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        float a = br[j];
-#pragma unroll
-        for (int k = 0; k < 9; ++k) a = fmaf(wr[j][k], in[k], a);
-        a = fmaxf(a, 0.0f);
-        o[j] = fmaf(a, sr[j], hr[j]);
-      }
-      yp[(size_t)f1 * G] = make_uint4(pack_f16x2(o[0], o[1]), pack_f16x2(o[2], o[3]),
-                                      pack_f16x2(o[4], o[5]), pack_f16x2(o[6], o[7]));
-    }
   }
 }
 
@@ -542,17 +472,7 @@ extern "C" int fbkst_conv1_relu_bn(const float* x, const float* w, const float* 
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int T1 = (T + 1) / 2, F1 = (F + 1) / 2;
   FBKST_REQUIRE((long long)B * T1 * F1 < (1ll << 31), "fbkst_conv1_relu_bn: too many pixels");
-  // default: the tcgen05 kernel (conv1_tcgen05.cu); FBKST_CONV1_SIMT=1 selects the SIMT kernel above
-  static const bool simt = getenv("FBKST_CONV1_SIMT") != nullptr;
-  if (!simt) return conv1_tc_dispatch(x, w, bias, bn_scale, bn_shift, y, B, T, F, C, T1, F1, 0, st);
-  const long long total = (long long)B * T1 * (C / 8);
-  const int grid = grid_for(total, 256, 8);
-  if (C == 64)
-    conv1_kernel<64><<<grid, 256, 0, st>>>(x, w, bias, bn_scale, bn_shift, (uint4*)y, B, T, F, T1, F1);
-  else
-    conv1_kernel<128><<<grid, 256, 0, st>>>(x, w, bias, bn_scale, bn_shift, (uint4*)y, B, T, F, T1, F1);
-  FBKST_CHECK_CUDA(cudaGetLastError());
-  return FBKST_OK;
+  return conv1_tc_dispatch(x, w, bias, bn_scale, bn_shift, y, B, T, F, C, T1, F1, 0, st);
 }
 
 extern "C" int fbkst_conv1_relu_bn_planes(const float* x, const float* w, const float* bias,

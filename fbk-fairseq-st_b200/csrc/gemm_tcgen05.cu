@@ -6,12 +6,12 @@
 //   warps 4-7   epilogue          (tcgen05.ld -> bias/ReLU/residual/pos-emb -> global)
 //
 // Tile 128 x BN x 64, STAGES-deep smem ring, two TMEM accumulator stages so that the epilogue
-// of tile i overlaps the main loop of tile i+1.  Replaces every nn.Linear on the reference
-// path (conv_transformer.py:227,279; local_attention.py:178,141; transformer_layer.py:131-133).
+// of tile i overlaps the main loop of tile i+1.  It serves the row-remap / position-embedding
+// epilogues; fbkst_linear_bf16 sends every other nn.Linear of the reference path
+// (conv_transformer.py:227,279; local_attention.py:178,141; transformer_layer.py:131-133) to the
+// CTA-pair kernel of gemm2_tcgen05.cu.
 #include "host_common.h"
 #include "ptx.cuh"
-
-#include <stdlib.h>
 
 namespace fbkst {
 
@@ -253,335 +253,6 @@ __global__ void __launch_bounds__(256, 1)
   }
 }
 
-__device__ __forceinline__ float4 bcast4(const float4& v, int src_lane) {
-  return make_float4(__shfl_sync(0xffffffffu, v.x, src_lane), __shfl_sync(0xffffffffu, v.y, src_lane),
-                     __shfl_sync(0xffffffffu, v.z, src_lane), __shfl_sync(0xffffffffu, v.w, src_lane));
-}
-
-// ------------------------------------------------------------------------------------------
-// v2: 128 x 256 tiles, EIGHT epilogue warps (two per TMEM lane quarter, each owning 128 columns),
-// bias staged in smem, outputs staged through swizzled smem and written with per-warp TMA stores
-// (coalesced, asynchronous, no LSU wavefront per row), residual tiles prefetched with per-warp TMA
-// loads into the same staging buffers.  A row-per-thread global store costs one L1 wavefront per
-// 16 bytes (4096-8192 per tile, i.e. as long as the whole K=512 main loop); the TMA path removes it.
-template <bool OUT_F32, bool RESID, int STAGES>
-__global__ void __launch_bounds__(384, 1)
-    gemm_tma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                    const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmR,
-                    int M, int N, int K, const float* __restrict__ bias, int relu) {
-  constexpr int BN = 256;
-  constexpr int A_BYTES = BM * BK * 2;
-  constexpr int B_BYTES = BN * BK * 2;
-  constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  constexpr int EPI_BUFS = RESID ? 2 : 1;
-  constexpr int EPI_BYTES = 8 * EPI_BUFS * 4096;
-  constexpr uint32_t TMEM_COLS = 2 * BN;
-  constexpr uint32_t IDESC = idesc_bf16_f32(BM, BN, 0, 0);
-
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);  // keeps .shared
-  uint8_t* smem_epi = smem + STAGES * STAGE_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_epi + EPI_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* tfull_bar = empty_bar + STAGES;
-  uint64_t* tempty_bar = tfull_bar + 2;
-  uint64_t* res_bar = tempty_bar + 2;  // [8][2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_bar + 16);
-
-  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
-  const int lane = threadIdx.x & 31;
-  const int num_n = (N + BN - 1) / BN;
-  const int num_m = (M + BM - 1) / BM;
-  const int num_tiles = num_m * num_n;
-  const int num_kb = (K + BK - 1) / BK;
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
-    tma_prefetch_desc(&tmO);
-    if (RESID) tma_prefetch_desc(&tmR);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&tfull_bar[s], 1);
-      mbar_init(&tempty_bar[s], 8);
-    }
-    for (int s = 0; s < 16; ++s) mbar_init(&res_bar[s], 1);
-    fence_barrier_init();
-  }
-  if (warp == 2) {
-    tmem_alloc(tmem_slot, TMEM_COLS);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int m_blk = tile / num_n, n_blk = tile - m_blk * num_n;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&empty_bar[stage], phase ^ 1);
-          mbar_arrive_expect_tx(&full_bar[stage], STAGE_BYTES);
-          uint8_t* sa = smem + stage * STAGE_BYTES;
-          tma_load_2d(sa, &tmA, &full_bar[stage], kb * BK, m_blk * BM);
-          tma_load_2d(sa + A_BYTES, &tmB, &full_bar[stage], kb * BK, n_blk * BN);
-          if (++stage == STAGES) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      int acc = 0;
-      uint32_t acc_phase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * BN;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after();
-          const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES);
-          const uint64_t adesc = desc_kmajor_sw128(sa);
-          const uint64_t bdesc = desc_kmajor_sw128(sa + A_BYTES);
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k)
-            umma_bf16_ss(d_tmem, adesc + 2 * k, bdesc + 2 * k, IDESC, (kb | k) != 0);
-          umma_commit(&empty_bar[stage]);
-          if (++stage == STAGES) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
-        umma_commit(&tfull_bar[acc]);
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-      }
-    }
-  } else if (warp >= 4) {
-    const int ew = warp - 4;
-    const int q = ew & 3;      // TMEM lane quarter == row block of 32
-    const int half = ew >> 2;  // column half of the tile
-    uint8_t* stg = smem_epi + ew * EPI_BUFS * 4096;
-    uint64_t* rbar = res_bar + ew * 2;
-    uint32_t rphase[2] = {0, 0};
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    const int swz = lane & 7;
-    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-      const int m_blk = tile / num_n, n_blk = tile - m_blk * num_n;
-      const int m0 = m_blk * BM + q * 32;
-      const int n0 = n_blk * BN + half * 128;
-      if (n0 >= N) {  // this warp's column half is entirely out of range (warp-uniform)
-        mbar_wait(&tfull_bar[acc], acc_phase);
-        tc_fence_before();
-        if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-        acc ^= 1;
-        if (acc == 0) acc_phase ^= 1;
-        continue;
-      }
-      // bias slice of this warp (128 columns): lane l keeps columns 4l..4l+3, broadcast by shuffle
-      // (with the maximum smem carve-out there is no L1 left to serve repeated __ldg).
-      float4 b4 = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (bias != nullptr) {
-        const int c = n0 + lane * 4;
-        if (c + 3 < N) {
-          b4 = __ldg(reinterpret_cast<const float4*>(bias + c));
-        } else {
-          if (c + 0 < N) b4.x = __ldg(bias + c + 0);
-          if (c + 1 < N) b4.y = __ldg(bias + c + 1);
-          if (c + 2 < N) b4.z = __ldg(bias + c + 2);
-        }
-      }
-      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN + half * 128;
-      if (RESID) {  // fp32 out, 4 units of 32 columns, residual prefetched one unit ahead
-        if (lane == 0) {
-          tma_store_wait_read<0>();
-          mbar_arrive_expect_tx(&rbar[0], 4096);
-          tma_load_2d(stg, &tmR, &rbar[0], n0, m0);
-        }
-        mbar_wait(&tfull_bar[acc], acc_phase);
-        tc_fence_after();
-        uint32_t v[32];
-        tmem_ld32(taddr, v);
-#pragma unroll 1
-        for (int u = 0; u < 4; ++u) {
-          const int col0 = n0 + u * 32;
-          if (col0 >= N) break;
-          const int bsel = u & 1;
-          if (u + 1 < 4 && col0 + 32 < N && lane == 0) {  // prefetch the next residual unit
-            tma_store_wait_read<0>();                    // its buffer was read by store(u-1)
-            mbar_arrive_expect_tx(&rbar[bsel ^ 1], 4096);
-            tma_load_2d(stg + (bsel ^ 1) * 4096, &tmR, &rbar[bsel ^ 1], col0 + 32, m0);
-          }
-          tmem_ld_wait();
-          float f[32];
-#pragma unroll
-          for (int j = 0; j < 32; ++j) f[j] = __uint_as_float(v[j]);
-          if (u + 1 < 4) tmem_ld32(taddr + (u + 1) * 32, v);
-          mbar_wait(&rbar[bsel], rphase[bsel]);
-          rphase[bsel] ^= 1;
-          uint8_t* rowp = stg + bsel * 4096 + lane * 128;
-#pragma unroll
-          for (int g = 0; g < 8; ++g) {
-            const float4 bb = bcast4(b4, u * 8 + g);
-            float4* sp = reinterpret_cast<float4*>(rowp + ((g ^ swz) << 4));
-            float4 r = *sp;
-            float a0 = f[4 * g] + bb.x, a1 = f[4 * g + 1] + bb.y, a2 = f[4 * g + 2] + bb.z,
-                  a3 = f[4 * g + 3] + bb.w;
-            if (relu) {
-              a0 = fmaxf(a0, 0.f);
-              a1 = fmaxf(a1, 0.f);
-              a2 = fmaxf(a2, 0.f);
-              a3 = fmaxf(a3, 0.f);
-            }
-            r.x += a0;
-            r.y += a1;
-            r.z += a2;
-            r.w += a3;
-            *sp = r;
-          }
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (lane == 0) {
-            tma_store_2d(&tmO, stg + bsel * 4096, col0, m0);
-            tma_store_commit();
-          }
-        }
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-      } else {
-        mbar_wait(&tfull_bar[acc], acc_phase);
-        tc_fence_after();
-        constexpr int UNITS = OUT_F32 ? 4 : 2;  // staging rows are 128 B: 32 fp32 or 64 bf16 columns
-        constexpr int UCOLS = OUT_F32 ? 32 : 64;
-#pragma unroll 1
-        for (int u = 0; u < UNITS; ++u) {
-          const int col0 = n0 + u * UCOLS;
-          if (col0 >= N) break;
-          uint32_t v0[32], v1[32];
-          tmem_ld32(taddr + u * UCOLS, v0);
-          if (!OUT_F32) tmem_ld32(taddr + u * UCOLS + 32, v1);
-          if (lane == 0) tma_store_wait_read<0>();  // staging buffer free again
-          tmem_ld_wait();
-          __syncwarp();
-          uint8_t* rowp = stg + lane * 128;
-          if (OUT_F32) {
-#pragma unroll
-            for (int g = 0; g < 8; ++g) {
-              const float4 bb = bcast4(b4, u * 8 + g);
-              float a0 = __uint_as_float(v0[4 * g]) + bb.x, a1 = __uint_as_float(v0[4 * g + 1]) + bb.y,
-                    a2 = __uint_as_float(v0[4 * g + 2]) + bb.z, a3 = __uint_as_float(v0[4 * g + 3]) + bb.w;
-              if (relu) {
-                a0 = fmaxf(a0, 0.f);
-                a1 = fmaxf(a1, 0.f);
-                a2 = fmaxf(a2, 0.f);
-                a3 = fmaxf(a3, 0.f);
-              }
-              *reinterpret_cast<float4*>(rowp + ((g ^ swz) << 4)) = make_float4(a0, a1, a2, a3);
-            }
-          } else {
-#pragma unroll
-            for (int g = 0; g < 8; ++g) {
-              const uint32_t* src = (g < 4) ? v0 : v1;
-              const int o = (g & 3) * 8;
-              const float4 b0 = bcast4(b4, u * 16 + 2 * g);
-              const float4 b1 = bcast4(b4, u * 16 + 2 * g + 1);
-              float a[8] = {__uint_as_float(src[o]) + b0.x,     __uint_as_float(src[o + 1]) + b0.y,
-                            __uint_as_float(src[o + 2]) + b0.z, __uint_as_float(src[o + 3]) + b0.w,
-                            __uint_as_float(src[o + 4]) + b1.x, __uint_as_float(src[o + 5]) + b1.y,
-                            __uint_as_float(src[o + 6]) + b1.z, __uint_as_float(src[o + 7]) + b1.w};
-              if (relu) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j) a[j] = fmaxf(a[j], 0.f);
-              }
-              *reinterpret_cast<uint4*>(rowp + ((g ^ swz) << 4)) =
-                  make_uint4(pack_bf16x2(a[0], a[1]), pack_bf16x2(a[2], a[3]), pack_bf16x2(a[4], a[5]),
-                             pack_bf16x2(a[6], a[7]));
-            }
-          }
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (lane == 0) {
-            tma_store_2d(&tmO, stg, col0, m0);
-            tma_store_commit();
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-      }
-      acc ^= 1;
-      if (acc == 0) acc_phase ^= 1;
-    }
-    if (lane == 0) tma_store_wait<0>();
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, TMEM_COLS);
-  }
-}
-
-template <bool OUT_F32, bool RESID, int STAGES>
-static int launch_gemm_tma(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias,
-                           const float* resid, int64_t ldr, void* out, int64_t ldo, int M, int N,
-                           int K, int relu, cudaStream_t stream) {
-  constexpr int BN = 256;
-  constexpr int SMEM = STAGES * (BM * BK * 2 + BN * BK * 2) + 8 * (RESID ? 2 : 1) * 4096 + 1024 + 512;
-  static_assert(SMEM <= 232448, "shared memory budget exceeded");
-  auto kern = gemm_tma_kernel<OUT_F32, RESID, STAGES>;
-  static PerDeviceFlag configured;
-  if (!configured) {
-    FBKST_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    configured = true;
-  }
-  CUtensorMap tmA, tmB, tmO, tmR;
-  int rc = make_tensor_map_2d_bf16(&tmA, A, (uint64_t)M, (uint64_t)K, (uint64_t)lda, BM, BK);
-  if (rc) return rc;
-  rc = make_tensor_map_2d_bf16(&tmB, W, (uint64_t)N, (uint64_t)K, (uint64_t)ldw, BN, BK);
-  if (rc) return rc;
-  {
-    uint64_t dims[2] = {(uint64_t)N, (uint64_t)M};
-    uint64_t strides[1] = {(uint64_t)ldo * (OUT_F32 ? 4 : 2)};
-    uint32_t box[2] = {OUT_F32 ? 32u : 64u, 32u};
-    rc = make_tensor_map(&tmO, out,
-                         OUT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16,
-                         OUT_F32 ? 4 : 2, 2, dims, strides, box, nullptr);
-    if (rc) return rc;
-  }
-  if (RESID) {
-    uint64_t dims[2] = {(uint64_t)N, (uint64_t)M};
-    uint64_t strides[1] = {(uint64_t)ldr * 4};
-    uint32_t box[2] = {32u, 32u};
-    rc = make_tensor_map(&tmR, resid, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, 2, dims, strides, box, nullptr);
-    if (rc) return rc;
-  } else {
-    tmR = tmO;
-  }
-  const int tiles = ((M + BM - 1) / BM) * ((N + BN - 1) / BN);
-  const int grid = tiles < num_sms() ? tiles : num_sms();
-  kern<<<grid, 384, SMEM, stream>>>(tmA, tmB, tmO, tmR, M, N, K, bias, relu);
-  FBKST_CHECK_CUDA(cudaGetLastError());
-  return FBKST_OK;
-}
-
 template <int BN, int STAGES>
 static int launch_gemm(const void* A, int64_t lda, const void* W, int64_t ldw, int M, int N, int K,
                        const EpiParams& ep, cudaStream_t stream) {
@@ -645,20 +316,9 @@ extern "C" int fbkst_linear_bf16(const void* A, int64_t lda, const void* W, int6
   const int relu = (flags & FBKST_EPI_RELU) ? 1 : 0;
   if (residual != nullptr)
     FBKST_REQUIRE(flags & FBKST_EPI_OUT_F32, "fbkst_linear_bf16: a residual requires fp32 output");
-  static const bool single_cta = getenv("FBKST_GEMM_1CTA") != nullptr;  // A/B switch for profiling
-  if (!single_cta)
-    return linear_pair_dispatch(A, lda, W, ldw, bias, residual, ldr, out, ldo, M, N, K, relu,
-                                (flags & FBKST_EPI_OUT_F32) ? 1 : 0, m_limit, m_limit_mult, nullptr, 0.f,
-                                nullptr, 0, nullptr, (flags & FBKST_EPI_AB_F16) ? 1 : 0, st);
-  FBKST_REQUIRE(!(flags & FBKST_EPI_AB_F16), "fbkst_linear_bf16: fp16 operands need the CTA-pair kernel");
-  FBKST_REQUIRE(m_limit == nullptr, "fbkst_linear_bf16: m_limit is not supported by the single-CTA kernel "
-                                    "(FBKST_GEMM_1CTA)");
-  if (residual != nullptr) {
-    return launch_gemm_tma<true, true, 3>(A, lda, W, ldw, bias, residual, ldr, out, ldo, M, N, K, relu, st);
-  }
-  if (flags & FBKST_EPI_OUT_F32)
-    return launch_gemm_tma<true, false, 4>(A, lda, W, ldw, bias, nullptr, 0, out, ldo, M, N, K, relu, st);
-  return launch_gemm_tma<false, false, 4>(A, lda, W, ldw, bias, nullptr, 0, out, ldo, M, N, K, relu, st);
+  return linear_pair_dispatch(A, lda, W, ldw, bias, residual, ldr, out, ldo, M, N, K, relu,
+                              (flags & FBKST_EPI_OUT_F32) ? 1 : 0, m_limit, m_limit_mult, nullptr, 0.f, nullptr, 0,
+                              nullptr, (flags & FBKST_EPI_AB_F16) ? 1 : 0, st);
 }
 
 extern "C" int fbkst_linear_ln_bf16(const void* A, int64_t lda, const void* W, int64_t ldw,

@@ -29,7 +29,7 @@ from . import ops
 # A/B switch: FBKST_CONV_PLANES=1 makes conv1 write four (t1, f1)-parity planes so that conv2's stride-2 taps
 # are unit-stride TMA boxes.  Bit-identical output (tests/test_gpu_ops.py), but measured time-neutral
 # (conv2 51.2 us either way at cfg2), so the reference layout [B,T1,F1,C] stays the default.
-_CONV_PLANES = os.environ.get("FBKST_CONV_PLANES", "0") == "1" and "FBKST_CONV1_SIMT" not in os.environ
+_CONV_PLANES = os.environ.get("FBKST_CONV_PLANES", "0") == "1"
 
 try:  # plug into fairseq when it is importable (train.py / generate.py --user-dir)
     from fairseq.models import FairseqEncoder as _Base  # type: ignore

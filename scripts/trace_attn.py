@@ -1,4 +1,4 @@
-"""Timeline of CTA 0 of the attention kernel (debug hook fbkst_debug_set_attention_trace)."""
+"""Timeline of CTA 0 of the wide attention kernel (debug hook fbkst_debug_set_attention_wide_trace)."""
 import ctypes
 import os
 import sys
@@ -10,7 +10,7 @@ sys.path.insert(0, os.path.join(ROOT, "fbk-fairseq-st_b200"))
 from fbkst_b200 import _lib, ops  # noqa: E402
 
 lib = _lib.load()
-lib.fbkst_debug_set_attention_trace.argtypes = [ctypes.c_void_p]
+lib.fbkst_debug_set_attention_wide_trace.argtypes = [ctypes.c_void_p]
 d = torch.device("cuda:0")
 L, B, H = 375, 64, 8
 qkv = (torch.randn(L * B, 3 * H * 64, device=d) * 0.7).bfloat16()
@@ -25,37 +25,14 @@ ops.attention = lambda *a, **k: _attention(*a, q_limit=q_limit, **k)
 for _ in range(3):
     ops.attention(qkv, lengths, L, B, H, True)
 buf = torch.zeros(64 * 16, dtype=torch.int64, device=d)
-if os.environ.get("FBKST_ATTN_WIDE", "1") != "0":
-    # wide kernel (attention_wide.cu): its own hook and column set
-    lib.fbkst_debug_set_attention_wide_trace.argtypes = [ctypes.c_void_p]
-    assert lib.fbkst_debug_set_attention_wide_trace(buf.data_ptr()) == 0
-    ops.attention(qkv, lengths, L, B, H, True)
-    torch.cuda.synchronize()
-    lib.fbkst_debug_set_attention_wide_trace(None)
-    t = buf.view(64, 16).cpu()
-    t0 = int(t[t > 0].min())
-    order = [(14, "tma:K"), (11, "mma:QK"), (0, "s_full"), (1, "S_regs"), (2, "guard"), (3, "P_done"), (4, "P_free"),
-             (5, "p_full"), (12, "mma:PV"), (9, "last_pv"), (10, "stored")]
-    print("tile " + " ".join("%9s" % n for _, n in order))
-    for i in range(40):
-        print("%4d " % i + " ".join("%9d" % (int(t[i][k]) - t0 if t[i][k] > 0 else -1) for k, _ in order))
-    sys.exit(0)
-assert lib.fbkst_debug_set_attention_trace(buf.data_ptr()) == 0
+assert lib.fbkst_debug_set_attention_wide_trace(buf.data_ptr()) == 0
 ops.attention(qkv, lengths, L, B, H, True)
 torch.cuda.synchronize()
-lib.fbkst_debug_set_attention_trace(None)
-t = buf.view(64, 16).cpu()[:, :13]
+lib.fbkst_debug_set_attention_wide_trace(None)
+t = buf.view(64, 16).cpu()
 t0 = int(t[t > 0].min())
-if os.environ.get("FBKST_TRACE_SOFTMAX"):
-    # decoupled one-pass kernel, softmax warp of each group (rows: even = group 0, odd = group 1), in time order
-    order = [(3, "s_full"), (8, "ld_a"), (4, "max_a"), (5, "pv_lo_ok"), (9, "ld_b"), (10, "s_free"), (11, "p_lo"),
-             (12, "pv_hi_ok"), (0, "ch7"), (6, "p_hi"), (7, "epilogue")]
-    print("tile " + " ".join("%9s" % n for _, n in order))
-    for i in range(40):
-        print("%4d " % i + " ".join("%9d" % (int(t[i][k]) - t0 if t[i][k] > 0 else -1) for k, _ in order))
-    sys.exit(0)
-names = ["mma:p_full", "mma:PV", "mma:QK+2", "sm:s_full", "sm:pass1", "sm:PO_free", "sm:arrive", "epilogue",
-         "mma:s_free", "mma:k_full", "tma:K", "tma:V", "mma:v_full"]
-print("tile " + " ".join("%11s" % n for n in names))
+order = [(14, "tma:K"), (11, "mma:QK"), (0, "s_full"), (1, "S_regs"), (2, "guard"), (3, "P_done"), (4, "P_free"),
+         (5, "p_full"), (12, "mma:PV"), (9, "last_pv"), (10, "stored")]
+print("tile " + " ".join("%9s" % n for _, n in order))
 for i in range(40):
-    print("%4d " % i + " ".join("%11d" % (int(v) - t0 if v > 0 else -1) for v in t[i]))
+    print("%4d " % i + " ".join("%9d" % (int(t[i][k]) - t0 if t[i][k] > 0 else -1) for k, _ in order))

@@ -3,7 +3,7 @@
 ``ops.attention`` (bf16) picks its kernel by shape alone (``attention_entry``, csrc/attention_tcgen05.cu):
 the wide kernel (attention_wide.cu, 128-key tiles) whenever its shared memory fits -- always without the
 penalty, L <= 2560 with it, where the penalty LUT fills shared memory -- and otherwise the split-KV kernel
-``attention_fwd_kernel<1>`` (64-key tiles) up to L = 17216; beyond that the call is refused.  The cases below sit
+``attention_fwd_kernel`` (64-key tiles) up to L = 17216; beyond that the call is refused.  The cases below sit
 on the edges where such kernels go wrong: lengths at tile multiples +-1, tiles made only of padding, odd work-item
 counts (an idle softmax group in the wide kernel), more than the 64 work items per CTA that both kernels keep
 decoded in shared memory, the first L of each kernel, the largest L each accepts, and more than 255 key tiles per
@@ -27,12 +27,11 @@ TOL_XATTN_F32 = (1e-5, 1e-6)   # fp32 cross-attention (test_gpu_xattn_fp32.py)
 
 # ---------------------------------------------------------------------------------- host-side restatement
 # Shared memory of the inference kernels as the launch code computes it (attention_wide.cu: aw_smem_bytes;
-# attention_tcgen05.cu: attention_smem_bytes, attention_dec_smem_bytes; cross_attention.cu: xattn_smem_bytes).
+# attention_tcgen05.cu: attention_smem_bytes; cross_attention.cu: xattn_smem_bytes).
 SMEM_MAX = 227 * 1024       # per CTA
 SMEM_SM = 228 * 1024        # per SM (1 KB of it reserved per resident CTA)
 AW_SMEM_FIXED = 2 * 16384 + 3 * 16384 + 2 * 16384 + 2 * 16384 + 256 + 64 * 16 + 1024
 AT_SMEM_FIXED = 16384 + 3 * 8192 + 2 * 8192 + 2 * 16384 + 256 + 2 * 2 * 128 * 4 + 64 * 16 + 1024
-ATD_SMEM_FIXED = 2 * 16384 + 3 * 8192 + 2 * 8192 + 2 * 16384 + 256 + 64 * 16 + 1024
 ITEM_TABLE = 64             # AW_TABLE / AT_TABLE: work items per CTA decoded once into shared memory
 
 
@@ -44,8 +43,8 @@ def wide_smem(L, pen):
     return AW_SMEM_FIXED + (4 * (4 * 2 * 128 * _ceil(L, 128) + 32) if pen else 0)
 
 
-def split_smem(L, pen, fixed=AT_SMEM_FIXED):
-    return fixed + (4 * (128 * _ceil(L, 128) + 64 * _ceil(L, 64)) if pen else 0)
+def split_smem(L, pen):
+    return AT_SMEM_FIXED + (4 * (128 * _ceil(L, 128) + 64 * _ceil(L, 64)) if pen else 0)
 
 
 def dispatch(L, B, H, pen, sms):
@@ -53,8 +52,6 @@ def dispatch(L, B, H, pen, sms):
     n_items = _ceil(L, 128) * B * H
     if wide_smem(L, pen) <= SMEM_MAX:
         return "attention_fwd_wide_kernel", sms if 2 * sms <= n_items else (n_items + 1) // 2
-    if 2 * (split_smem(L, pen, ATD_SMEM_FIXED) + 1024) <= SMEM_SM:
-        return "attention_fwd_dec_kernel", min(2 * sms, n_items)
     smem = split_smem(L, pen)
     if smem > SMEM_MAX:
         return None, 0
@@ -75,8 +72,6 @@ def test_dispatch_limits():
     assert largest(lambda L: wide_smem(L, True) <= SMEM_MAX) == 2560
     assert wide_smem(10 ** 6, False) <= SMEM_MAX  # no penalty: no LUT, any L
     assert largest(lambda L: split_smem(L, True) <= SMEM_MAX) == 17216
-    # the decoupled kernel fits two CTAs per SM only where the wide kernel already serves
-    assert largest(lambda L: 2 * (split_smem(L, True, ATD_SMEM_FIXED) + 1024) <= SMEM_SM) < 2560
     for L, kernel in [(2560, "attention_fwd_wide_kernel"), (2561, "attention_fwd_kernel"),
                       (17216, "attention_fwd_kernel"), (17217, None)]:
         assert dispatch(L, 1, 1, True, 148)[0] == kernel
@@ -248,8 +243,8 @@ def test_attention_bf16_vs_fp64(case):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("L,pen,kernel", [(2560, True, "attention_fwd_wide_kernel<1>"),
-                                          (2561, True, "attention_fwd_kernel<1>"),
-                                          (17216, True, "attention_fwd_kernel<1>"),
+                                          (2561, True, "attention_fwd_kernel"),
+                                          (17216, True, "attention_fwd_kernel"),
                                           (40000, False, "attention_fwd_wide_kernel<0>")])
 def test_attention_dispatch(L, pen, kernel):
     """The kernel each side of a dispatch limit actually runs; past the last one the call is refused."""
