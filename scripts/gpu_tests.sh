@@ -18,6 +18,7 @@ run ctc tests/test_gpu_ops.py -k "ctc"
 run conv tests/test_gpu_ops.py -k "conv_stack"
 run attn tests/test_gpu_ops.py -k "attention"
 run attn_edges tests/test_attention_edges.py
+run attn_train_edges tests/test_attention_train_edges.py
 run encoder tests/test_gpu_encoder.py
 run misc tests/test_gpu_ops.py -k "custom_ops or collater"
 run criterion tests/test_gpu_criterion.py
