@@ -71,32 +71,11 @@ __device__ __forceinline__ float ex2(float x) {
   return y;
 }
 
-// 2^x on the FMA/ALU pipes for part of every row (Cody-Waite range reduction + degree-3 minimax
-// polynomial, max rel. error 7.5e-5 -- far below the bf16 rounding of P): the MUFU pipe runs 16 ex2
-// per clock and SM, i.e. 512 clocks for a 128x64 tile whose two UMMAs need 256, so with head_dim 64
-// the exponentials -- not the tensor pipe -- set the floor.  AT_NPOLY of every 4 register pairs
-// take this path (0 = all MUFU).  x is clamped at -126 (2^-126 * p is ~1e-38, i.e. zero in P).
-// MEASURED (profiles/r01f_attention_poly_ab.txt): every pair moved off the MUFU makes the kernel
-// SLOWER (cfg2 L=375: 61.4 / 63.5 / 65.5 / 67.6 us for 0..3 of 4) -- the softmax warps are bound by
-// issue slots and the MMA round trip, not by the MUFU pipe, so the default stays 0.
-#ifndef FBKST_ATTN_NPOLY
-#define FBKST_ATTN_NPOLY 0
-#endif
-constexpr int AT_NPOLY = FBKST_ATTN_NPOLY;
-__device__ __forceinline__ float2 ex2_poly2(float2 x) {
-  const float kMagic = 12582912.0f;  // 1.5 * 2^23: the integer part of x lands in the low mantissa bits
-  x.x = fmaxf(x.x, -126.0f);
-  x.y = fmaxf(x.y, -126.0f);
-  const float2 r = fadd2(x, make_float2(kMagic, kMagic));
-  const float2 n = fadd2(r, make_float2(-kMagic, -kMagic));
-  const float2 f = ffma2(n, make_float2(-1.0f, -1.0f), x);  // x - round(x) in [-0.5, 0.5]
-  float2 p = ffma2(f, make_float2(0.0551716648f, 0.0551716648f), make_float2(0.2426111251f, 0.2426111251f));
-  p = ffma2(p, f, make_float2(0.6932609677f, 0.6932609677f));
-  p = ffma2(p, f, make_float2(0.9999280572f, 0.9999280572f));
-  p.x = __uint_as_float(__float_as_uint(p.x) + (__float_as_uint(r.x) << 23));
-  p.y = __uint_as_float(__float_as_uint(p.y) + (__float_as_uint(r.y) << 23));
-  return p;
-}
+// Every exponential runs on the MUFU pipe: 16 ex2 per clock and SM, i.e. 512 clocks for a 128x64 tile
+// whose two UMMAs need 256.  Moving part of each row to an FMA-pipe polynomial 2^x (Cody-Waite + degree-3
+// minimax) was MEASURED slower (profiles/r01f_attention_poly_ab.txt, cfg2 L=375: 61.4 / 63.5 / 65.5 /
+// 67.6 us for 0..3 of every 4 register pairs): the softmax warps are bound by issue slots and the MMA
+// round trip, not by the MUFU pipe.
 
 // Static work list of a CTA: items w = blockIdx.x, blockIdx.x + gridDim.x, ...; item index
 // w = (b*H + h)*nq + q_tile, so CTAs running side by side share K/V of one (b, h) through L2.
@@ -471,12 +450,8 @@ __global__ void __launch_bounds__(AT_THREADS, 2)
             }
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-              if (c < AT_NPOLY) {
-                t[c] = ex2_poly2(t[c]);
-              } else {
-                t[c].x = ex2(t[c].x);
-                t[c].y = ex2(t[c].y);
-              }
+              t[c].x = ex2(t[c].x);
+              t[c].y = ex2(t[c].y);
             }
 #pragma unroll
             for (int c = 0; c < 4; ++c) sm2[c & 1] = fadd2(sm2[c & 1], t[c]);

@@ -50,21 +50,13 @@ constexpr int AW_BN = 128;  // keys per tile
 constexpr int AW_HD = 64;
 constexpr int AW_QB = AW_BM * AW_HD * 2;  // 16 KB
 constexpr int AW_KB = AW_BN * AW_HD * 2;  // 16 KB (K tile; V tile = two 8 KB halves)
-// P handed to the PV product through tensor memory (A operand of tcgen05.mma from TMEM) instead of two
+// P is handed to the PV product through tensor memory (A operand of tcgen05.mma from TMEM), not through two
 // swizzled shared-memory sub-tiles: no 64 KB store + 64 KB operand fetch per tile pair on the 128 B/clk
-// shared-memory path, no generic -> async proxy fence.  0 = shared memory (A/B switch).
-#ifndef FBKST_AW_PTMEM
-#define FBKST_AW_PTMEM 1
-#endif
-// per-group shared-memory tile behind sP: the output staging rows (4 warps x 32 rows x 128 B) and, without
-// FBKST_AW_PTMEM, the whole 128 x 128 bf16 P tile
-constexpr int AW_PB = FBKST_AW_PTMEM ? AW_BM * AW_HD * 2 : AW_BM * AW_BN * 2;  // 16 KB / 32 KB
-constexpr int AW_PSUB = AW_BM * AW_HD * 2;  // one 64-key sub-tile of P (FBKST_AW_PTMEM=0)
-#ifndef FBKST_AW_KST
-#define FBKST_AW_KST 3
-#endif
-static_assert(FBKST_AW_KST >= 2 && FBKST_AW_KST <= 4, "K ring: 2..4 stages");
-constexpr int AW_KST = FBKST_AW_KST;  // K ring stages (4 measured the same: r02z_attention_wide.txt)
+// shared-memory path, no generic -> async proxy fence (profiles/r02z_attention_wide.txt).
+// Per-group shared-memory tile behind sP: the output staging rows (4 warps x 32 rows x 128 B).
+constexpr int AW_PB = AW_BM * AW_HD * 2;  // 16 KB
+constexpr int AW_KST = 3;  // K ring stages (4 measured the same: r02z_attention_wide.txt)
+static_assert(AW_KST <= 4, "k_full / k_empty hold 4 barriers each");
 constexpr int AW_THREADS = 384;
 constexpr int AW_TABLE = 64;
 constexpr int AW_SMEM_FIXED = 2 * AW_QB + AW_KST * AW_KB + 2 * AW_KB + 2 * AW_PB + 256 /*barriers*/ +
@@ -95,59 +87,23 @@ __device__ __forceinline__ float ex2(float x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-// 2^x on the FMA pipe for FBKST_AW_NPOLY of every 4 register pairs (Cody-Waite range reduction + degree-3
-// minimax polynomial, max rel. error 7.5e-5, far below the bf16 rounding of P; x clamped at -126): the MUFU
-// pipe runs 16 ex2 per clock and SM = 1024 clocks for each 128 x 128 tile of each group.
-// Cycles by which group 1 falls behind group 0 at the start of its item FBKST_AW_STAGGER_ITEM: 51.2 -> 47.1 us
-// at cfg2 L = 375 (0 = off).
-#ifndef FBKST_AW_STAGGER
-#define FBKST_AW_STAGGER 1200
-#endif
-#ifndef FBKST_AW_STAGGER_ITEM
-#define FBKST_AW_STAGGER_ITEM 1
-#endif
-#ifndef FBKST_AW_NPOLY
-#define FBKST_AW_NPOLY 0
-#endif
+// Cycles by which group 1 falls behind group 0 once, at the start of its item AW_STAGGER_ITEM: 51.2 -> 47.1 us
+// at cfg2 L = 375.
+constexpr int AW_STAGGER = 1200;
+constexpr int AW_STAGGER_ITEM = 1;
 // registers per thread after the split: 128 producer threads + 256 softmax threads <= 384 x 168 at launch
-#ifndef FBKST_AW_REGS_PRODUCER
-#define FBKST_AW_REGS_PRODUCER 56
-#endif
-#ifndef FBKST_AW_REGS_SOFTMAX
-#define FBKST_AW_REGS_SOFTMAX 224
-#endif
-static_assert(128 * FBKST_AW_REGS_PRODUCER + 256 * FBKST_AW_REGS_SOFTMAX <= 384 * 168, "register split");
-#ifndef FBKST_AW_IDLE_NS
-#define FBKST_AW_IDLE_NS 64  // back-off of the idle load loop
-#endif
-// Experimental: strict alternation of the two groups' exponential phases (a token passed through two mbarriers),
-// so that one group's guard / hand-over / TMEM-load phases always run under the other group's exponentials.
-#ifndef FBKST_AW_PINGPONG
-#define FBKST_AW_PINGPONG 0
-#endif
-__device__ __forceinline__ float2 aw_ex2_poly2(float2 x) {
-  const float kMagic = 12582912.0f;  // 1.5 * 2^23: the integer part of x lands in the low mantissa bits
-  x.x = fmaxf(x.x, -126.0f);
-  x.y = fmaxf(x.y, -126.0f);
-  const float2 r = fadd2(x, make_float2(kMagic, kMagic));
-  const float2 n = fadd2(r, make_float2(-kMagic, -kMagic));
-  const float2 f = ffma2(n, make_float2(-1.0f, -1.0f), x);  // x - round(x) in [-0.5, 0.5]
-  float2 p = ffma2(f, make_float2(0.0551716648f, 0.0551716648f), make_float2(0.2426111251f, 0.2426111251f));
-  p = ffma2(p, f, make_float2(0.6932609677f, 0.6932609677f));
-  p = ffma2(p, f, make_float2(0.9999280572f, 0.9999280572f));
-  p.x = __uint_as_float(__float_as_uint(p.x) + (__float_as_uint(r.x) << 23));
-  p.y = __uint_as_float(__float_as_uint(p.y) + (__float_as_uint(r.y) << 23));
-  return p;
-}
+constexpr int AW_REGS_PRODUCER = 56;
+constexpr int AW_REGS_SOFTMAX = 224;
+static_assert(128 * AW_REGS_PRODUCER + 256 * AW_REGS_SOFTMAX <= 384 * 168, "register split");
+constexpr int AW_IDLE_NS = 64;  // back-off of the idle load loop
+// Every exponential runs on the MUFU pipe (16 ex2 per clock per SM = 1024 clocks for each 128 x 128 tile of
+// each group).  Moving some of them to an FMA-pipe polynomial, and strictly alternating the two groups'
+// exponential phases, were both measured and rejected (DESIGN.md section 4d, profiles/r02z_attention_wide.txt).
 __device__ __forceinline__ void aw_exp4(float2 (&t)[4]) {
 #pragma unroll
   for (int cc = 0; cc < 4; ++cc) {
-    if (cc < FBKST_AW_NPOLY) {
-      t[cc] = aw_ex2_poly2(t[cc]);
-    } else {
-      t[cc].x = ex2(t[cc].x);
-      t[cc].y = ex2(t[cc].y);
-    }
+    t[cc].x = ex2(t[cc].x);
+    t[cc].y = ex2(t[cc].y);
   }
 }
 __device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
@@ -320,7 +276,7 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
   uint8_t* sQ = smem;                 // 2 x 16 KB: one per group
   uint8_t* sK = sQ + 2 * AW_QB;       // AW_KST stages, shared by both groups (fixed interleaved order)
   uint8_t* sV = sK + AW_KST * AW_KB;  // one 16 KB tile (128 keys) per group
-  uint8_t* sP = sV + 2 * AW_KB;       // per group: the output staging rows (and the P tile without FBKST_AW_PTMEM)
+  uint8_t* sP = sV + 2 * AW_KB;       // per group: the output staging rows
   uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 2 * AW_PB);
   int4* sItems = reinterpret_cast<int4*>(bars + 32);
   float* sLut = reinterpret_cast<float*>(sItems + AW_TABLE);
@@ -334,10 +290,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
   uint64_t* pv_done = bars + 18;  // [2]  the PV product of the group's tile has completed: P[g] / V[g] free, O[g] updated
   uint64_t* s_free = bars + 20;   // [2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 26);
-#if FBKST_AW_PINGPONG
-  uint64_t* turn = bars + 22;  // [2] token: group g may run its exponentials
-  volatile uint32_t* grp_done = reinterpret_cast<volatile uint32_t*>(bars + 24);  // [2] group g has no tiles left
-#endif
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm128);
@@ -354,10 +306,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
       mbar_init(&p_full[s], 128);
       mbar_init(&pv_done[s], 1);
       mbar_init(&s_free[s], 128);
-#if FBKST_AW_PINGPONG
-      mbar_init(&turn[s], 128);
-      grp_done[s] = 0u;
-#endif
     }
     fence_barrier_init();
   }
@@ -384,7 +332,7 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
 #define AW_PICK(c0, c1, turn) (((turn) == 0) ? ((c0).valid(n_items) ? 0 : 1) : ((c1).valid(n_items) ? 1 : 0))
 
   if (warp < 4) {
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(FBKST_AW_REGS_PRODUCER));
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(AW_REGS_PRODUCER));
     if (warp == 0) {
       // ------------------------------------------------ TMA loads (Q, K, V halves): event loop over
       // non-blocking mbarrier.test_wait probes, so no load queues behind a wait that belongs to the other group
@@ -437,7 +385,7 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
           const bool ok = (AW_PICK(kc0, kc1, kturn) == 0) ? try_k(kc0, 0) : try_k(kc1, 1);
           if (ok) { kturn ^= 1; progressed = true; }
         }
-        if (!progressed) __nanosleep(FBKST_AW_IDLE_NS);
+        if (!progressed) __nanosleep(AW_IDLE_NS);
 #if FBKST_WATCHDOG
         idle = progressed ? 0 : idle + 1;
         if (idle > (1u << 26)) {
@@ -487,9 +435,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
       WCursor pc;
       pc.init(items, g);
       const uint32_t va = smem_u32(sV + g * AW_KB);
-#if !FBKST_AW_PTMEM
-      const uint32_t pa = smem_u32(sP + g * AW_PB);
-#endif
       while (pc.valid(n_items)) {
         const uint32_t ph = pc.c & 1;
         mbar_wait(&p_full[g], ph);
@@ -498,14 +443,9 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
         if (elect_one()) {
 #pragma unroll
           for (int kk = 0; kk < 8; ++kk) {
-#if FBKST_AW_PTMEM
             // A = P[g] from tensor memory: 128 lanes (query rows) x 8 columns (16 bf16 keys) per k-step
             umma_bf16_ts(tmem_O + g * AW_HD, tmem_P + g * (AW_BN / 2) + 8 * kk,
                          desc_mnmajor_sw128(va + kk * 2048, AW_KB), IDESC_PV, (pc.j > 0) || kk != 0);
-#else
-            umma_bf16_ss(tmem_O + g * AW_HD, desc_kmajor_sw128(pa + (kk >> 2) * AW_PSUB) + 2 * (kk & 3),
-                         desc_mnmajor_sw128(va + kk * 2048, AW_KB), IDESC_PV, (pc.j > 0) || kk != 0);
-#endif
           }
           umma_commit(&pv_done[g]);
           AW_TRACE(2 * pc.c + g, 12);
@@ -515,7 +455,7 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
       }
     }
   } else {
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(FBKST_AW_REGS_SOFTMAX));
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(AW_REGS_SOFTMAX));
     // ---- softmax / correction / output: thread <-> (query row of the group's own item)
     const int grp = (warp - 4) >> 2;
     const int q = (warp & 3) * 32 + lane;  // row in the tile == TMEM lane
@@ -528,9 +468,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
     uint64_t* my_p_full = &p_full[grp];
     uint64_t* my_pv_done = &pv_done[grp];
     uint64_t* my_s_free = &s_free[grp];
-    // the row's eight 16-byte chunks inside a 128B-swizzled sub-tile
-    // (the row starts on a 128-byte boundary: chunk c8 sits at p_row ^ (c8 << 4), one LOP3 per store)
-    const uint32_t p_row = smem_u32(sP + grp * AW_PB + q * 128) + ((uint32_t)(q & 7) << 4);
     uint8_t* stage_warp = sP + grp * AW_PB + (warp & 3) * 4096;  // epilogue staging: 32 rows x 128 B
     const int lut_off = nq * AW_BM;
     const int lut_n = aw_lut_floats(L);
@@ -545,9 +482,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
     // first LUT index of row i for key k0 is lut_off - i + k0 = r (mod 4) with r = (-q) & 3
     const int lut_r = (4 - (q & 3)) & 3;
     uint32_t c = 0;  // key tiles of this group before the current one
-#if FBKST_AW_PINGPONG
-    bool partner_done = false;
-#endif
     const int q_lim = q_limit ? __ldg(q_limit) : L;  // (after pdl_wait: written by the previous kernel)
     WItem it;
     // (item index, stride and count pinned in registers: ptxas otherwise rebuilds them from the kernel
@@ -586,18 +520,16 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
         const float4* lp = lut_row + (k0 >> 2);
         float2 sm2[4];
         uint32_t s[8][16], pk[64];
-#if FBKST_AW_STAGGER && !FBKST_AW_PINGPONG
         // The two groups share one MUFU pipe per scheduler.  Started together they stay in lockstep: both run
         // their exponentials at the same time (2400 cycles for the pair, the pipe's floor being 2048) and both
         // sit in their guard / hand-over / TMEM-load phases at the same time (~1100 cycles per tile in which
         // the pipe idles: timeline in profiles/r02z_attention_wide.txt).  Group 1 therefore drops a third of a
         // tile behind, once, after the instruction-cache-cold first item (which re-aligns the groups)
-        if (grp == 1 && j == 0 && k == 1 + 2 * FBKST_AW_STAGGER_ITEM) {
-          const long long t_go = clock64() + FBKST_AW_STAGGER;
+        if (grp == 1 && j == 0 && k == 1 + 2 * AW_STAGGER_ITEM) {
+          const long long t_go = clock64() + AW_STAGGER;
           while (clock64() < t_go) {
           }
         }
-#endif
         mbar_wait(my_s_full, ph);
         AW_TRACE(2 * c + grp, 0);
         tc_fence_after();
@@ -656,35 +588,14 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
         }
         const float2 negm2 = make_float2(-m_used, -m_used);
         AW_TRACE(2 * c + grp, 2);
-#if FBKST_AW_PINGPONG
-        // group 0's first phase needs no token; afterwards the token alternates (the partner's flag releases a
-        // group whose partner has run out of tiles)
-        if (!partner_done && (grp == 1 || c >= 1)) {
-          const uint32_t par = (grp == 0 ? (c - 1) : c) & 1u;
-          for (uint32_t spins = 0; !mbar_try_wait(&turn[grp], par); ++spins) {
-            if (grp_done[grp ^ 1]) {
-              partner_done = true;
-              break;
-            }
-            if (spins > (1u << 24)) {  // ~30 s: never legitimate
-              printf("fbkst: wide attention ping-pong watchdog block=%d group=%d tile=%u\n", blockIdx.x, grp, c);
-              __trap();
-            }
-          }
-        }
-#endif
         // all 16 chunks of 8 scores in ONE basic block, P packed into registers (they replace the score
         // registers as those die) ...
         aw_half<LOGPEN>(s[0], s[1], s[2], s[3], lp, negm2, sm2, pk);
         aw_half<LOGPEN>(s[4], s[5], s[6], s[7], lp + 16, negm2, sm2, pk + 32);
-#if FBKST_AW_PINGPONG
-        mbar_arrive(&turn[grp ^ 1]);
-#endif
         AW_TRACE(2 * c + grp, 3);
         // ... and stored once the PV product of the previous tile, which read this buffer, has completed
         if (c >= 1) mbar_wait(my_pv_done, ph ^ 1);
         AW_TRACE(2 * c + grp, 4);
-#if FBKST_AW_PTMEM
         tc_fence_after();
         tmem_st32(tP, *reinterpret_cast<uint32_t(*)[32]>(&pk[0]));
         tmem_st32(tP + 32, *reinterpret_cast<uint32_t(*)[32]>(&pk[32]));
@@ -692,16 +603,6 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
         tmem_st_wait();
         tc_fence_before();  // (also orders the O reads of the previous item's epilogue / a rescale before PV)
         mbar_arrive(my_p_full);
-#else
-#pragma unroll
-        for (int ch = 0; ch < 16; ++ch)
-          sts128((p_row ^ (uint32_t)((ch & 7) << 4)) + (ch >> 3) * AW_PSUB, pk[4 * ch], pk[4 * ch + 1],
-                 pk[4 * ch + 2], pk[4 * ch + 3]);
-        l += (sm2[0].x + sm2[0].y) + (sm2[1].x + sm2[1].y) + (sm2[2].x + sm2[2].y) + (sm2[3].x + sm2[3].y);
-        tc_fence_before();  // (also orders the O reads of the previous item's epilogue / a rescale before PV)
-        fence_proxy_async_smem();
-        mbar_arrive(my_p_full);
-#endif
         AW_TRACE(2 * c + grp, 5);
       }
       // ---- item epilogue (this group only): O / l -> bf16.  A thread owns a query row (128 B); stored
@@ -736,22 +637,12 @@ __global__ void __launch_bounds__(AW_THREADS, 1)
         if (lane == 0) {
           tma_store_3d(&tmO, stage_warp, it.h * AW_HD, it.b, it.q0 + (warp & 3) * 32);
           tma_store_commit();
-#if !FBKST_AW_PTMEM
-          tma_store_wait_read<0>();  // the staging rows are this warp's P rows of the next tile
-#endif
         }
-#if !FBKST_AW_PTMEM
-        __syncwarp();
-#endif
       }
       // O[grp] is overwritten by the PV of the group's next tile, which waits for this group's next
       // p_full arrival (ordered after the TMEM reads above by the fence before that arrive)
       AW_TRACE(2 * (c - 1) + grp, 10);
     }
-#if FBKST_AW_PINGPONG
-    grp_done[grp] = 1u;
-    __threadfence_block();
-#endif
     if (lane == 0) tma_store_wait<0>();  // output stores complete (and staging rows read) before the CTA retires
   }
 #undef AW_PICK

@@ -14,9 +14,6 @@
 // Small CTAs (160 threads, ~42 KB smem, C TMEM columns), as many per SM as fit: while one CTA waits for
 // its loads or its MMA the others build / drain.  Inputs, weights and the output are IEEE fp16 (saturating
 // conversions; accumulation stays fp32): the front end runs in fp16, not bf16 -- see ptx.cuh idesc_f16_f32.
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "host_common.h"
 #include "ptx.cuh"
 
@@ -28,8 +25,8 @@ template <int C>
 __global__ void __launch_bounds__(C1_THREADS, 4)
     conv1_tc_kernel(const __grid_constant__ CUtensorMap tmY, const float* __restrict__ x,
                     const float* __restrict__ w, const float* __restrict__ bias,
-                    const float* __restrict__ scale, const float* __restrict__ shift, int B, int T, int F,
-                    int T1, int F1, int n_pix, int planes) {
+                    const float* __restrict__ scale, const float* __restrict__ shift, int T, int F,
+                    int T1, int F1, int n_pix) {
   constexpr uint32_t IDESC = idesc_f16_f32(128, C, 0, 0);
   constexpr int HALVES = C / 64;                 // 64-column (128-byte) output pieces per pixel
   constexpr int OUT_WARP_BYTES = HALVES * 4096;  // [half][32 rows][128 B] per epilogue warp
@@ -104,36 +101,16 @@ __global__ void __launch_bounds__(C1_THREADS, 4)
     const int ppu = T1 * F1;  // pixels per utterance
     uint32_t ph = 0;
     float in[9];
-    // planes != 0: the output is FOUR (t1, f1)-parity planes [pt*2+pf][B][TH][FH][C], TH = ceil(T1/2), FH =
-    // ceil(F1/2), pixel (t1, f1) at (t1 & 1, f1 & 1, t1 >> 1, f1 >> 1); slots past T1 / F1 hold zeros.  The
-    // thread <-> pixel mapping is free here, and conv2's stride-2 taps become UNIT-stride TMA boxes of one
-    // plane (its 4-D boxes with element strides {1,2,2,1} move twice the bytes they deliver).
-    const int TH = (T1 + 1) >> 1, FH = (F1 + 1) >> 1;
-    bool live = true;  // false: a padding slot of a plane (written as zeros)
     auto load_taps = [&](int tile) {  // the 9 taps of this thread's pixel of `tile` (zero outside the image)
       const int p = tile * 128 + row;
 #pragma unroll
       for (int k = 0; k < 9; ++k) in[k] = 0.0f;
-      live = true;
       if (tile < n_tiles && p < n_pix) {
-        int b, t1, f1;
-        if (planes) {
-          const int per = B * TH * FH;
-          const int pl = p / per, r = p - pl * per;
-          b = r / (TH * FH);
-          const int r2 = r - b * (TH * FH);
-          const int th = r2 / FH, fh = r2 - th * FH;
-          t1 = 2 * th + (pl >> 1);
-          f1 = 2 * fh + (pl & 1);
-          live = t1 < T1 && f1 < F1;
-        } else {
-          b = p / ppu;
-          const int rem = p - b * ppu;
-          t1 = rem / F1;
-          f1 = rem - t1 * F1;
-        }
+        const int b = p / ppu;
+        const int rem = p - b * ppu;
+        const int t1 = rem / F1;
+        const int f1 = rem - t1 * F1;
         const float* xb = x + (size_t)b * T * F;
-        if (live)
 #pragma unroll
         for (int kh = 0; kh < 3; ++kh) {
           const int t = 2 * t1 - 1 + kh;
@@ -181,10 +158,10 @@ __global__ void __launch_bounds__(C1_THREADS, 4)
             const float a1 = fmaxf(__uint_as_float(v[j * 8 + h * 4 + 1]) + bb.y, 0.0f);
             const float a2 = fmaxf(__uint_as_float(v[j * 8 + h * 4 + 2]) + bb.z, 0.0f);
             const float a3 = fmaxf(__uint_as_float(v[j * 8 + h * 4 + 3]) + bb.w, 0.0f);
-            o[h * 4 + 0] = live ? fmaf(a0, sc.x, sh.x) : 0.0f;
-            o[h * 4 + 1] = live ? fmaf(a1, sc.y, sh.y) : 0.0f;
-            o[h * 4 + 2] = live ? fmaf(a2, sc.z, sh.z) : 0.0f;
-            o[h * 4 + 3] = live ? fmaf(a3, sc.w, sh.w) : 0.0f;
+            o[h * 4 + 0] = fmaf(a0, sc.x, sh.x);
+            o[h * 4 + 1] = fmaf(a1, sc.y, sh.y);
+            o[h * 4 + 2] = fmaf(a2, sc.z, sh.z);
+            o[h * 4 + 3] = fmaf(a3, sc.w, sh.w);
           }
           const int chunk = (c32 & 1) * 4 + j;  // 16-byte chunk inside the 128-byte half row
           *reinterpret_cast<uint4*>(orow + ((chunk ^ (lane & 7)) << 4)) =
@@ -212,21 +189,16 @@ __global__ void __launch_bounds__(C1_THREADS, 4)
 
 template <int C>
 static int launch_conv1_tc(const float* x, const float* w, const float* bias, const float* scale,
-                           const float* shift, void* y, int B, int T, int F, int T1, int F1, int planes,
-                           cudaStream_t st) {
+                           const float* shift, void* y, int B, int T, int F, int T1, int F1, cudaStream_t st) {
   constexpr int SMEM = 128 * 128 + C * 128 + 4 * (C / 64) * 4096 + 3 * C * 4 + 64 + 1024;
   auto kern = conv1_tc_kernel<C>;
   static PerDeviceFlag configured;
   if (!configured) {
+    // (no shared-memory carve-out preference: the driver default and 100 % measure the same, 41 us)
     FBKST_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    // shared-memory carve-out: the driver default and 100 % measure the same (41 us); switch kept for A/B
-    int carve = -1;
-    if (const char* e = getenv("FBKST_CONV1_CARVEOUT")) carve = atoi(e);  // A/B switch (-1: driver default)
-    if (carve >= 0)
-      FBKST_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
     configured = true;
   }
-  const long long n_pix = planes ? 4ll * B * ((T1 + 1) / 2) * ((F1 + 1) / 2) : (long long)B * T1 * F1;
+  const long long n_pix = (long long)B * T1 * F1;
   FBKST_REQUIRE(n_pix < (1ll << 31), "fbkst_conv1_relu_bn: too many pixels");
   CUtensorMap tmY;
   uint64_t dims[2] = {(uint64_t)C, (uint64_t)n_pix};
@@ -239,26 +211,18 @@ static int launch_conv1_tc(const float* x, const float* w, const float* bias, co
   // columns give 4 / 3.  cudaOccupancyMaxActiveBlocksPerMultiprocessor answers 1 for this kernel (it
   // appears to charge a tcgen05.alloc-ing kernel the whole TMEM), which halves the throughput: measured
   // 3 / 4 / 5 / 6 CTAs per SM -> 49 / 41 / 53 / 49 us at cfg2, 1 -> 86 us.
-  int per_sm = (C == 64) ? 4 : 3;
-  if (const char* e = getenv("FBKST_CONV1_PER_SM")) per_sm = atoi(e) > 0 ? atoi(e) : per_sm;  // A/B switch
+  const int per_sm = (C == 64) ? 4 : 3;
   int grid = num_sms() * per_sm;
   if (grid > n_tiles) grid = n_tiles;
-  static const bool dbg = getenv("FBKST_CONV1_DBG") != nullptr;
-  if (dbg) {
-    int occ = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, C1_THREADS, SMEM);
-    fprintf(stderr, "conv1_tc: grid %d, occupancy API %d CTAs/SM, smem %d\n", grid, occ, SMEM);
-  }
-  kern<<<grid, C1_THREADS, SMEM, st>>>(tmY, x, w, bias, scale, shift, B, T, F, T1, F1, (int)n_pix, planes);
+  kern<<<grid, C1_THREADS, SMEM, st>>>(tmY, x, w, bias, scale, shift, T, F, T1, F1, (int)n_pix);
   FBKST_CHECK_CUDA(cudaGetLastError());
   return FBKST_OK;
 }
 
 int conv1_tc_dispatch(const float* x, const float* w, const float* bias, const float* scale,
-                      const float* shift, void* y, int B, int T, int F, int C, int T1, int F1, int planes,
-                      cudaStream_t st) {
-  if (C == 64) return launch_conv1_tc<64>(x, w, bias, scale, shift, y, B, T, F, T1, F1, planes, st);
-  return launch_conv1_tc<128>(x, w, bias, scale, shift, y, B, T, F, T1, F1, planes, st);
+                      const float* shift, void* y, int B, int T, int F, int C, int T1, int F1, cudaStream_t st) {
+  if (C == 64) return launch_conv1_tc<64>(x, w, bias, scale, shift, y, B, T, F, T1, F1, st);
+  return launch_conv1_tc<128>(x, w, bias, scale, shift, y, B, T, F, T1, F1, st);
 }
 
 }  // namespace fbkst

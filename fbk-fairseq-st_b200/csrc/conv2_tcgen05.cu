@@ -9,7 +9,7 @@
 // Epilogue: +bias -> ReLU -> BatchNorm(eval) affine -> fp16, written channels-last, which is the
 // (t, f*C + c) operand layout of the fc3 GEMM (its weight columns are permuted to match).
 //
-// Same warp roles as gemm_tcgen05.cu (TMA / MMA / TMEM alloc / 4 epilogue warps), persistent.
+// Warp roles: TMA producer / MMA issuer / TMEM allocator / 4 epilogue warps, persistent.
 #include "host_common.h"
 #include "ptx.cuh"
 
@@ -21,7 +21,6 @@ struct Conv2Params {
   const float* shift;
   __nv_bfloat16* out;
   int B, T2, F2, R, tiles_per_utt;
-  int planes;  // input = four (t1, f1)-parity planes written by conv1_tc (unit-stride tap boxes)
 };
 
 template <int C, int STAGES>
@@ -32,8 +31,8 @@ __global__ void __launch_bounds__(256, 1)
   constexpr int B_BYTES = C * 64 * 2;
   // C == 64: all nine weight taps (72 KB) stay resident in shared memory for the life of the CTA and a
   // stage holds only the A box (35 % fewer bytes through TMA / L2, two more A stages).  MEASURED: on its
-  // own this did not move the kernel (51.2 us at cfg2), nor did unit-stride tap boxes over parity planes
-  // (p.planes): the bound was the issue code of the single-lane MMA / TMA warps (see the comment at the
+  // own this did not move the kernel (51.2 us at cfg2), nor did unit-stride tap boxes over conv1 output
+  // written as four (t1, f1)-parity planes (DESIGN.md finding 15, since removed): the bound was the issue code of the single-lane MMA / TMA warps (see the comment at the
   // warp roles); with that fixed and the epilogue constants in shared memory conv2 runs in 37-40 us.
   constexpr bool WRES = (C == 64);
   constexpr int STAGE_BYTES = A_BYTES + (WRES ? 0 : B_BYTES);
@@ -119,11 +118,7 @@ __global__ void __launch_bounds__(256, 1)
         uint8_t* sa = smem + stage * STAGE_BYTES;
         if (elect_one()) {
           mbar_arrive_expect_tx(&full_bar[stage], a_tx + (WRES ? 0 : B_BYTES));
-          if (p.planes)  // tap (kh, kw) reads conv1 pixel (2*t2 + kh - 1, 2*f2 + kw - 1): plane (kh != 1, kw != 1)
-            tma_load_5d(sa, &tmX, &full_bar[stage], kc * 64, kw == 0 ? -1 : 0, t0 + (kh == 0 ? -1 : 0), b,
-                        (kh != 1) * 2 + (kw != 1));
-          else
-            tma_load_4d(sa, &tmX, &full_bar[stage], kc * 64, kw - 1, 2 * t0 + kh - 1, b);
+          tma_load_4d(sa, &tmX, &full_bar[stage], kc * 64, kw - 1, 2 * t0 + kh - 1, b);
           if (!WRES) tma_load_2d(sa + A_BYTES, &tmW, &full_bar[stage], kc * 64, tap * C);
         }
         __syncwarp();
@@ -242,13 +237,7 @@ static int launch_conv2(const void* x, const void* w_taps, const Conv2Params& p,
   }
   CUtensorMap tmX, tmW;
   int rc;
-  if (p.planes) {  // [4 planes][B][T2][F2][C], unit-stride boxes of one plane
-    uint64_t dims[5] = {(uint64_t)C, (uint64_t)p.F2, (uint64_t)p.T2, (uint64_t)p.B, 4};
-    uint64_t strides[4] = {(uint64_t)C * 2, (uint64_t)p.F2 * C * 2, (uint64_t)p.T2 * p.F2 * C * 2,
-                           (uint64_t)p.B * p.T2 * p.F2 * C * 2};
-    uint32_t box[5] = {64, (uint32_t)p.F2, (uint32_t)p.R, 1, 1};
-    rc = make_tensor_map(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, 5, dims, strides, box, nullptr);
-  } else {
+  {
     uint64_t dims[4] = {(uint64_t)C, (uint64_t)F1, (uint64_t)T1, (uint64_t)p.B};
     uint64_t strides[3] = {(uint64_t)C * 2, (uint64_t)F1 * C * 2, (uint64_t)T1 * F1 * C * 2};
     uint32_t box[4] = {64, (uint32_t)(2 * p.F2), (uint32_t)(2 * p.R), 1};
@@ -275,9 +264,9 @@ static int launch_conv2(const void* x, const void* w_taps, const Conv2Params& p,
 
 }  // namespace fbkst
 
-static int conv2_entry(const void* x, const void* w_taps, const float* bias, const float* bn_scale,
-                       const float* bn_shift, void* y, int B, int T1, int F1, int C, int planes,
-                       fbkst_stream_t stream) {
+extern "C" int fbkst_conv2_relu_bn(const void* x, const void* w_taps, const float* bias,
+                                   const float* bn_scale, const float* bn_shift, void* y, int B,
+                                   int T1, int F1, int C, fbkst_stream_t stream) {
   using namespace fbkst;
   FBKST_REQUIRE(x && w_taps && bias && bn_scale && bn_shift && y, "fbkst_conv2_relu_bn: null pointer");
   FBKST_REQUIRE(C == 64 || C == 128, "fbkst_conv2_relu_bn: C must be 64 or 128 (got %d)", C);
@@ -294,20 +283,7 @@ static int conv2_entry(const void* x, const void* w_taps, const float* bias, con
   p.R = 128 / p.F2;
   if (p.R > p.T2) p.R = p.T2;
   p.tiles_per_utt = (p.T2 + p.R - 1) / p.R;
-  p.planes = planes;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (C == 64) return launch_conv2<64, 8>(x, w_taps, p, T1, F1, st);  // resident weights leave room for 8 A stages
   return launch_conv2<128, 6>(x, w_taps, p, T1, F1, st);
-}
-
-extern "C" int fbkst_conv2_relu_bn(const void* x, const void* w_taps, const float* bias,
-                                   const float* bn_scale, const float* bn_shift, void* y, int B,
-                                   int T1, int F1, int C, fbkst_stream_t stream) {
-  return conv2_entry(x, w_taps, bias, bn_scale, bn_shift, y, B, T1, F1, C, 0, stream);
-}
-
-extern "C" int fbkst_conv2_relu_bn_planes(const void* x_planes, const void* w_taps, const float* bias,
-                                          const float* bn_scale, const float* bn_shift, void* y, int B,
-                                          int T1, int F1, int C, fbkst_stream_t stream) {
-  return conv2_entry(x_planes, w_taps, bias, bn_scale, bn_shift, y, B, T1, F1, C, 1, stream);
 }

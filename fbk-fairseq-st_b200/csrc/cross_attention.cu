@@ -37,10 +37,7 @@ namespace fbkst {
 
 constexpr int XA_HD = 64;
 constexpr int XA_RC = 8;       // query rows served per pass over K/V
-#ifndef FBKST_XA_WARPS
-#define FBKST_XA_WARPS 8
-#endif
-constexpr int XA_WARPS = FBKST_XA_WARPS;
+constexpr int XA_WARPS = 8;
 constexpr int XA_THREADS = XA_WARPS * 32;
 constexpr int XA_SCAN = 1024;  // hypothesis rows scanned per list refill
 

@@ -472,17 +472,7 @@ extern "C" int fbkst_conv1_relu_bn(const float* x, const float* w, const float* 
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int T1 = (T + 1) / 2, F1 = (F + 1) / 2;
   FBKST_REQUIRE((long long)B * T1 * F1 < (1ll << 31), "fbkst_conv1_relu_bn: too many pixels");
-  return conv1_tc_dispatch(x, w, bias, bn_scale, bn_shift, y, B, T, F, C, T1, F1, 0, st);
-}
-
-extern "C" int fbkst_conv1_relu_bn_planes(const float* x, const float* w, const float* bias,
-                                          const float* bn_scale, const float* bn_shift, void* y, int B,
-                                          int T, int F, int C, fbkst_stream_t stream) {
-  FBKST_REQUIRE(x && w && bias && bn_scale && bn_shift && y, "fbkst_conv1_relu_bn_planes: null pointer");
-  FBKST_REQUIRE(C == 64 || C == 128, "fbkst_conv1_relu_bn_planes: C must be 64 or 128 (got %d)", C);
-  FBKST_REQUIRE(B > 0 && T > 0 && F > 0, "fbkst_conv1_relu_bn_planes: bad shape");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  return conv1_tc_dispatch(x, w, bias, bn_scale, bn_shift, y, B, T, F, C, (T + 1) / 2, (F + 1) / 2, 1, st);
+  return conv1_tc_dispatch(x, w, bias, bn_scale, bn_shift, y, B, T, F, C, T1, F1, st);
 }
 
 extern "C" int fbkst_layernorm(const float* x, const float* gamma, const float* beta, void* y,

@@ -1,6 +1,6 @@
 // out = epilogue(A @ W^T) with CTA-PAIR tensor-core tiles (tcgen05 cta_group::2).
 //
-// The single-CTA kernel (gemm_tcgen05.cu) moves 48 KB of operands from L2 per 128x256x64 MMA
+// A single-CTA kernel with 128x256 tiles (since removed) moves 48 KB of operands from L2 per 128x256x64 MMA
 // block, i.e. 94 B/clk/SM at full tensor rate -- more than twice what L2 can deliver to 148 SMs
 // (measured: the kernel saturates at ~11.5 TB/s of L2->SM traffic, ~50% tensor-pipe utilisation).
 // Here two CTAs of a cluster (one TPC) compute ONE 256x256 tile: each CTA stages its own 128 rows
@@ -13,8 +13,6 @@
 // Per CTA: warp 0 TMA producer (loads signal the LEADER's full barrier), warp 1 MMA issuer
 // (leader only; commits are multicast to both CTAs), warp 2 TMEM allocator, warps 4-11 epilogue
 // (TMEM -> registers -> bias/ReLU/residual -> swizzled smem -> per-warp TMA store).
-#include <stdlib.h>
-
 #include "host_common.h"
 #include "ptx.cuh"
 
@@ -157,7 +155,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(384, 1)
     gemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmR,
                  const __grid_constant__ CUtensorMap tmX, int M, int N, int K,
-                 const float* __restrict__ bias, int relu, int dbg, const int* __restrict__ m_limit,
+                 const float* __restrict__ bias, int relu, const int* __restrict__ m_limit,
                  int m_limit_mult, const LnStatsIn ln_in, float2* __restrict__ stats_out,
                  const uint32_t idesc, const int splits, const int split_rows, const ArgmaxEpi am) {
   static_assert(!LNS || (OUT_F32 && RESID), "row statistics are produced by the residual epilogue");
@@ -453,7 +451,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(384, 1)
           }
           __syncwarp();
           uint8_t* rowp = stg + sbuf * 4096 + lane * 128;
-          if (dbg & 2) continue;
           if (OUT_F32) {
 #pragma unroll
             for (int g = 0; g < 8; ++g) {
@@ -538,7 +535,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(384, 1)
           }
           fence_proxy_async_smem();
           __syncwarp();
-          if (lane == 0 && !(dbg & 1)) {
+          if (lane == 0) {
             tma_store_2d(&tmO, stg + sbuf * 4096, col0, m0 + m_store);
             tma_store_commit();
           }
@@ -629,9 +626,8 @@ static int launch_gemm2(const void* A, int64_t lda, const void* W, int64_t ldw, 
   const int tiles = ((M + 2 * G2_BM - 1) / (2 * G2_BM)) * ((N + G2_BN - 1) / G2_BN) * splits;
   const int max_clusters = num_sms() / 2;
   const int clusters = tiles < max_clusters ? tiles : max_clusters;
-  static const int dbg = getenv("FBKST_GEMM_DBG") ? atoi(getenv("FBKST_GEMM_DBG")) : 0;
   FBKST_CHECK_CUDA(launch_pdl(kern, dim3(2 * clusters), dim3(384), SMEM, stream, tmA, tmB, tmO, tmR, tmX,
-                              M, N, K, bias, relu, dbg, m_limit, m_limit_mult, ln_in,
+                              M, N, K, bias, relu, m_limit, m_limit_mult, ln_in,
                               reinterpret_cast<float2*>(stats_out),
                               MNM ? idesc_bf16_f32(256, G2_BN, 1, 1)
                                   : (ab_f16 ? idesc_f16_f32(256, G2_BN, 0, 0) : idesc_bf16_f32(256, G2_BN, 0, 0)),
@@ -639,7 +635,7 @@ static int launch_gemm2(const void* A, int64_t lda, const void* W, int64_t ldw, 
   return FBKST_OK;
 }
 
-// Entry used by fbkst_linear_bf16 / fbkst_linear_ln_bf16 (gemm_tcgen05.cu) for the plain / residual
+// Entry used by fbkst_linear_bf16 / fbkst_linear_ln_bf16 (below) for the plain / residual
 // epilogues.  stats_in (with its LayerNorm width == K and eps): consumer side of the folded
 // LayerNorm; out_bf16 + stats_out: producer side (residual epilogue only).
 int linear_pair_dispatch(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias,
@@ -741,6 +737,58 @@ static int wgrad_splits(int M, int N, int K) {
 }
 
 }  // namespace fbkst
+
+extern "C" int fbkst_linear_bf16(const void* A, int64_t lda, const void* W, int64_t ldw,
+                                 const float* bias, const float* residual, int64_t ldr, void* out,
+                                 int64_t ldo, int M, int N, int K, int flags, const int32_t* m_limit,
+                                 int m_limit_mult, fbkst_stream_t stream) {
+  using namespace fbkst;
+  FBKST_REQUIRE(A && W && out, "fbkst_linear_bf16: null operand");
+  FBKST_REQUIRE(M > 0 && N > 0 && K > 0, "fbkst_linear_bf16: empty problem M=%d N=%d K=%d", M, N, K);
+  FBKST_REQUIRE(K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0,
+                "fbkst_linear_bf16: K, lda, ldw must be multiples of 8 (K=%d lda=%lld ldw=%lld)", K,
+                (long long)lda, (long long)ldw);
+  FBKST_REQUIRE(ldo % 8 == 0, "fbkst_linear_bf16: ldo must be a multiple of 8 (got %lld)",
+                (long long)ldo);
+  FBKST_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "fbkst_linear_bf16: out must be 16-byte aligned");
+  FBKST_REQUIRE(residual == nullptr || ldr % 4 == 0, "fbkst_linear_bf16: ldr must be a multiple of 4");
+  const int relu = (flags & FBKST_EPI_RELU) ? 1 : 0;
+  if (residual != nullptr)
+    FBKST_REQUIRE(flags & FBKST_EPI_OUT_F32, "fbkst_linear_bf16: a residual requires fp32 output");
+  return linear_pair_dispatch(A, lda, W, ldw, bias, residual, ldr, out, ldo, M, N, K, relu,
+                              (flags & FBKST_EPI_OUT_F32) ? 1 : 0, m_limit, m_limit_mult, nullptr, 0.f, nullptr, 0,
+                              nullptr, (flags & FBKST_EPI_AB_F16) ? 1 : 0, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int fbkst_linear_ln_bf16(const void* A, int64_t lda, const void* W, int64_t ldw,
+                                    const float* bias, const float* residual, int64_t ldr, void* out,
+                                    int64_t ldo, int M, int N, int K, int flags,
+                                    const float* row_stats_in, float ln_eps, void* out_bf16,
+                                    int64_t ldob, float* row_stats_out, const int32_t* m_limit,
+                                    int m_limit_mult, fbkst_stream_t stream) {
+  using namespace fbkst;
+  FBKST_REQUIRE(A && W && out, "fbkst_linear_ln_bf16: null operand");
+  FBKST_REQUIRE(M > 0 && N > 0 && K > 0, "fbkst_linear_ln_bf16: empty problem M=%d N=%d K=%d", M, N, K);
+  FBKST_REQUIRE(K % 8 == 0 && lda % 8 == 0 && ldw % 8 == 0 && ldo % 8 == 0,
+                "fbkst_linear_ln_bf16: K, lda, ldw, ldo must be multiples of 8");
+  FBKST_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "fbkst_linear_ln_bf16: out must be 16-byte aligned");
+  if (residual != nullptr)
+    FBKST_REQUIRE((flags & FBKST_EPI_OUT_F32) && ldr % 4 == 0,
+                  "fbkst_linear_ln_bf16: a residual requires fp32 output and ldr %% 4 == 0");
+  FBKST_REQUIRE((out_bf16 == nullptr) == (row_stats_out == nullptr),
+                "fbkst_linear_ln_bf16: out_bf16 and row_stats_out come together");
+  if (row_stats_out != nullptr) {
+    FBKST_REQUIRE(residual != nullptr, "fbkst_linear_ln_bf16: row statistics need the residual epilogue");
+    FBKST_REQUIRE(N % 32 == 0 && ldob % 8 == 0 && (reinterpret_cast<uintptr_t>(out_bf16) & 15) == 0,
+                  "fbkst_linear_ln_bf16: N %% 32, ldob %% 8 and 16-byte alignment required (N=%d)", N);
+  }
+  if (row_stats_in != nullptr)
+    FBKST_REQUIRE(residual == nullptr, "fbkst_linear_ln_bf16: row_stats_in applies to the plain epilogue");
+  return linear_pair_dispatch(A, lda, W, ldw, bias, residual, ldr, out, ldo, M, N, K,
+                              (flags & FBKST_EPI_RELU) ? 1 : 0, (flags & FBKST_EPI_OUT_F32) ? 1 : 0, m_limit,
+                              m_limit_mult, row_stats_in, ln_eps, out_bf16, ldob, row_stats_out,
+                              (flags & FBKST_EPI_AB_F16) ? 1 : 0, reinterpret_cast<cudaStream_t>(stream));
+}
 
 extern "C" long long fbkst_linear_wgrad_workspace(int n_out, int k_in, int tokens) {
   using namespace fbkst;

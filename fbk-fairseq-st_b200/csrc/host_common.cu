@@ -1,5 +1,3 @@
-#include <stdlib.h>
-
 #include "host_common.h"
 
 #include <stdarg.h>
@@ -86,14 +84,6 @@ int num_sms() {
     n = 148;
   cache[dev].store(n, std::memory_order_relaxed);
   return n;
-}
-
-bool pdl_enabled() {
-  static const int v = [] {
-    const char* e = getenv("FBKST_PDL");
-    return (e != nullptr && e[0] == '0') ? 0 : 1;
-  }();
-  return v != 0;
 }
 
 }  // namespace fbkst

@@ -68,11 +68,7 @@ class PerDeviceFlag {
 
 // conv1 on the tensor pipe (conv1_tcgen05.cu); C is 64 or 128
 int conv1_tc_dispatch(const float* x, const float* w, const float* bias, const float* scale,
-                      const float* shift, void* y, int B, int T, int F, int C, int T1, int F1, int planes,
-                      cudaStream_t st);
-
-// 0 when FBKST_PDL=0 is set in the environment (A/B switch); default 1.
-bool pdl_enabled();
+                      const float* shift, void* y, int B, int T, int F, int C, int T1, int F1, cudaStream_t st);
 
 // Launch `kernel` with programmatic stream serialisation (programmatic dependent launch): the grid
 // may be scheduled while the previous kernel of the stream is still draining, runs its prologue
@@ -90,7 +86,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);

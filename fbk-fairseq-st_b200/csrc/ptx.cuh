@@ -129,14 +129,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const void* tmap, ui
       "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_5d(void* smem_dst, const void* tmap, uint64_t* bar,
-                                            int c0, int c1, int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(smem_u32(smem_dst)),
-      "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
 __device__ __forceinline__ void tma_store_2d(const void* tmap, const void* smem_src, int c0,
                                              int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.tile.bulk_group [%0, {%2, %3}], [%1];" ::

@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(_HERE, "libfbkst_b200.so")
 ERR_ARG, ERR_CUDA, ERR_OOM = -1, -2, -3
 BF16, F32 = 0, 1
 CTC_STRATEGY = {"avg": 0, "weighted": 1, "softmax": 2}
-EPI_RELU, EPI_OUT_F32, EPI_ROW_REMAP, EPI_POSEMB, EPI_AB_F16 = 1, 2, 4, 8, 16
+EPI_RELU, EPI_OUT_F32, EPI_AB_F16 = 1, 2, 16
 SA_INCREMENTAL, SA_FULL, SA_CAUSAL = 0, 1, 2
 
 P, I, I64, F, U64 = c_void_p, c_int, c_int64, c_float, c_uint64
@@ -22,9 +22,7 @@ SIGNATURES = {
     "fbkst_collate_cmvn_f32": [P, P, P, P, I, I, I, I, P, P],
     "fbkst_conv1_relu_bn": [P, P, P, P, P, P, I, I, I, I, P],
     "fbkst_conv2_relu_bn": [P, P, P, P, P, P, I, I, I, I, P],
-    "fbkst_conv1_relu_bn_planes": [P, P, P, P, P, P, I, I, I, I, P],
-    "fbkst_conv2_relu_bn_planes": [P, P, P, P, P, P, I, I, I, I, P],
-    "fbkst_linear_bf16": [P, I64, P, I64, P, P, I64, P, I64, I, I, I, I, I, I, P, P, I, P],
+    "fbkst_linear_bf16": [P, I64, P, I64, P, P, I64, P, I64, I, I, I, I, P, I, P],
     "fbkst_linear_ln_bf16": [P, I64, P, I64, P, P, I64, P, I64, I, I, I, I, P, F, P, I64, P, P, I, P],
     "fbkst_row_stats_cast": [P, P, P, I, I, P, I, P],
     "fbkst_embed_remap_stats": [P, P, I64, P, P, P, P, I, I, I, P],

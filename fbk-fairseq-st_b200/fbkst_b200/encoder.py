@@ -22,14 +22,7 @@ import torch
 import torch.nn as nn
 from torch import Tensor
 
-import os
-
 from . import ops
-
-# A/B switch: FBKST_CONV_PLANES=1 makes conv1 write four (t1, f1)-parity planes so that conv2's stride-2 taps
-# are unit-stride TMA boxes.  Bit-identical output (tests/test_gpu_ops.py), but measured time-neutral
-# (conv2 51.2 us either way at cfg2), so the reference layout [B,T1,F1,C] stays the default.
-_CONV_PLANES = os.environ.get("FBKST_CONV_PLANES", "0") == "1"
 
 try:  # plug into fairseq when it is importable (train.py / generate.py --user-dir)
     from fairseq.models import FairseqEncoder as _Base  # type: ignore
@@ -581,13 +574,8 @@ def make_encoder_class(base):
             (only needed when ``want_states``)."""
             dev = x_in.device
             D, H = self.embed_dim, self.heads
-            if _CONV_PLANES:  # conv1 writes parity planes: conv2's taps are unit-stride TMA boxes
-                T_in, F_in = x_in.shape[1], x_in.shape[2]
-                y = ops.conv1_relu_bn_planes(x_in, P["w1"], P["b1"], *P["bn0"])
-                y = ops.conv2_relu_bn_planes(y, (T_in + 1) // 2, (F_in + 1) // 2, P["w2"], P["b2"], *P["bn1"])
-            else:
-                y = ops.conv1_relu_bn(x_in, P["w1"], P["b1"], *P["bn0"])
-                y = ops.conv2_relu_bn(y, P["w2"], P["b2"], *P["bn1"])  # [B, T2, F2, C]
+            y = ops.conv1_relu_bn(x_in, P["w1"], P["b1"], *P["bn0"])
+            y = ops.conv2_relu_bn(y, P["w2"], P["b2"], *P["bn1"])  # [B, T2, F2, C]
             assert y.shape[1] == L
             a = y.view(B * L, -1)
             # fc3 + ReLU on the CTA-pair GEMM in the conv layout's (b, t) row order; the transpose to
@@ -827,8 +815,7 @@ def make_encoder_class(base):
             # sum of exponentials (weighted / softmax) the 8 epilogue warps become the bottleneck (342 us against
             # 217 + 127: a tie), so those strategies keep the separate pass (scripts/bench_ctc_fc.py)
             fused = (not self.ctc_fc._forward_hooks and not self.ctc_fc._forward_pre_hooks
-                     and self.ctc_fc.logits_dtype == torch.float32 and not want_prob and self._precision == "bf16"
-                     and os.environ.get("FBKST_CTC_FUSED", "1") != "0")
+                     and self.ctc_fc.logits_dtype == torch.float32 and not want_prob and self._precision == "bf16")
             if fused:
                 # ctc_fc on tcgen05 with the arg-max (+ sum exp) folded into its epilogue: the logits are written
                 # once and never re-read (conv_transformer.py:279 + :282-284)

@@ -4,7 +4,7 @@ library or the GPU is missing (no fallback)."""
 import torch
 
 from . import _lib
-from ._lib import (BF16, CTC_STRATEGY, EPI_AB_F16, EPI_OUT_F32, EPI_POSEMB, EPI_RELU, EPI_ROW_REMAP, F32, SA_CAUSAL,
+from ._lib import (BF16, CTC_STRATEGY, EPI_AB_F16, EPI_OUT_F32, EPI_RELU, F32, SA_CAUSAL,
                    SA_FULL, SA_INCREMENTAL, check)
 
 LAUNCHES = 0  # kernels launched through this module (bench.py reports it as gpu_launches)
@@ -121,42 +121,13 @@ def conv2_relu_bn(x, w_taps, bias, scale, shift):
     return y
 
 
-def conv1_relu_bn_planes(x, w, bias, scale, shift):
-    """conv1 -> four (t1, f1)-parity planes [4, B, ceil(T1/2), ceil(F1/2), C] bf16 (see the header)."""
-    lib = _lib.require_device()
-    _req(x, torch.float32, "conv1.x")
-    B, T, Fd = x.shape
-    C = w.shape[0]
-    T1, F1 = (T + 1) // 2, (Fd + 1) // 2
-    y = torch.empty(4, B, (T1 + 1) // 2, (F1 + 1) // 2, C, dtype=torch.float16, device=x.device)
-    check(lib.fbkst_conv1_relu_bn_planes(x.data_ptr(), _req(w, torch.float32, "conv1.w").data_ptr(),
-                                         bias.data_ptr(), scale.data_ptr(), shift.data_ptr(),
-                                         y.data_ptr(), B, T, Fd, C, _stream()))
-    _count()
-    return y
-
-
-def conv2_relu_bn_planes(x_planes, T1, F1, w_taps, bias, scale, shift):
-    """conv2 over the plane layout of ``conv1_relu_bn_planes``; output as ``conv2_relu_bn``."""
-    lib = _lib.require_device()
-    _req(x_planes, torch.float16, "conv2.x_planes"); _req(w_taps, torch.float16, "conv2.w_taps")
-    four, B, TH, FH, C = x_planes.shape
-    if four != 4 or TH != (T1 + 1) // 2 or FH != (F1 + 1) // 2:
-        raise ValueError("conv2_relu_bn_planes: plane shape %s does not match T1=%d F1=%d"
-                         % (tuple(x_planes.shape), T1, F1))
-    y = torch.empty(B, TH, FH, C, dtype=torch.float16, device=x_planes.device)
-    check(lib.fbkst_conv2_relu_bn_planes(x_planes.data_ptr(), w_taps.data_ptr(), bias.data_ptr(),
-                                         scale.data_ptr(), shift.data_ptr(), y.data_ptr(), B, T1, F1, C,
-                                         _stream()))
-    _count()
-    return y
+# bench.py's per-kernel profile wraps these names; the parity-plane conv layout they served is gone
+conv1_relu_bn_planes = conv2_relu_bn_planes = None
 
 
 def linear(a, w, bias=None, relu=False, residual=None, out_dtype=torch.bfloat16, out=None,
-           remap=None, posemb=None, rows_limit=None):
+           rows_limit=None):
     """out = epi(a @ w.T).  a [M,K] bf16, w [N,K] bf16 (or both fp16), bias [N] fp32, residual [M,N] fp32.
-    remap=(inner, outer): out row = (m % inner)*outer + m // inner.
-    posemb=(table [P,N] fp32, lengths [outer] int32): adds table[pos(m)] (needs remap dims).
     rows_limit=(count [1] int32 device tensor, mult): only rows < count*mult are computed."""
     lib = _lib.require_device()
     if a.dtype == torch.float16:  # the conv front end's operands are IEEE fp16 (conv2 output x fc3 weight)
@@ -169,18 +140,10 @@ def linear(a, w, bias=None, relu=False, residual=None, out_dtype=torch.bfloat16,
         raise ValueError("fbkst_b200.linear: K mismatch %s vs %s" % (tuple(a.shape), tuple(w.shape)))
     flags = (EPI_RELU if relu else 0) | (EPI_OUT_F32 if out_dtype == torch.float32 else 0) | \
         (EPI_AB_F16 if a.dtype == torch.float16 else 0)
-    inner = outer = 0
-    lengths = None
-    res, ldr = residual, 0
-    if remap is not None:
-        inner, outer = remap
-        flags |= EPI_ROW_REMAP
-    if posemb is not None:
-        res, lengths = posemb
-        flags |= EPI_POSEMB
-    if res is not None:
-        _req(res, torch.float32, "linear.residual")
-        ldr = res.stride(0)
+    ldr = 0
+    if residual is not None:
+        _req(residual, torch.float32, "linear.residual")
+        ldr = residual.stride(0)
     if out is None:
         # rows start on 128-byte lines when N is not already a multiple of 8: the epilogue's 128-byte TMA store
         # boxes then map to whole lines (V = 8005 logits: pitch 8032 instead of 8008)
@@ -191,8 +154,7 @@ def linear(a, w, bias=None, relu=False, residual=None, out_dtype=torch.bfloat16,
     if out.dtype != out_dtype or out.stride(-1) != 1:
         raise ValueError("fbkst_b200.linear: bad out tensor")
     check(lib.fbkst_linear_bf16(a.data_ptr(), a.stride(0), w.data_ptr(), w.stride(0), _ptr(bias),
-                                _ptr(res), ldr, out.data_ptr(), out.stride(0), M, N, K, flags,
-                                inner, outer, _ptr(lengths),
+                                _ptr(residual), ldr, out.data_ptr(), out.stride(0), M, N, K, flags,
                                 _ptr(rows_limit[0]) if rows_limit else 0,
                                 rows_limit[1] if rows_limit else 0, _stream()))
     _count()

@@ -18,7 +18,6 @@ The per-batch work is exactly ``apply_mv_norm`` (data/fbank_dataset.py:44-45) fo
 ``ConvolutionalTransformerEncoder.forward`` (models/conv_transformer.py:195-276).
 """
 import collections
-import os
 
 import torch
 
@@ -27,8 +26,8 @@ from . import ops
 
 class EncoderPipeline:
     def __init__(self, encoder, normalize=True, device=None, lanes=None):
-        if lanes is None:  # A/B switch; two lanes measured best (profiles/r01g_overlap_probe.txt, r02y)
-            lanes = int(os.environ.get("FBKST_LANES", "2"))
+        if lanes is None:  # two lanes measured best (profiles/r01g_overlap_probe.txt, r02y)
+            lanes = 2
         self.enc = encoder
         self.normalize = normalize
         self.device = device or next(encoder.parameters()).device

@@ -23,8 +23,6 @@ Operand precision: bf16 GEMM operands / fp16 conv-front-end activations, fp32 ac
 stream and fp32 parameter gradients in the reference's parameter layout (so fairseq's optimizers, gradient
 clipping and the legacy DDP all-reduce see exactly what they expect).
 """
-import os
-
 import torch
 
 from . import ops
@@ -157,16 +155,6 @@ def _bn_state(enc, i, y_relu, train):
     return mean, rstd, sc, sh
 
 
-def wgrad_nt():
-    """Weight gradients of the encoder layers' nn.Linear from the operands' natural [tokens, features] layouts
-    (``fbkst_linear_wgrad_nt``: both operands MN-major in the tensor cores) instead of token-contiguous transposed
-    copies.  Same tiles and split-K order, bit-identical results; A/B switch ``FBKST_WGRAD_NT``."""
-    return os.environ.get("FBKST_WGRAD_NT", _WGRAD_NT_DEFAULT) == "1"
-
-
-_WGRAD_NT_DEFAULT = "1"  # measured (cfg4, r02x): backward 20.7 -> 20.05 ms
-
-
 def pretranspose(S):
     """Token-contiguous (transposed) bf16 copies of the activations the weight-gradient GEMMs read, for the saved
     state ``S`` of one training forward: one batched launch (+ conv2's im2col).  Idempotent."""
@@ -181,9 +169,6 @@ def pretranspose(S):
         out = ops.transposed_buffer(t.shape[0], t.shape[1], dev)
         jobs.append((t, None, out))
         return out
-    if not wgrad_nt():  # (the natural-layout weight-gradient GEMM reads the saved activations as they are)
-        for rec in S["layers"]:
-            rec["T"] = dict(f=tjob(rec["f"]), ln2=tjob(rec["ln2"]), att=tjob(rec["att"]), ln1=tjob(rec["ln1"]))
     y2 = S["y2"]
     S["y2T"] = tjob(y2.view(y2.shape[0] * y2.shape[1], -1))
     ops.prep_batch(jobs)
@@ -302,7 +287,7 @@ class EncoderTrainFn(torch.autograd.Function):
         # which is bound by the host's launch rate and leaves the GPU idle) -- inside this node's backward they
         # sit on the GPU-bound critical path (44 launches, ~1.3 ms per cfg4 step).
         mode = getattr(enc, "pretranspose_activations", True)
-        mode = os.environ.get("FBKST_PRETRANSPOSE", "bwd" if mode is True else ("off" if not mode else mode))
+        mode = "bwd" if mode is True else ("off" if not mode else mode)
         enc._train_pending = S if mode == "bwd" else None
         if mode == "fwd":
             pretranspose(S)
@@ -328,11 +313,9 @@ class EncoderTrainFn(torch.autograd.Function):
         if getattr(enc, "_train_pending", None) is S:  # no criterion node did it earlier: one batched launch here
             enc._train_pending = None
             pretranspose(S)
-        elif not S.get("pretransposed") and getattr(enc, "pretranspose_activations", True) and \
-                os.environ.get("FBKST_PRETRANSPOSE", "") != "off":
+        elif not S.get("pretransposed") and getattr(enc, "pretranspose_activations", True):
             pretranspose(S)
         W = prepare_train_weights(enc)
-        nt = wgrad_nt()
         B, L, D, H, C = S["B"], S["L"], enc.embed_dim, enc.heads, enc.conv_channels
         seed, p, p_act, p_att, p_conv = S["seed"], S["p"], S["p_act"], S["p_att"], S["p_conv"]
         # every reduction whose result is only read when the backward returns (bias gradients, split-K slices of
@@ -350,10 +333,6 @@ class EncoderTrainFn(torch.autograd.Function):
                 cur_L, cur_len, sites = R["L"], R["lengths"], R["sites"]
                 M = cur_L * B
                 g = {}
-                RT = R.get("T") or {}
-
-                def tr(name):  # token-contiguous copy of a saved activation (made at the end of the forward)
-                    return RT[name] if name in RT else ops.transpose_bf16(R[name])
                 if R["ctc"] is not None:
                     ct = R["ctc"]
                     # dx holds the L2*B compressed rows; a frame's segment id is < its utterance's new length <= L2
@@ -371,23 +350,25 @@ class EncoderTrainFn(torch.autograd.Function):
                         wcT = W["wcT"]
                         wcT_full = wcT if Vp == V else torch.as_strided(wcT, (D, Vp), (wcT.stride(0), 1))
                         dx = ops.linear(gb, wcT_full, None, residual=dx, out_dtype=torch.float32)
-                # ---- feed-forward block (transformer_layer.py:124-136)
-                g2, g2T, g["b2"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["ffn"], dp_cols=D, want_gT=not nt)
-                g["w2"] = ops.linear_wgrad_nt(g2, R["f"]) if nt else ops.linear_wgrad(g2T, tr("f"))
+                # ---- feed-forward block (transformer_layer.py:124-136).  The weight gradients read the saved
+                # activations in their natural [tokens, features] layout (both operands MN-major in the tensor
+                # cores), not token-contiguous transposed copies: measured (cfg4, r02x) backward 20.7 -> 20.05 ms
+                g2, _, g["b2"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["ffn"], dp_cols=D, want_gT=False)
+                g["w2"] = ops.linear_wgrad_nt(g2, R["f"])
                 df = ops.linear(g2, Wl["w2T"])
-                dh, dhT, g["b1"] = ops.grad_prep(df, act=R["f"], act_scale=1.0 / (1.0 - p_act) if p_act > 0 else 1.0,
-                                                 want_gT=not nt)
-                g["w1"] = ops.linear_wgrad_nt(dh, R["ln2"]) if nt else ops.linear_wgrad(dhT, tr("ln2"))
+                dh, _, g["b1"] = ops.grad_prep(df, act=R["f"], act_scale=1.0 / (1.0 - p_act) if p_act > 0 else 1.0,
+                                               want_gT=False)
+                g["w1"] = ops.linear_wgrad_nt(dh, R["ln2"])
                 dln2 = ops.linear(dh, Wl["w1T"], out_dtype=torch.float32)
                 dx, g["g2"], g["be2"] = ops.ln_bwd(dln2, R["x1"], Wl["g2"], dx=dx, eps=Wl["eps2"])
                 # ---- self-attention block (:104-122)
-                g1, g1T, g["bo"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["out"], dp_cols=D, want_gT=not nt)
-                g["wo"] = ops.linear_wgrad_nt(g1, R["att"]) if nt else ops.linear_wgrad(g1T, tr("att"))
+                g1, _, g["bo"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["out"], dp_cols=D, want_gT=False)
+                g["wo"] = ops.linear_wgrad_nt(g1, R["att"])
                 dO = ops.linear(g1, Wl["woT"])
                 dqkv = ops.attention_train_bwd(R["qkv"], R["att"], dO, R["lse"], cur_len, cur_L, B, H, enc.log_penalty,
                                                p_att, seed, sites["att"])
-                _, dqkvT, g["bqkv"] = ops.grad_prep(dqkv, want_gb=False, want_gT=not nt)
-                g["wqkv"] = ops.linear_wgrad_nt(dqkv, R["ln1"]) if nt else ops.linear_wgrad(dqkvT, tr("ln1"))
+                _, _, g["bqkv"] = ops.grad_prep(dqkv, want_gb=False, want_gT=False)
+                g["wqkv"] = ops.linear_wgrad_nt(dqkv, R["ln1"])
                 dln1 = ops.linear(dqkv, Wl["wqkvT"], out_dtype=torch.float32)
                 dx, g["g1"], g["be1"] = ops.ln_bwd(dln1, R["x"], Wl["g1"], dx=dx, eps=Wl["eps1"])
                 G[li] = g

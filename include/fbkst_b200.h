@@ -46,8 +46,6 @@ enum { FBKST_SA_INCREMENTAL = 0, FBKST_SA_FULL = 1, FBKST_SA_CAUSAL = 2 };
 enum {
   FBKST_EPI_RELU = 1,      /* y = max(y, 0) after the bias                                  */
   FBKST_EPI_OUT_F32 = 2,   /* out is fp32 (default bf16)                                    */
-  FBKST_EPI_ROW_REMAP = 4, /* out row = (m % remap_inner) * remap_outer + m / remap_inner    */
-  FBKST_EPI_POSEMB = 8,    /* residual is a [*, N] table indexed by position (see fc3)      */
   FBKST_EPI_AB_F16 = 16    /* A and W hold IEEE fp16 instead of bf16 (the conv front end)    */
 };
 
@@ -94,26 +92,13 @@ int fbkst_conv2_relu_bn(const void* x, const void* w_taps, const float* bias,
                         const float* bn_scale, const float* bn_shift, void* y, int B, int T1,
                         int F1, int C, fbkst_stream_t stream);
 
-/* ---- a2, plane layout (default inside the encoder): conv1 writes FOUR (t1, f1)-parity planes
- * [ (t1&1)*2 + (f1&1) ][B][ceil(T1/2)][ceil(F1/2)][C] fp16 (slots past T1 / F1 are zeros) instead of
- * [B][T1][F1][C]; conv2's stride-2 taps then are unit-stride TMA boxes of one plane.  Same arithmetic, same
- * conv2 output as the pair above (conv_transformer.py:203-214). */
-int fbkst_conv1_relu_bn_planes(const float* x, const float* w, const float* bias, const float* bn_scale,
-                               const float* bn_shift, void* y_planes, int B, int T, int F, int C,
-                               fbkst_stream_t stream);
-int fbkst_conv2_relu_bn_planes(const void* x_planes, const void* w_taps, const float* bias,
-                               const float* bn_scale, const float* bn_shift, void* y, int B, int T1,
-                               int F1, int C, fbkst_stream_t stream);
-
 /* ---- generic fused linear: out = epi(A @ W^T) on tcgen05 --------------------------------
  * replaces every F.linear / nn.Linear on the path (conv_transformer.py:227,279;
  * local_attention.py:178,141; fairseq/modules/transformer_layer.py:131-133).
  * A [M,K] bf16 (row pitch lda), W [N,K] bf16 (row pitch ldw), bias [N] fp32 or NULL.
- * y = A W^T + bias; ReLU if FBKST_EPI_RELU; then, if residual != NULL:
- *   default            : y += residual[m, n]            (fp32, row pitch ldr)
- *   FBKST_EPI_POSEMB   : y += residual[pos(m), n]  with m = b*remap_inner + t,
- *                        pos = t < lengths[b] ? t+1 : 0   (sinusoidal table, row 0 = 0)
- * out row is m, or the remapped row if FBKST_EPI_ROW_REMAP; out pitch ldo; dtype by flag.
+ * y = A W^T + bias; ReLU if FBKST_EPI_RELU; then, if residual != NULL (requires FBKST_EPI_OUT_F32):
+ *   y += residual[m, n]   (fp32, row pitch ldr)
+ * out row m, out pitch ldo; dtype by flag.
  * m_limit (device, may be NULL): only rows m < m_limit[0] * m_limit_mult are computed -- the
  * number of rows that are valid after CTC compression is known only on the device, so the
  * layers after it are launched for the worst case and skip the tiles beyond the limit
@@ -121,9 +106,7 @@ int fbkst_conv2_relu_bn_planes(const void* x_planes, const void* w_taps, const f
  * K % 8 == 0; lda, ldw % 8 == 0; all bases 16-byte aligned. */
 int fbkst_linear_bf16(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias,
                       const float* residual, int64_t ldr, void* out, int64_t ldo, int M, int N,
-                      int K, int flags, int remap_inner, int remap_outer,
-                      const int32_t* lengths, const int32_t* m_limit, int m_limit_mult,
-                      fbkst_stream_t stream);
+                      int K, int flags, const int32_t* m_limit, int m_limit_mult, fbkst_stream_t stream);
 
 /* ---- a6/a8 fused: linear with the pre-LayerNorm of the reference's residual block folded in ---
  * replaces the pairs  LayerNorm -> F.linear  of fairseq/modules/transformer_layer.py:108-110
@@ -132,7 +115,7 @@ int fbkst_linear_bf16(const void* A, int64_t lda, const void* W, int64_t ldw, co
  *     LN(x) W^T + b = rstd(x) * (x W''^T) + c,
  *     W''[n,k] = gamma[k] W[n,k] - mean_k(gamma[k] W[n,k]),   c[n] = b[n] + sum_k beta[k] W[n,k]
  * (every row of W'' sums to zero, so the row mean of x drops out; W'' and c are prepared by the host).
- * Same operands and flags as fbkst_linear_bf16 (no row remap / position table), plus
+ * Same operands and flags as fbkst_linear_bf16, plus
  *   producer side (residual epilogue, i.e. out_proj / fc2):  out_bf16 [M,N] bf16 (pitch ldob)
  *     receives bf16(out) and row_stats_out [M, ceil(N/128)] x 2 fp32 the (mean, M2) of each
  *     128-column slice of every output row; both NULL to skip.  N % 32 == 0;

@@ -80,11 +80,6 @@ w2 = ops.prep_conv2_weight(torch.randn(C, C, 3, 3, device=d) * 0.05)
 y2 = ops.conv2_relu_bn(y1, w2, b1, sc, sh)
 timeit("conv2", lambda: ops.conv2_relu_bn(y1, w2, b1, sc, sh), y1.numel() * 2 + y2.numel() * 2)
 
-p1 = ops.conv1_relu_bn_planes(x, w1, b1, sc, sh)
-timeit("conv1 planes", lambda: ops.conv1_relu_bn_planes(x, w1, b1, sc, sh), x.numel() * 4 + p1.numel() * 2)
-timeit("conv2 planes", lambda: ops.conv2_relu_bn_planes(p1, y1.shape[1], y1.shape[2], w2, b1, sc, sh),
-       p1.numel() * 2 + y2.numel() * 2)
-
 xr = torch.randn(L * B, D, device=d)
 g, b_ = torch.randn(D, device=d), torch.randn(D, device=d)
 timeit("layernorm f32->bf16", lambda: ops.layernorm(xr, g, b_), xr.numel() * 6)

@@ -5,6 +5,3 @@ run am tests/test_gpu_ops.py -k "argmax or ctc"
 run fused tests/test_gpu_encoder.py tests/test_gpu_parity_full.py
 grep -E "^(E |FAILED|ERROR)|assert|Error" gpurun_out/am.log gpurun_out/fused.log | head -n 20
 timeout 300 python scripts/bench_ctc_fc.py 2>&1 | tee gpurun_out/bench_ctc_fc.txt
-# natural-layout wgrad in the training step: parity, then A/B
-FBKST_WGRAD_NT=1 timeout 900 python -m pytest tests/test_gpu_train.py tests/test_gpu_dropin.py -x -q > gpurun_out/train_nt.log 2>&1; echo "train_nt exit=$? :: $(tail -n 1 gpurun_out/train_nt.log)"
-bash scripts/ab_cfg4.sh "FBKST_WGRAD_NT=0 FBKST_WGRAD_NT=1" 2 8

@@ -5,7 +5,7 @@ Every kernel of the step is a persistent grid of <=148 CTAs (or 296 for attentio
 each launch leaves SMs idle (tile counts at cfg2: qkv 7.6 waves, fc1 10.2, out_proj/fc2 2.5, attention
 5.2).  With two independent batches in flight on two streams the CTAs of one stream's kernel start on
 the SMs the other stream's kernel has already left.  Diagnostic only: prints ms/step (device, CUDA
-events across both streams) for 1 stream and 2 streams; run with FBKST_PDL=0/1.
+events across both streams) for 1 stream and 2 streams.
 """
 import copy
 import json
@@ -65,7 +65,7 @@ def main():
         with torch.cuda.stream(streams[i % n_streams]):
             encs[i % n_streams](ops.cmvn(devb[i % 4][0], len32), devb[i % 4][1])
     torch.cuda.synchronize()
-    res = dict(n_streams=n_streams, pdl=os.environ.get("FBKST_PDL", "1"), steps=steps)
+    res = dict(n_streams=n_streams, steps=steps)
     for rep in range(2):
         s0, e0 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         main_s = torch.cuda.current_stream()

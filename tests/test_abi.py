@@ -61,7 +61,7 @@ def test_no_cpu_fallback(lib):
 
 
 def test_argument_errors_do_not_need_a_gpu(lib):
-    rc = lib.fbkst_linear_bf16(None, 8, None, 8, None, None, 0, None, 8, 4, 4, 8, 0, 0, 0, None, None, 0, None)
+    rc = lib.fbkst_linear_bf16(None, 8, None, 8, None, None, 0, None, 8, 4, 4, 8, 0, None, 0, None)
     assert rc == -1 and b"null operand" in lib.fbkst_last_error()
     rc = lib.fbkst_layernorm(1, 1, 1, 1, 0, 4, 100, ctypes.c_float(1e-5), None, 0, None)
     assert rc == -1 and b"unsupported D" in lib.fbkst_last_error()
