@@ -117,8 +117,9 @@ class B200ConvolutionalTransformerModel(_ref.ConvolutionalTransformerModel):
 # SURVEY 8f N1: the CTC half of ``ctc_multi_loss`` on the device kernels.  Same class, flags, sample fields,
 # logging keys and loss value as the reference criterion (criterions/ctc_multi_loss.py:107-194 +
 # CTC_loss.py:101-175); what changes is where the arithmetic runs: the frame arg-max, log-sum-exp, alpha /
-# beta recursions, the gradient w.r.t. the logits and the edit distance are CUDA kernels (fbkst_b200.criterion),
-# the T x B x V log-softmax is never materialised and nothing is pulled to the host per utterance.
+# beta recursions, the gradient w.r.t. the logits, the edit distance and (without --ctc-compress-out) the
+# criterion's CTC projection are CUDA kernels (fbkst_b200.criterion), the T x B x V log-softmax is never
+# materialised and nothing is pulled to the host per utterance.
 from fairseq import utils as _utils  # noqa: E402
 from fairseq.criterions import register_criterion  # noqa: E402
 from examples.speech_recognition.criterions import ctc_multi_loss as _cml  # noqa: E402
@@ -158,11 +159,15 @@ class B200CTCLoss(_cml.BaseCTCLoss):
 
 @register_criterion("ctc_multi_loss_b200")
 class B200CTCMultiLoss(_cml.CTCMultiLoss):
-    """``--criterion ctc_multi_loss_b200``: the reference's CTCMultiLoss with its CTC term on the GPU kernels."""
+    """``--criterion ctc_multi_loss_b200``: the reference's CTCMultiLoss with its CTC term on the GPU kernels.
+    Without --ctc-compress-out the criterion projects ``encoder_states[ctc_encoder_layer - 1]`` with its own
+    ``fc_out`` (SURVEY F13: ``ctc_aware_model.fc_out``): that Linear is swapped for ``criterion.CtcProjection``
+    (same parameters and state-dict keys; tcgen05 GEMMs, and its backward runs inside the CTC loss node)."""
 
     def __init__(self, args, task):
         super().__init__(args, task)
         self.ctc_criterion = B200CTCLoss(args, task)
+        _crit.install_ctc_projection(self)
 
 
 for _name, _fn in (("conv_transformer_b200", _ref.base_architecture),

@@ -300,15 +300,20 @@ class EncoderTrainFn(torch.autograd.Function):
         ctx.has_ctc = x_ctc is not None
         extras = dict(mask=mask, ctc_mask=ctc_mask, states=states, out_len=cur_host)
         enc._train_extras = extras
+        # the intermediate states (x2 after each layer but the last, compressed after the CTC layer) come last:
+        # a loss on one of them (the CTC-multitask recipe without --ctc-compress-out projects encoder_states[k-1])
+        # sends its gradient back into this node.  They are the saved activations the backward reads.
         if x_ctc is None:
-            return (out,)
+            return (out,) + tuple(states[:-1])
         # third output: the CTC projection's INPUT.  A criterion that computes the projection's backward itself
         # (criterion.CtcProjLossFn: early in the backward, while the decoder's backward keeps the host busy)
         # sends d loss / d x back through it; with any other criterion the gradient arrives through ctc_ret
-        return out, ctc_ret, ctc_tap
+        return (out, ctc_ret, ctc_tap) + tuple(states[:-1])
 
     @staticmethod
-    def backward(ctx, d_out, d_ctc=None, d_tap=None):
+    def backward(ctx, d_out, *d_rest):
+        d_ctc, d_tap = (d_rest[0], d_rest[1]) if ctx.has_ctc else (None, None)
+        d_states = d_rest[2:] if ctx.has_ctc else d_rest
         S, enc = ctx.S, ctx.enc
         if getattr(enc, "_train_pending", None) is S:  # no criterion node did it earlier: one batched launch here
             enc._train_pending = None
@@ -333,6 +338,11 @@ class EncoderTrainFn(torch.autograd.Function):
                 cur_L, cur_len, sites = R["L"], R["lengths"], R["sites"]
                 M = cur_L * B
                 g = {}
+                d_state = d_states[li] if li < len(d_states) else None
+                if d_state is not None:
+                    # dx is d loss / d (this layer's output): the state's own gradient joins it here, on the
+                    # compressed rows for the CTC layer (before ctc_compress_bwd)
+                    dx += d_state.reshape(dx.shape)
                 if R["ctc"] is not None:
                     ct = R["ctc"]
                     # dx holds the L2*B compressed rows; a frame's segment id is < its utterance's new length <= L2
@@ -423,7 +433,10 @@ def _assemble_grads(enc, G, have_ctc):
 
 def forward_train(enc, src_tokens, src_lengths, return_all_hiddens):
     """The encoder's forward when gradients are required: returns the reference's output tuple, with
-    ``encoder_out`` and ``ctc_out`` attached to the autograd graph."""
+    ``encoder_out``, ``ctc_out`` and (``return_all_hiddens``) every entry of ``encoder_states`` attached to the
+    autograd graph: a loss on an intermediate state (CTC multitask without --ctc-compress-out) trains the layers
+    below it.  The intermediate states are the saved activations the backward reads: consumers must not modify
+    them in place (fairseq does not; autograd refuses it in fp32, where they are views the node created)."""
     from .encoder import CTCAwareEncoderOut, EncoderOut  # (resolved late: the plugin swaps in fairseq's types)
     from . import encoder as _e
     if enc.training and enc.encoder_layerdrop > 0:
@@ -438,10 +451,12 @@ def forward_train(enc, src_tokens, src_lengths, return_all_hiddens):
     seed = int(torch.empty((), dtype=torch.int64).random_().item()) if enc.training else 0
     params = flat_parameters(enc)
     res = EncoderTrainFn.apply(enc, src_tokens, len_host, seed, *params)
-    tap = res[2] if len(res) > 2 else None
-    res = res[:2]
     ex = enc._train_extras
     enc._train_extras = None
+    n_head = len(res) - (len(ex["states"]) - 1)
+    res, mid = res[:n_head], list(res[n_head:])
+    tap = res[2] if len(res) > 2 else None
+    res = res[:2]
     out = res[0]
     odt = enc.layer_norm.weight.dtype
     if odt != torch.float32:  # model.half(): hand fp16 activations to the fp16 decoder (differentiable casts)
@@ -453,7 +468,11 @@ def forward_train(enc, src_tokens, src_lengths, return_all_hiddens):
         res[1]._fbkst_tap = (tap, enc)
     states = None
     if return_all_hiddens:
-        states = [s.detach() for s in ex["states"][:-1]] + [out]
+        if odt != torch.float32:
+            mid = [s.to(odt) for s in mid]
+        for s in mid:  # read by criterion.CtcProjection: whose pending activation transposes its backward starts
+            s._fbkst_encoder = enc
+        states = mid + [out]
     out_lengths = torch.tensor(ex["out_len"], dtype=src_lengths.dtype, device=src_tokens.device)
     if enc.ctc_compress_out:
         return _e.CTCAwareEncoderOut(out, ex["mask"], None, states, src_tokens, out_lengths,
