@@ -12,6 +12,7 @@
 //   im2col_t                 conv2 wgrad operand: colT[(tap, ci), pixel] (bf16) from conv1's fp16 output
 //   col2im                   conv2 dgrad: gather-sum of the <= 4 taps that reach an input pixel
 //   conv1_wgrad              dW1[co, tap], db1[co]: K = 9 outer products, SIMT (HBM-bound on the gradient read)
+//   conv1_dgrad              dx[b, t, f]: the gradient of the input features (attribution, input-gradient losses)
 // The contractions themselves (conv2 wgrad / dgrad as GEMMs over these operands, fc3) run on the CTA-pair
 // tcgen05 kernel (gemm2_tcgen05.cu).
 #include <cuda_bf16.h>
@@ -372,6 +373,89 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+// ------------------------------------------------------------------ conv1 data gradient (input features)
+// dx[b, t, f] = sum_{kt, kf, c} w1[c, 3kt+kf] dz1[b, (t+1-kt)/2, (f+1-kf)/2, c] over the taps whose indices are
+// even and in range (stride 2, padding 1).  Input pixels come in 2x2 blocks (2i..2i+1, 2j..2j+1), one block per
+// conv1 output pixel (i, j); a block reads the four dz1 pixels (i|i+1, j|j+1) and every tap of every output lands
+// on one of them:
+//   dx[2i,   2j  ] = w4 z(i,j)
+//   dx[2i,   2j+1] = w3 z(i,j+1) + w5 z(i,j)
+//   dx[2i+1, 2j  ] = w1 z(i+1,j) + w7 z(i,j)
+//   dx[2i+1, 2j+1] = w0 z(i+1,j+1) + w2 z(i+1,j) + w6 z(i,j+1) + w8 z(i,j)
+// A group of C/8 lanes shares a block: lane k owns channels 8k..8k+7 (one 16-byte load per dz1 pixel, so a group
+// reads each pixel's C channels as one contiguous segment) and keeps those channels' 9 taps in registers for the
+// whole grid-stride loop.  The group's four partial sums are combined with a fixed xor butterfly: no atomics, the
+// same bits on every call.
+template <int C>
+__global__ void __launch_bounds__(256)
+    conv1_dgrad_kernel(const __nv_bfloat16* __restrict__ dz1, const float* __restrict__ w1, float* __restrict__ dx,
+                       int B, int T, int F, int T1, int F1) {
+  constexpr int G = C / 8;  // lanes per block: 8 or 16
+  const int k = threadIdx.x % G;
+  float w[9][8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+#pragma unroll
+    for (int tap = 0; tap < 9; ++tap) w[tap][j] = __ldg(w1 + (k * 8 + j) * 9 + tap);
+  }
+  // the loop runs warp by warp (the butterfly needs every lane): a group past the last block computes zeros.
+  // 32-bit indices (the host checks B*T1*F1 < 2^31): 64-bit divisions dominated the first version's time.
+  constexpr int GPW = 32 / G;  // groups per warp
+  const unsigned blocks = (unsigned)B * T1 * F1;
+  const unsigned stride = gridDim.x * (blockDim.x / 32) * GPW;
+  for (unsigned base = (blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32) * GPW; base < blocks; base += stride) {
+    const unsigned blk = base + (threadIdx.x % 32) / G;
+    const bool valid = blk < blocks;
+    const unsigned r = blk / F1;
+    const int j = (int)(blk - r * F1), i = (int)(r % T1), b = (int)(r / T1);
+    const bool right = valid && j + 1 < F1, down = valid && i + 1 < T1;
+    const __nv_bfloat16* p = dz1 + (size_t)blk * C + k * 8;
+    const uint4 zero = make_uint4(0, 0, 0, 0);
+    const uint4 u00 = valid ? __ldg(reinterpret_cast<const uint4*>(p)) : zero;
+    const uint4 u01 = right ? __ldg(reinterpret_cast<const uint4*>(p + C)) : zero;
+    const uint4 u10 = down ? __ldg(reinterpret_cast<const uint4*>(p + (size_t)F1 * C)) : zero;
+    const uint4 u11 = right && down ? __ldg(reinterpret_cast<const uint4*>(p + (size_t)(F1 + 1) * C)) : zero;
+    const uint32_t a00[4] = {u00.x, u00.y, u00.z, u00.w}, a01[4] = {u01.x, u01.y, u01.z, u01.w};
+    const uint32_t a10[4] = {u10.x, u10.y, u10.z, u10.w}, a11[4] = {u11.x, u11.y, u11.z, u11.w};
+    // one accumulator per tap: nine independent FMA chains of 8 instead of one chain of 32 for dx[2i+1, 2j+1]
+    float acc[9];
+#pragma unroll
+    for (int tap = 0; tap < 9; ++tap) acc[tap] = 0.f;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      const int h = q >> 1;
+      const float z00 = (q & 1) ? bf_hi(a00[h]) : bf_lo(a00[h]), z01 = (q & 1) ? bf_hi(a01[h]) : bf_lo(a01[h]);
+      const float z10 = (q & 1) ? bf_hi(a10[h]) : bf_lo(a10[h]), z11 = (q & 1) ? bf_hi(a11[h]) : bf_lo(a11[h]);
+      acc[4] = fmaf(w[4][q], z00, acc[4]);
+      acc[3] = fmaf(w[3][q], z01, acc[3]);
+      acc[5] = fmaf(w[5][q], z00, acc[5]);
+      acc[1] = fmaf(w[1][q], z10, acc[1]);
+      acc[7] = fmaf(w[7][q], z00, acc[7]);
+      acc[0] = fmaf(w[0][q], z11, acc[0]);
+      acc[2] = fmaf(w[2][q], z10, acc[2]);
+      acc[6] = fmaf(w[6][q], z01, acc[6]);
+      acc[8] = fmaf(w[8][q], z00, acc[8]);
+    }
+    float s00 = acc[4], s01 = acc[3] + acc[5], s10 = acc[1] + acc[7], s11 = (acc[0] + acc[2]) + (acc[6] + acc[8]);
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) {
+      s00 += __shfl_xor_sync(0xffffffffu, s00, o);
+      s01 += __shfl_xor_sync(0xffffffffu, s01, o);
+      s10 += __shfl_xor_sync(0xffffffffu, s10, o);
+      s11 += __shfl_xor_sync(0xffffffffu, s11, o);
+    }
+    // lanes 0..3 of the group store the four outputs that exist (T and F may be odd)
+    if (valid && k < 4) {
+      const int dt = k >> 1, df = k & 1;
+      const int t = 2 * i + dt, f = 2 * j + df;
+      if (t < T && f < F) {
+        const float v = k == 0 ? s00 : k == 1 ? s01 : k == 2 ? s10 : s11;
+        dx[((size_t)b * T + t) * F + f] = v;
+      }
+    }
+  }
+}
+
 static inline int cv_grid(long long n, int cap_mult) {
   long long g = (n + 255) / 256;
   const long long cap = (long long)num_sms() * cap_mult;
@@ -419,13 +503,16 @@ extern "C" int fbkst_bn_apply(const void* x_f16, void* y_f16, const float* scale
 }
 
 /* dz [P, C] bf16 = autograd of dropout(BatchNorm(relu_out)) . relu w.r.t. the conv output, given dy [P, C] bf16;
- * sums [2, C] receives (dbeta | dgamma);  partial: [fbkst_bn_partial_blocks(), 2, C] floats */
+ * sums [2, C] receives (dbeta | dgamma);  partial: [fbkst_bn_partial_blocks(), 2, C] floats.  With running
+ * statistics dz does not read the sums: sums == NULL (and partial == NULL) skips their reduction pass. */
 extern "C" int fbkst_bn_relu_bwd(const void* dy_bf16, const void* relu_out_f16, const float* gamma,
                                  const float* mean, const float* rstd, int batch_stats, void* dz_bf16,
                                  float* sums, float* partial, int64_t pixels, int C, float p, uint64_t seed,
                                  int site, fbkst_stream_t stream) {
-  FBKST_REQUIRE(dy_bf16 && relu_out_f16 && gamma && mean && rstd && dz_bf16 && sums && partial && pixels > 0,
+  FBKST_REQUIRE(dy_bf16 && relu_out_f16 && gamma && mean && rstd && dz_bf16 && pixels > 0,
                 "fbkst_bn_relu_bwd: bad arguments");
+  FBKST_REQUIRE(sums ? partial != nullptr : !batch_stats,
+                "fbkst_bn_relu_bwd: sums and partial are required (batch statistics read the sums)");
   FBKST_REQUIRE(C == 64 || C == 128, "fbkst_bn_relu_bwd: C must be 64 or 128");
   FBKST_REQUIRE(p >= 0.f && p < 1.f, "fbkst_bn_relu_bwd: p must be in [0, 1)");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -433,13 +520,15 @@ extern "C" int fbkst_bn_relu_bwd(const void* dy_bf16, const void* relu_out_f16, 
   const int G = fbkst_bn_partial_blocks();
   const __nv_bfloat16* dy = reinterpret_cast<const __nv_bfloat16*>(dy_bf16);
   const __half* xr = reinterpret_cast<const __half*>(relu_out_f16);
-  if (C == 64)
-    bn_bwd_reduce_kernel<64><<<G, 256, 0, st>>>(dy, xr, mean, rstd, pixels, partial, dp);
-  else
-    bn_bwd_reduce_kernel<128><<<G, 256, 0, st>>>(dy, xr, mean, rstd, pixels, partial, dp);
-  FBKST_CHECK_CUDA(cudaGetLastError());
-  int rc = fbkst_reduce_sum(partial, G, 2 * C, 1, 2 * C, 2 * C, sums, 2 * C, 1.0f, stream);
-  if (rc) return rc;
+  if (sums != nullptr) {
+    if (C == 64)
+      bn_bwd_reduce_kernel<64><<<G, 256, 0, st>>>(dy, xr, mean, rstd, pixels, partial, dp);
+    else
+      bn_bwd_reduce_kernel<128><<<G, 256, 0, st>>>(dy, xr, mean, rstd, pixels, partial, dp);
+    FBKST_CHECK_CUDA(cudaGetLastError());
+    int rc = fbkst_reduce_sum(partial, G, 2 * C, 1, 2 * C, 2 * C, sums, 2 * C, 1.0f, stream);
+    if (rc) return rc;
+  }
   bn_bwd_apply_kernel<<<cv_grid(pixels * (C / 4), 8), 256, 0, st>>>(dy, xr, gamma, mean, rstd, sums, batch_stats,
                                                                    reinterpret_cast<__nv_bfloat16*>(dz_bf16),
                                                                    pixels, C, dp);
@@ -491,4 +580,23 @@ extern "C" int fbkst_conv1_wgrad(const void* dz1_bf16, const float* x, float* dw
     conv1_wgrad_kernel<128><<<G, 256, smem, st>>>(dz, x, B, T, F, T1, F1, partial);
   FBKST_CHECK_CUDA(cudaGetLastError());
   return fbkst_reduce_sum(partial, G, (int64_t)C * 10, 1, C * 10, C * 10, dw1b, C * 10, 1.0f, stream);
+}
+
+/* dx [B,T,F] fp32 = gradient of conv1's input from dz1 [B,T1,F1,C] bf16 and w1 [C, 9] fp32 (every input position,
+ * padded frames included) */
+extern "C" int fbkst_conv1_dgrad(const void* dz1_bf16, const float* w1, float* dx, int B, int T, int F, int C,
+                                 fbkst_stream_t stream) {
+  FBKST_REQUIRE(dz1_bf16 && w1 && dx && B > 0 && T > 0 && F > 0 && (C == 64 || C == 128),
+                "fbkst_conv1_dgrad: bad arguments");
+  const int T1 = (T + 1) / 2, F1 = (F + 1) / 2;
+  FBKST_REQUIRE((long long)B * T1 * F1 < (1LL << 31) - 256 * 32, "fbkst_conv1_dgrad: batch too large");
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const long long lanes = (long long)B * T1 * F1 * (C / 8);
+  const __nv_bfloat16* dz = reinterpret_cast<const __nv_bfloat16*>(dz1_bf16);
+  if (C == 64)
+    conv1_dgrad_kernel<64><<<cv_grid(lanes, 2), 256, 0, st>>>(dz, w1, dx, B, T, F, T1, F1);
+  else
+    conv1_dgrad_kernel<128><<<cv_grid(lanes, 2), 256, 0, st>>>(dz, w1, dx, B, T, F, T1, F1);
+  FBKST_CHECK_CUDA(cudaGetLastError());
+  return FBKST_OK;
 }

@@ -79,6 +79,7 @@ SIGNATURES = {
     "fbkst_conv2_im2col_t": [P, P, I64, I, I, I, I, P],
     "fbkst_conv2_col2im": [P, P, I, I, I, I, P],
     "fbkst_conv1_wgrad": [P, P, P, P, I, I, I, I, P],
+    "fbkst_conv1_dgrad": [P, P, P, I, I, I, I, P],
 }
 _RESTYPES = {"fbkst_linear_wgrad_workspace": (c_int64, [I, I, I]),
              "fbkst_ctc_loss_bwd_workspace": (c_int64, [I, I, I])}

@@ -444,9 +444,11 @@ def make_encoder_class(base):
                 raise RuntimeError("fbkst_b200: src_tokens must be a CUDA tensor (no CPU fallback)")
             # Training semantics (BatchNorm batch statistics, dropout) whenever the module is in train();
             # the differentiable chain also serves eval() with gradients enabled (running statistics, no
-            # dropout).  Both run fbkst_b200.train: hand-written forward + backward kernels, no PyTorch
+            # dropout) when a parameter or the input features require a gradient (attribution with a frozen
+            # model).  Both run fbkst_b200.train: hand-written forward + backward kernels, no PyTorch
             # arithmetic.  Everything else is the inference path.
-            if self.training or (torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())):
+            if self.training or (torch.is_grad_enabled() and (
+                    src_tokens.requires_grad or any(p.requires_grad for p in self.parameters()))):
                 if self._precision != "bf16":
                     raise NotImplementedError(
                         "fbkst_b200: precision=%r is inference only (eval() under torch.no_grad()); training and "

@@ -804,9 +804,9 @@ def dropout_add_ln(y, residual=None, gamma=None, beta=None, eps=1e-5, p=0.0, see
     return x1, ln
 
 
-def ln_bwd(dy, x, gamma, dx=None, eps=1e-5):
+def ln_bwd(dy, x, gamma, dx=None, eps=1e-5, want_params=True):
     """LayerNorm backward.  dx: fp32 [M, D] holding the residual branch's gradient (accumulated into), or None.
-    -> (dx, dgamma [D], dbeta [D])."""
+    -> (dx, dgamma [D], dbeta [D]); want_params=False skips the parameter reduction: (dx, None, None)."""
     lib = _lib.require_device()
     _req(dy, torch.float32, "ln_bwd.dy"); _req(x, torch.float32, "ln_bwd.x")
     M, D = x.shape
@@ -818,8 +818,10 @@ def ln_bwd(dy, x, gamma, dx=None, eps=1e-5):
     partial = torch.empty(G, 2, D, dtype=torch.float32, device=x.device)
     check(lib.fbkst_ln_bwd(dy.data_ptr(), x.data_ptr(), gamma.data_ptr(), dx.data_ptr(), acc, partial.data_ptr(),
                            float(eps), M, D, _stream()))
-    dgb = torch.empty(2, D, dtype=torch.float32, device=x.device)
     _count()
+    if not want_params:
+        return dx, None, None
+    dgb = torch.empty(2, D, dtype=torch.float32, device=x.device)
     reduce_sum(partial, G, 2 * D, 1, 2 * D, 2 * D, dgb, 2 * D)
     return dx, dgb[0], dgb[1]
 
@@ -982,19 +984,24 @@ def bn_apply(x, scale, shift, p=0.0, seed=0, site=0):
     return y
 
 
-def bn_relu_bwd(dy, relu_out, gamma, mean, rstd, batch_stats, p=0.0, seed=0, site=0):
-    """-> (dz bf16 like dy, dbeta [C], dgamma [C])."""
+def bn_relu_bwd(dy, relu_out, gamma, mean, rstd, batch_stats, p=0.0, seed=0, site=0, want_params=True):
+    """-> (dz bf16 like dy, dbeta [C], dgamma [C]).  want_params=False with running statistics (a frozen
+    BatchNorm in eval()) skips the parameter reduction and returns (dz, None, None)."""
     lib = _lib.require_device()
     _req(dy, torch.bfloat16, "bn_relu_bwd.dy"); _req(relu_out, torch.float16, "bn_relu_bwd.relu_out")
     C = dy.shape[-1]
     P = dy.numel() // C
     dz = torch.empty_like(dy)
-    sums = torch.empty(2, C, dtype=torch.float32, device=dy.device)
-    partial = torch.empty(lib.fbkst_bn_partial_blocks(), 2, C, dtype=torch.float32, device=dy.device)
+    sums = partial = None
+    if want_params or batch_stats:
+        sums = torch.empty(2, C, dtype=torch.float32, device=dy.device)
+        partial = torch.empty(lib.fbkst_bn_partial_blocks(), 2, C, dtype=torch.float32, device=dy.device)
     check(lib.fbkst_bn_relu_bwd(dy.data_ptr(), relu_out.data_ptr(), gamma.data_ptr(), mean.data_ptr(),
-                                rstd.data_ptr(), 1 if batch_stats else 0, dz.data_ptr(), sums.data_ptr(),
-                                partial.data_ptr(), P, C, float(p), int(seed), int(site), _stream()))
-    _count(3)
+                                rstd.data_ptr(), 1 if batch_stats else 0, dz.data_ptr(), _ptr(sums),
+                                _ptr(partial), P, C, float(p), int(seed), int(site), _stream()))
+    _count(3 if sums is not None else 1)
+    if not want_params:
+        return dz, None, None
     return dz, sums[0], sums[1]
 
 
@@ -1033,6 +1040,21 @@ def conv1_wgrad(dz1, x):
                                 _stream()))
     _count(2)
     return out[:, :9], out[:, 9]
+
+
+def conv1_dgrad(dz1, w1, T, Fd):
+    """dz1 [B,T1,F1,C] bf16, w1 [C, 9] fp32 -> dx [B,T,Fd] fp32: the gradient of conv1's input (stride 2,
+    padding 1; T1 = (T+1)//2, F1 = (Fd+1)//2; T and Fd are not recoverable from dz1 when odd)."""
+    lib = _lib.require_device()
+    _req(dz1, torch.bfloat16, "conv1_dgrad.dz1"); _req(w1, torch.float32, "conv1_dgrad.w1")
+    B, T1, F1, C = dz1.shape
+    if T1 != (T + 1) // 2 or F1 != (Fd + 1) // 2 or tuple(w1.shape) != (C, 9):
+        raise ValueError("fbkst_b200.conv1_dgrad: dz1 %s / w1 %s do not fit an input of %d x %d"
+                         % (tuple(dz1.shape), tuple(w1.shape), T, Fd))
+    dx = torch.empty(B, T, Fd, dtype=torch.float32, device=dz1.device)
+    check(lib.fbkst_conv1_dgrad(dz1.data_ptr(), w1.data_ptr(), dx.data_ptr(), B, T, Fd, C, _stream()))
+    _count()
+    return dx
 
 
 def ctc_loss_bwd(logits, lse, in_lengths, targets, target_lengths, blank, grad_loss, L, B, V):

@@ -18,6 +18,11 @@ few [C]-sized views / permutes of weight gradients):
   tcgen05 (scores recomputed, no L x L buffer); LayerNorm / BatchNorm / ReLU / dropout backward as streaming
   kernels (dropout masks are regenerated from (seed, site, position)); conv2 as im2col GEMMs, conv1 (K = 9)
   as a reduction kernel; CTC compression backward (W is constant: d x[t] = W[t, seg(t)] d out[seg(t)]).
+  ``src_tokens`` is differentiable: its gradient is conv1's data gradient (``ops.conv1_dgrad``), in the input's dtype.
+* only what autograd asks for (``ctx.needs_input_grad``, read in the forward by ``_grad_plan``): a frozen parameter
+  gets no weight-gradient GEMM, no bias / LayerNorm / BatchNorm reduction and no transposed operand copy, and the
+  backward stops at the lowest tensor that needs a gradient (attribution with a frozen model, fine-tuning the top
+  layers).  Requested gradients are bitwise the same whatever else is frozen.
 
 Operand precision: bf16 GEMM operands / fp16 conv-front-end activations, fp32 accumulation, fp32 residual
 stream and fp32 parameter gradients in the reference's parameter layout (so fairseq's optimizers, gradient
@@ -138,6 +143,43 @@ def flat_parameters(enc):
     return ps
 
 
+_FRONT = ("cw1", "cb1", "bn0_w", "bn0_b", "cw2", "cb2", "bn1_w", "bn1_b", "w3", "b3")
+_LAYER = ("wo", "bo", "g1", "be1", "w1", "b1", "w2", "b2", "g2", "be2")
+# a layer's backward in order: the gradients each step yields (6 = the layer's input gradient, for what lies below)
+_LAYER_STEPS = (("w2", "b2"), ("w1", "b1"), ("g2", "be2"), ("wo", "bo"), ("wqkv", "bqkv"), ("g1", "be1"))
+
+
+def _grad_plan(enc, need, need_x):
+    """Which gradients the backward computes, from autograd's ``needs_input_grad`` for ``flat_parameters(enc)``
+    (``need``) and for ``src_tokens`` (``need_x``): flags under ``_assemble_grads``' names, plus per layer the
+    last step of its backward that has to run (``depth``, -1: none) and whether the front end runs at all."""
+    it = iter(need)
+    front = dict(zip(_FRONT, it))
+    layers = []
+    for lyr in enc.layers:
+        if hasattr(lyr.self_attn, "in_proj_weight"):
+            w, b = next(it), next(it)
+        else:  # q, k, v: one GEMM computes all three (autograd gets None for the frozen slices)
+            f = [next(it) for _ in range(6)]
+            w, b = any(f[0::2]), any(f[1::2])
+        d = dict(wqkv=w, bqkv=b)
+        d.update(zip(_LAYER, it))
+        layers.append(d)
+    top = dict(zip(("gf", "bf", "wc", "bc"), it))
+    below = need_x or any(front.values())
+    for li, d in enumerate(layers):  # bottom-up: a layer above anything that needs a gradient runs in full
+        own = max((s for s, names in enumerate(_LAYER_STEPS) if d[names[0]] or d[names[1]]), default=-1)
+        d["depth"] = len(_LAYER_STEPS) if below else own
+        # the CTC projection's gradients need the backward to reach the top of the CTC layer
+        d["ctc"] = enc.ctc_compress_out and enc.ctc_layer == li + 1 and (top.get("wc") or top.get("bc"))
+        below = below or own >= 0 or d["ctc"]
+    front["x"] = need_x
+    front["any"] = need_x or any(front[k] for k in _FRONT)
+    front["below_fc3"] = need_x or any(front[k] for k in _FRONT[:8])
+    front["below_conv2"] = need_x or any(front[k] for k in _FRONT[:4])
+    return dict(front=front, layers=layers, top=top)
+
+
 def _bn_state(enc, i, y_relu, train):
     """(mean, rstd, scale, shift) of BatchNorm i for this step: batch statistics (+ running-stat update,
     nn.BatchNorm2d momentum 0.1) in training, running statistics in eval."""
@@ -157,10 +199,12 @@ def _bn_state(enc, i, y_relu, train):
 
 def pretranspose(S):
     """Token-contiguous (transposed) bf16 copies of the activations the weight-gradient GEMMs read, for the saved
-    state ``S`` of one training forward: one batched launch (+ conv2's im2col).  Idempotent."""
+    state ``S`` of one training forward: one batched launch (+ conv2's im2col), each only when its weight gradient
+    is requested.  Idempotent."""
     if S is None or S.get("pretransposed"):
         return
     S["pretransposed"] = True
+    front = S["plan"]["front"]
     x_in = S["x_in"]
     dev = x_in.device
     jobs = []
@@ -169,10 +213,12 @@ def pretranspose(S):
         out = ops.transposed_buffer(t.shape[0], t.shape[1], dev)
         jobs.append((t, None, out))
         return out
-    y2 = S["y2"]
-    S["y2T"] = tjob(y2.view(y2.shape[0] * y2.shape[1], -1))
+    if front["w3"]:
+        y2 = S["y2"]
+        S["y2T"] = tjob(y2.view(y2.shape[0] * y2.shape[1], -1))
     ops.prep_batch(jobs)
-    S["colT"] = ops.conv2_im2col_t(S["y1"])
+    if front["cw2"]:
+        S["colT"] = ops.conv2_im2col_t(S["y1"])
 
 
 class EncoderTrainFn(torch.autograd.Function):
@@ -194,8 +240,14 @@ class EncoderTrainFn(torch.autograd.Function):
         lengths = torch.tensor(sub, dtype=torch.int32, device=dev)
         ones = torch.ones(C, dtype=torch.float32, device=dev)
         zeros = torch.zeros(C, dtype=torch.float32, device=dev)
+        # the plan is read-only and depends on the request alone: rebuilt only when it changes (30 us of host time
+        # per step at cfg4)
+        plan = getattr(enc, "_grad_plan", None)
+        if plan is None or plan[0] != ctx.needs_input_grad:
+            plan = enc._grad_plan = (ctx.needs_input_grad,
+                                     _grad_plan(enc, ctx.needs_input_grad[4:], ctx.needs_input_grad[1]))
         S = dict(B=B, T=T, Fd=Fd, L=L, train=train, seed=seed, p=p, p_conv=p_conv, p_att=p_att, p_act=p_act,
-                 x_in=x_in, lengths=lengths)
+                 x_in=x_in, lengths=lengths, plan=plan[1])
 
         # ---- conv front end: ReLU(conv) kept (BatchNorm / ReLU backward need it), BN + dropout as its own pass
         y1r = ops.conv1_relu_bn(x_in, W["w1"], W["b1"], ones, zeros)
@@ -291,7 +343,7 @@ class EncoderTrainFn(torch.autograd.Function):
         enc._train_pending = S if mode == "bwd" else None
         if mode == "fwd":
             pretranspose(S)
-        ctx.S, ctx.enc = S, enc
+        ctx.S, ctx.enc, ctx.x_dtype = S, enc, src_tokens.dtype
         if getattr(enc, "keep_train_state", False):  # tests: the activation patterns of this forward
             enc.last_train_state = S
         ctx.n_params = len(params)
@@ -323,6 +375,11 @@ class EncoderTrainFn(torch.autograd.Function):
         W = prepare_train_weights(enc)
         B, L, D, H, C = S["B"], S["L"], enc.embed_dim, enc.heads, enc.conv_channels
         seed, p, p_act, p_att, p_conv = S["seed"], S["p"], S["p_act"], S["p_att"], S["p_conv"]
+        # only what autograd asks for: weight gradients of frozen parameters (their GEMMs, bias / LayerNorm /
+        # BatchNorm reductions, transposed operands) are skipped, and the walk down the layers stops at the lowest
+        # tensor that needs a gradient
+        plan = S["plan"]
+        front, top = plan["front"], plan["top"]
         # every reduction whose result is only read when the backward returns (bias gradients, split-K slices of
         # the weight gradients, LayerNorm parameter gradients: ~120 per step) is queued and launched as ONE batch
         with ops.deferred_reductions():
@@ -332,103 +389,155 @@ class EncoderTrainFn(torch.autograd.Function):
                 dx = torch.zeros(M_out, D, dtype=torch.float32, device=S["x_in"].device)
             else:
                 dy = d_out.reshape(M_out, D).float().contiguous()
-                dx, G["gf"], G["bf"] = ops.ln_bwd(dy, S["x_last"], W["gf"], eps=enc.layer_norm.eps)
+                dx, G["gf"], G["bf"] = ops.ln_bwd(dy, S["x_last"], W["gf"], eps=enc.layer_norm.eps,
+                                                  want_params=top["gf"] or top["bf"])
             for li in range(len(S["layers"]) - 1, -1, -1):
-                R, Wl = S["layers"][li], W["layers"][li]
+                R, Wl, need = S["layers"][li], W["layers"][li], plan["layers"][li]
+                depth = need["depth"]
+                if depth < 0 and not need["ctc"]:
+                    break  # nothing at or below this layer needs a gradient
                 cur_L, cur_len, sites = R["L"], R["lengths"], R["sites"]
                 M = cur_L * B
                 g = {}
+                G[li] = g
                 d_state = d_states[li] if li < len(d_states) else None
-                if d_state is not None:
+                if d_state is not None and depth >= 0:
                     # dx is d loss / d (this layer's output): the state's own gradient joins it here, on the
                     # compressed rows for the CTC layer (before ctc_compress_bwd)
                     dx += d_state.reshape(dx.shape)
                 if R["ctc"] is not None:
                     ct = R["ctc"]
-                    # dx holds the L2*B compressed rows; a frame's segment id is < its utterance's new length <= L2
-                    dx = ops.ctc_compress_bwd(dx, ct["seg_id"], ct["weight"], cur_L, B)
-                    if d_tap is not None:
-                        dx += d_tap.reshape(M, D)
+                    if depth >= 0:
+                        # dx holds the L2*B compressed rows; a frame's segment id is < its utterance's new length
+                        # <= L2
+                        dx = ops.ctc_compress_bwd(dx, ct["seg_id"], ct["weight"], cur_L, B)
+                        if d_tap is not None:
+                            dx += d_tap.reshape(M, D)
                     if d_ctc is not None:
                         V = ct["V"]
                         Vp = (V + 7) // 8 * 8
                         gc = d_ctc.reshape(M, V)
                         if gc.dtype != torch.float32 or gc.stride(-1) != 1:
                             gc = gc.float().contiguous()
-                        gb, gT, G["bc"] = ops.grad_prep(gc, n_pad=Vp)
-                        G["wc"] = ops.linear_wgrad(gT, ops.transpose_bf16(ct["xb"]))
-                        wcT = W["wcT"]
-                        wcT_full = wcT if Vp == V else torch.as_strided(wcT, (D, Vp), (wcT.stride(0), 1))
-                        dx = ops.linear(gb, wcT_full, None, residual=dx, out_dtype=torch.float32)
+                        gb, gT, G["bc"] = ops.grad_prep(gc, n_pad=Vp, want_gb=depth >= 0, want_gT=bool(top["wc"]),
+                                                        want_colsum=bool(top["bc"]))
+                        if top["wc"]:
+                            G["wc"] = ops.linear_wgrad(gT, ops.transpose_bf16(ct["xb"]))
+                        if depth >= 0:
+                            wcT = W["wcT"]
+                            wcT_full = wcT if Vp == V else torch.as_strided(wcT, (D, Vp), (wcT.stride(0), 1))
+                            dx = ops.linear(gb, wcT_full, None, residual=dx, out_dtype=torch.float32)
+                    if depth < 0:
+                        break
                 # ---- feed-forward block (transformer_layer.py:124-136).  The weight gradients read the saved
                 # activations in their natural [tokens, features] layout (both operands MN-major in the tensor
                 # cores), not token-contiguous transposed copies: measured (cfg4, r02x) backward 20.7 -> 20.05 ms
-                g2, _, g["b2"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["ffn"], dp_cols=D, want_gT=False)
-                g["w2"] = ops.linear_wgrad_nt(g2, R["f"])
-                df = ops.linear(g2, Wl["w2T"])
-                dh, _, g["b1"] = ops.grad_prep(df, act=R["f"], act_scale=1.0 / (1.0 - p_act) if p_act > 0 else 1.0,
-                                               want_gT=False)
-                g["w1"] = ops.linear_wgrad_nt(dh, R["ln2"])
-                dln2 = ops.linear(dh, Wl["w1T"], out_dtype=torch.float32)
-                dx, g["g2"], g["be2"] = ops.ln_bwd(dln2, R["x1"], Wl["g2"], dx=dx, eps=Wl["eps2"])
+                g2, _, g["b2"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["ffn"], dp_cols=D, want_gT=False,
+                                               want_colsum=need["b2"])
+                if need["w2"]:
+                    g["w2"] = ops.linear_wgrad_nt(g2, R["f"])
+                if depth >= 1:
+                    df = ops.linear(g2, Wl["w2T"])
+                    dh, _, g["b1"] = ops.grad_prep(df, act=R["f"],
+                                                   act_scale=1.0 / (1.0 - p_act) if p_act > 0 else 1.0,
+                                                   want_gT=False, want_colsum=need["b1"])
+                    if need["w1"]:
+                        g["w1"] = ops.linear_wgrad_nt(dh, R["ln2"])
+                if depth >= 2:
+                    dln2 = ops.linear(dh, Wl["w1T"], out_dtype=torch.float32)
+                    dx, g["g2"], g["be2"] = ops.ln_bwd(dln2, R["x1"], Wl["g2"], dx=dx, eps=Wl["eps2"],
+                                                       want_params=need["g2"] or need["be2"])
                 # ---- self-attention block (:104-122)
-                g1, _, g["bo"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["out"], dp_cols=D, want_gT=False)
-                g["wo"] = ops.linear_wgrad_nt(g1, R["att"])
-                dO = ops.linear(g1, Wl["woT"])
-                dqkv = ops.attention_train_bwd(R["qkv"], R["att"], dO, R["lse"], cur_len, cur_L, B, H, enc.log_penalty,
-                                               p_att, seed, sites["att"])
-                _, _, g["bqkv"] = ops.grad_prep(dqkv, want_gb=False, want_gT=False)
-                g["wqkv"] = ops.linear_wgrad_nt(dqkv, R["ln1"])
-                dln1 = ops.linear(dqkv, Wl["wqkvT"], out_dtype=torch.float32)
-                dx, g["g1"], g["be1"] = ops.ln_bwd(dln1, R["x"], Wl["g1"], dx=dx, eps=Wl["eps1"])
-                G[li] = g
-            # ---- embedding dropout, positions (constant), fc3 + ReLU (conv_transformer.py:225-232)
-            F2C = S["y2"].shape[2] * C
-            dh3, dh3T, G["b3"] = ops.grad_prep(dx, act=S["h3b"], remap=(L, B), p=p, seed=seed, site=_SITE_EMB, dp_cols=D)
-            y2T = S["y2T"] if "y2T" in S else ops.transpose_bf16(S["y2"].view(B * L, F2C))
-            dW3p = ops.linear_wgrad(dh3T, y2T)  # [D, F2*C] (f, c) order
-            dy2 = ops.linear(dh3, W["w3T"])  # [B*L, F2*C] bf16 == [B, T2, F2, C]
-            # ---- conv2 block
-            bn = enc.bn[1]
-            dz2, G["bn1_b"], G["bn1_w"] = ops.bn_relu_bwd(dy2.view(S["y2"].shape), S["y2r"], bn.weight.detach().float(),
-                                                          S["bn2"][0], S["bn2"][1], S["train"], p_conv, seed, _SITE_CONV2)
-            P2 = dz2.numel() // C
-            _, dz2T, G["cb2"] = ops.grad_prep(dz2.view(P2, C), want_gb=False)
-            dW2p = ops.linear_wgrad(dz2T, S["colT"] if "colT" in S else ops.conv2_im2col_t(S["y1"]))  # [Cout, (tap, ci)]
-            dcol = ops.linear(dz2.view(P2, C), W["w2d"])
-            T1, F1 = S["y1"].shape[1], S["y1"].shape[2]
-            dy1 = ops.conv2_col2im(dcol, B, T1, F1, C)
-            # ---- conv1 block
-            bn = enc.bn[0]
-            dz1, G["bn0_b"], G["bn0_w"] = ops.bn_relu_bwd(dy1, S["y1r"], bn.weight.detach().float(), S["bn1"][0],
-                                                          S["bn1"][1], S["train"], p_conv, seed, _SITE_CONV1)
-            dW1, G["cb1"] = ops.conv1_wgrad(dz1, S["x_in"])
-            G["cw1"] = dW1.reshape(C, 1, 3, 3)
-        G["w3"] = dW3p.view(D, enc.feat_out, C).permute(0, 2, 1).reshape(D, C * enc.feat_out)
-        G["cw2"] = dW2p.view(C, 3, 3, C).permute(0, 3, 1, 2).contiguous()
+                if depth >= 3:
+                    g1, _, g["bo"] = ops.grad_prep(dx, p=p, seed=seed, site=sites["out"], dp_cols=D, want_gT=False,
+                                                   want_colsum=need["bo"])
+                    if need["wo"]:
+                        g["wo"] = ops.linear_wgrad_nt(g1, R["att"])
+                if depth >= 4:
+                    dO = ops.linear(g1, Wl["woT"])
+                    dqkv = ops.attention_train_bwd(R["qkv"], R["att"], dO, R["lse"], cur_len, cur_L, B, H,
+                                                   enc.log_penalty, p_att, seed, sites["att"])
+                    if need["bqkv"]:
+                        _, _, g["bqkv"] = ops.grad_prep(dqkv, want_gb=False, want_gT=False)
+                    if need["wqkv"]:
+                        g["wqkv"] = ops.linear_wgrad_nt(dqkv, R["ln1"])
+                if depth >= 5:
+                    dln1 = ops.linear(dqkv, Wl["wqkvT"], out_dtype=torch.float32)
+                    dx, g["g1"], g["be1"] = ops.ln_bwd(dln1, R["x"], Wl["g1"], dx=dx, eps=Wl["eps1"],
+                                                       want_params=need["g1"] or need["be1"])
+            if front["any"]:
+                # ---- embedding dropout, positions (constant), fc3 + ReLU (conv_transformer.py:225-232)
+                F2C = S["y2"].shape[2] * C
+                dh3, dh3T, G["b3"] = ops.grad_prep(dx, act=S["h3b"], remap=(L, B), p=p, seed=seed, site=_SITE_EMB,
+                                                   dp_cols=D, want_gb=front["below_fc3"], want_gT=front["w3"],
+                                                   want_colsum=front["b3"])
+                if front["w3"]:
+                    y2T = S["y2T"] if "y2T" in S else ops.transpose_bf16(S["y2"].view(B * L, F2C))
+                    dW3p = ops.linear_wgrad(dh3T, y2T)  # [D, F2*C] (f, c) order
+            if front["below_fc3"]:
+                dy2 = ops.linear(dh3, W["w3T"])  # [B*L, F2*C] bf16 == [B, T2, F2, C]
+                # ---- conv2 block
+                bn = enc.bn[1]
+                dz2, G["bn1_b"], G["bn1_w"] = ops.bn_relu_bwd(dy2.view(S["y2"].shape), S["y2r"],
+                                                              bn.weight.detach().float(), S["bn2"][0], S["bn2"][1],
+                                                              S["train"], p_conv, seed, _SITE_CONV2,
+                                                              want_params=front["bn1_w"] or front["bn1_b"])
+                P2 = dz2.numel() // C
+                if front["cw2"] or front["cb2"]:
+                    _, dz2T, G["cb2"] = ops.grad_prep(dz2.view(P2, C), want_gb=False, want_gT=front["cw2"],
+                                                      want_colsum=front["cb2"])
+                if front["cw2"]:
+                    # [Cout, (tap, ci)]
+                    dW2p = ops.linear_wgrad(dz2T, S["colT"] if "colT" in S else ops.conv2_im2col_t(S["y1"]))
+            if front["below_conv2"]:
+                dcol = ops.linear(dz2.view(P2, C), W["w2d"])
+                T1, F1 = S["y1"].shape[1], S["y1"].shape[2]
+                dy1 = ops.conv2_col2im(dcol, B, T1, F1, C)
+                # ---- conv1 block
+                bn = enc.bn[0]
+                dz1, G["bn0_b"], G["bn0_w"] = ops.bn_relu_bwd(dy1, S["y1r"], bn.weight.detach().float(),
+                                                              S["bn1"][0], S["bn1"][1], S["train"], p_conv, seed,
+                                                              _SITE_CONV1, want_params=front["bn0_w"] or front["bn0_b"])
+                if front["cw1"] or front["cb1"]:
+                    dW1, G["cb1"] = ops.conv1_wgrad(dz1, S["x_in"])
+                    G["cw1"] = dW1.reshape(C, 1, 3, 3)
+                if front["x"]:
+                    # the input features' gradient (the fp16 rounding of the conv operand counts as identity)
+                    G["x"] = ops.conv1_dgrad(dz1, W["w1"], S["T"], S["Fd"])
+        if front["w3"]:
+            G["w3"] = dW3p.view(D, enc.feat_out, C).permute(0, 2, 1).reshape(D, C * enc.feat_out)
+        if front["cw2"]:
+            G["cw2"] = dW2p.view(C, 3, 3, C).permute(0, 3, 1, 2).contiguous()
         ctx.S = None  # release the saved activations
-        grads = _assemble_grads(enc, G, d_ctc is not None)
+        params = flat_parameters(enc)
+        grads = _assemble_grads(enc, G, ctx.needs_input_grad[4:])
         # fp16 training (`--fp16`: model.half(), fp32 master copy in fairseq's FP16Optimizer): autograd wants
-        # every gradient in its parameter's dtype
-        grads = [g if g is None or g.dtype == p.dtype else g.to(p.dtype) for g, p in zip(grads, flat_parameters(enc))]
-        return (None, None, None, None) + tuple(grads)
+        # every gradient in its parameter's dtype, and the input's gradient in the input's dtype
+        grads = [g if g is None or g.dtype == p.dtype else g.to(p.dtype) for g, p in zip(grads, params)]
+        dx_in = G.get("x")
+        if dx_in is not None and dx_in.dtype != ctx.x_dtype:
+            dx_in = dx_in.to(ctx.x_dtype)
+        return (None, dx_in, None, None) + tuple(grads)
 
 
-def _assemble_grads(enc, G, have_ctc):
+def _assemble_grads(enc, G, need):
+    """The gradients in ``flat_parameters`` order; None wherever autograd asked for none."""
     D = enc.embed_dim
-    out = [G["cw1"], G["cb1"], G["bn0_w"], G["bn0_b"], G["cw2"], G["cb2"], G["bn1_w"], G["bn1_b"], G["w3"], G["b3"]]
+    out = [G.get(k) for k in _FRONT]
     for li, lyr in enumerate(enc.layers):
-        g = G[li]
+        g = G.get(li, {})
+        wqkv, bqkv = g.get("wqkv"), g.get("bqkv")
         if hasattr(lyr.self_attn, "in_proj_weight"):
-            out += [g["wqkv"], g["bqkv"]]
+            out += [wqkv, bqkv]
         else:
             for k in range(3):
-                out += [g["wqkv"][k * D:(k + 1) * D], g["bqkv"][k * D:(k + 1) * D]]
-        out += [g["wo"], g["bo"], g["g1"], g["be1"], g["w1"], g["b1"], g["w2"], g["b2"], g["g2"], g["be2"]]
+                out += [wqkv[k * D:(k + 1) * D] if wqkv is not None else None,
+                        bqkv[k * D:(k + 1) * D] if bqkv is not None else None]
+        out += [g.get(k) for k in _LAYER]
     out += [G.get("gf"), G.get("bf")]
     if enc.ctc_compress_out:
-        out += [G.get("wc"), G.get("bc")] if have_ctc else [None, None]
-    return out
+        out += [G.get("wc"), G.get("bc")]
+    return [o if n else None for o, n in zip(out, need)]
 
 
 def forward_train(enc, src_tokens, src_lengths, return_all_hiddens):

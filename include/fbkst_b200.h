@@ -517,7 +517,8 @@ int fbkst_bn_apply(const void* x_f16, void* y_f16, const float* scale, const flo
                    float p, uint64_t seed, int site, fbkst_stream_t stream);
 /* autograd of dropout(BatchNorm(relu(z))) w.r.t. z: dz [pixels, C] bf16 from dy [pixels, C] bf16 and the saved
  * ReLU output; batch_stats != 0: training-mode BatchNorm (mean / rstd of the batch), else running statistics.
- * sums [2, C] fp32 receives (dbeta | dgamma). */
+ * sums [2, C] fp32 receives (dbeta | dgamma).  With running statistics (batch_stats == 0) sums and partial may be
+ * NULL: the parameter reduction is skipped (frozen BatchNorm). */
 int fbkst_bn_relu_bwd(const void* dy_bf16, const void* relu_out_f16, const float* gamma, const float* mean,
                       const float* rstd, int batch_stats, void* dz_bf16, float* sums, float* partial,
                       int64_t pixels, int C, float p, uint64_t seed, int site, fbkst_stream_t stream);
@@ -529,6 +530,11 @@ int fbkst_conv2_col2im(const void* dcol_bf16, void* dy1_bf16, int B, int T1, int
 /* conv1 weight + bias gradient: dw1b [C, 10] fp32 = (dW1[co, kh*3+kw] | db1[co]) from dz1 [B,T1,F1,C] bf16 and
  * the input batch x [B,T,F] fp32.  partial: [fbkst_bn_partial_blocks(), C, 10]. */
 int fbkst_conv1_wgrad(const void* dz1_bf16, const float* x, float* dw1b, float* partial, int B, int T, int F, int C,
+                      fbkst_stream_t stream);
+/* conv1 input gradient: dx [B,T,F] fp32 = sum over the taps (stride 2, padding 1) of w1 [C, 9] fp32 (= the
+ * Conv2d weight [C,1,3,3]) times dz1 [B,T1,F1,C] bf16, T1 = (T+1)/2, F1 = (F+1)/2.  Every input position gets its
+ * gradient, padded frames included; fixed summation order (bit-identical across calls). */
+int fbkst_conv1_dgrad(const void* dz1_bf16, const float* w1, float* dx, int B, int T, int F, int C,
                       fbkst_stream_t stream);
 
 #ifdef __cplusplus
